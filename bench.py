@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (sm_100a kernels)
     python bench.py --impl reference --steps K --warmup W    # CPU arm: the reference's own modules on the host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR  # + the sampled structures of the last timed step as .npy
 
 One "step" = one full reverse-diffusion pass (T=100 denoise + update steps) over the rank's batch of
 synthetic 128-residue CDR-H3 patches (BASELINE config 3: 256 patches per GPU; weak scaling: every
@@ -47,7 +48,36 @@ def parse():
     ap.add_argument("--reverse-steps", type=int, default=T,
                     help="PROFILING ONLY: run this many of the T reverse steps per pass (ncu launch lists); "
                          "the JSON line is then marked profile_only and is not a bench value")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32; a seeded sample of the "
+                         "patches above 64 MB); the same arguments give the same inputs and random draws on every run")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out, dirname, limit=DUMP_BYTES):
+    """Write every array of `out` (leading dimension = patches) as `dirname`/<name>.npy in float32 (seq_idx holds
+    integers < 21, exact in float32).  When all patches would exceed `limit` bytes, a fixed sample of them (seeded
+    permutation, in ascending order) is written instead, with their indices in patch_index.npy (float64)."""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+    n = len(next(iter(arrays.values())))
+    per_patch = sum(a[0].nbytes for a in arrays.values())
+    if n * per_patch > limit:
+        keep = (limit - 4096) // (per_patch + 8)          # 4 KB: room for the .npy headers
+        idx = np.sort(np.random.default_rng(0).permutation(n)[:keep])
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["patch_index"] = idx.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirname, f"{k}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -255,20 +285,28 @@ def main():
         res_ctx, pair_ctx = torch.cat(res_parts), torch.cat(pair_parts)
         del res_parts, pair_parts
         m = b["generation_mask"]
-        s0 = torch.where(m, torch.randint(0, 21, (B, L), device=dev), b["seq_idx"])
-        x0 = torch.where(m[..., None], torch.randn(B, L, 3, device=dev), b["xyz"][:, :, 1])
-        O0 = torch.where(m[..., None, None], synth.uniform_rotations(B, L, device=dev), b["orientations"])
+        # the t = T state from its own seeded generator: it does not depend on what model construction drew before
+        g = torch.Generator(device=dev).manual_seed(3000 + rank)
+        s0 = torch.where(m, torch.randint(0, 21, (B, L), device=dev, generator=g), b["seq_idx"])
+        x0 = torch.where(m[..., None], torch.randn(B, L, 3, device=dev, generator=g), b["xyz"][:, :, 1])
+        O0 = torch.where(m[..., None, None], synth.uniform_rotations(B, L, generator=g, device=dev), b["orientations"])
 
     t_stop = T - args.reverse_steps + 1
     n_warm = max(args.warmup, 3) if args.reverse_steps == T else args.warmup
 
     def one_step():
+        # every step restarts the sampler's random draws from one seed: a step's result depends on neither --steps nor
+        # --warmup, nor on how many draws anything before it took
+        torch.cuda.manual_seed(4000 + rank)
         out = model.sample_from_context(s0, x0, O0, res_ctx, pair_ctx, m, use_cuda_graph=not args.no_graph,
                                         t_stop=t_stop)
         if dist is not None:   # gather the sampled structures on every rank (7,168 B per patch)
+            gathered = {}
             for k in ("seq_idx", "translations", "orientations"):
                 buf = torch.empty((world,) + out[k].shape, device=dev, dtype=out[k].dtype)
                 dist.all_gather_into_tensor(buf, out[k].contiguous())
+                gathered[k] = buf.flatten(0, 1)
+            out = gathered
         return out
 
     def barrier():
@@ -291,11 +329,14 @@ def main():
     barrier()
     ev0.record()
     for _ in range(args.steps):
-        one_step()
+        out = one_step()
     ev1.record()
     barrier()
     elapsed_ms = ev0.elapsed_time(ev1)
     clock_info = clocks.stop(skip=n_clock_warm)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
+    del out
     if dist is not None:
         tmax = torch.tensor([elapsed_ms], device=dev)
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)

@@ -52,7 +52,7 @@ def test_schedule_matches_reference():
 
 def test_context_encoders_match_reference_bitwise():
     g = load_golden("denoiser.pt")
-    model = DiffAb(*TRAIN)
+    model = DiffAb(*TRAIN, device="cpu")     # CPU modules on CPU inputs, also on a machine with a GPU
     model.load_state_dict(synth.synthetic_state(load_golden("state_shapes.pt"), seed=g["seed_state"]))
     b = synth.make_patches(2, 128, seed=g["seed_patches"])
     with torch.no_grad():
@@ -68,7 +68,7 @@ def test_context_encoders_match_reference_bitwise():
 
 def test_pair_embedding_backward_works():
     # the reference's in-place distmat ops break autograd (SURVEY F5a); ours must not
-    model = DiffAb(32, 16, 1, 8, 4, 4, 4)
+    model = DiffAb(32, 16, 1, 8, 4, 4, 4, device="cpu")
     b = synth.make_patches(1, 12, seed=2, cdr=(4, 8))
     res, pair = model.encode_context(b["seq_idx"], b["xyz"], b["orientations"], b["backbone_dihedrals"],
                                      b["distmat"], b["pairwise_dihedrals"], b["atom_mask"], b["chain_idx"],
