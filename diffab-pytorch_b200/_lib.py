@@ -147,9 +147,26 @@ def weight_generation():
 
 
 def bump_weight_generation():
-    """Declare that parameters may have changed behind PyTorch's back (updates replayed from a CUDA graph)."""
+    """Declare that parameters may have changed behind PyTorch's back (updates replayed from a CUDA graph, raw
+    ``.data`` writes)."""
     global _weight_generation
     _weight_generation += 1
+
+
+def weight_key(tensors):
+    """The key every weight-derived cache (packed weights, glue constants, captured sampling graphs) is checked against:
+    it changes when any of ``tensors`` may have changed.  Noticed on their own: eager in-place updates of a tensor (its
+    version counter) and eager in-place updates of the flat parameter a tensor is a view of
+    (``distributed.GradientBucket.flatten_parameters`` records it on the view as ``_dab_flat_param``: a view made with
+    ``p.data = ...`` keeps its own version counter, so an optimizer step on the flat parameter moves no per-tensor
+    version).  Everything else - raw ``.data`` writes, updates replayed from a CUDA graph - must be declared with
+    ``bump_weight_generation``."""
+    key = []
+    for t in tensors:
+        flat = getattr(t, "_dab_flat_param", None)
+        key.append((t.data_ptr(), t._version, -1 if flat is None else flat._version))
+    key.append(_weight_generation)
+    return tuple(key)
 
 
 def lib():

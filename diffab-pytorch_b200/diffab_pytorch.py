@@ -496,7 +496,7 @@ class PairEmbedding(nn.Module):
               self.distance_embedding[0].weight, self.distance_embedding[0].bias, self.distance_embedding[2].weight,
               self.distance_embedding[2].bias, self.mlp[0].weight, self.mlp[0].bias, self.mlp[2].weight,
               self.mlp[2].bias, self.mlp[4].weight, self.mlp[4].bias)
-        key = tuple((w.data_ptr(), w._version) for w in ws) + (_lib.weight_generation(),)
+        key = _lib.weight_key(ws)
         if getattr(self, "_packed", None) is None or self._packed[0] != key:
             buf = _lib.aligned_empty(lib.dab_pair_embed_packed_bytes(), xyz.device)
             wd = [_lib.dev(w.detach(), torch.float32, "pair embedding weight") for w in ws]
@@ -934,7 +934,7 @@ class InvariantPointAttentionLayer(nn.Module):
 
     def _packed_weights(self, dims):
         ws = self._weights()
-        key = tuple((w.data_ptr(), w._version) for w in ws) + (_lib.weight_generation(),)
+        key = _lib.weight_key(ws)
         # While a training step is being captured into a CUDA graph (distributed.GraphedTrainStep): always repack, so that
         # the pack is part of the graph - its replays follow optimizer steps that no Python-side version counter sees.
         capturing = (_lib.repack_when_capturing and torch.is_grad_enabled() and ws[0].is_cuda
@@ -1701,17 +1701,16 @@ class DiffAb(nn.Module):
     def _sample_graphed(self, s, x, O, res_ctx, pair_ctx, generation_mask, t_start, t_stop, noises=None, valid_len=None):
         """Reverse steps captured in CUDA graphs and replayed; the step index lives in a device tensor.
         The graphs work on static buffers (state, context, mask, pair-bias planes, noise) and are cached per shape and
-        weight generation, so repeated ``sample()`` calls only copy their context in (~1 GB device-to-device, well
+        ``_lib.weight_key``, so repeated ``sample()`` calls only copy their context in (~1 GB device-to-device, well
         under a millisecond).  Two step graphs: one reverse step, and a block of ``graph_block_steps`` consecutive
         steps; each reads its random draws from static buffers that a small companion graph redraws before every
         replay - or that the caller's ``noises`` are copied into (injected draws, parity tests)."""
         B, L = s.shape
         dev = s.device
-        # the captured graphs bake in packed weights and per-run weight products: recapture when any parameter changed
-        # (in-place updates bump _version; updates replayed from a CUDA graph bump the library-wide weight generation)
-        wkey = tuple((p.data_ptr(), p._version) for p in self.denoiser.parameters())
-        key = (B, L, tuple(res_ctx.shape), tuple(pair_ctx.shape), pair_ctx.dtype, str(dev), wkey,
-               _lib.weight_generation())
+        # the captured graphs bake in packed weights and per-run weight products: recapture when any parameter may have
+        # changed (see _lib.weight_key for which updates are noticed on their own)
+        key = (B, L, tuple(res_ctx.shape), tuple(pair_ctx.shape), pair_ctx.dtype, str(dev),
+               _lib.weight_key(self.denoiser.parameters()))
         cache = getattr(self, "_graph_cache", None)
         fresh = cache is None or cache["key"] != key
         if fresh:
@@ -1797,9 +1796,10 @@ class DiffAb(nn.Module):
 
     def invalidate_weight_caches(self):
         """Forget every weight-derived cache (packed bf16 weights, glue constants, captured sampling graphs).  Needed after
-        weight updates PyTorch cannot see - optimizer steps replayed from a CUDA graph, raw ``.data`` writes: in-place
-        updates made eagerly bump the parameters' version counters and are noticed without this call.
-        ``distributed.GraphedTrainStep`` calls the library-wide equivalent (``_lib.bump_weight_generation``)."""
+        weight updates PyTorch cannot see - raw ``.data`` writes, optimizer steps replayed from a CUDA graph outside
+        ``distributed.GraphedTrainStep`` (which calls the library-wide equivalent, ``_lib.bump_weight_generation``, at
+        every replay).  Noticed without this call: eager in-place updates of the parameters, and eager optimizer steps on
+        the flat parameter of ``GradientBucket.flatten_parameters`` (``torch.optim`` optimizers and ``FlatAdam``)."""
         _lib.bump_weight_generation()
         self._graph_cache = None
 

@@ -96,7 +96,13 @@ class GradientBucket:
         optimizer built over ``[that parameter]`` updates all weights in one elementwise pass (PyTorch's fused Adam walks
         the 106 small tensors chunk by chunk: ~165 us per step against ~10 us).  Call it BEFORE constructing the optimizer,
         and only with elementwise optimizers (Adam / AdamW / SGD: the update of an element depends on that element alone,
-        so the result is the per-tensor one, bit for bit)."""
+        so the result is the per-tensor one, bit for bit).
+
+        An in-place update of the flat parameter moves neither the version counter nor the data pointer of any parameter,
+        so each parameter records the flat parameter (``_dab_flat_param``) and ``_lib.weight_key``, the key of the packed
+        weights and captured sampling graphs, includes its version: eager optimizer steps on it need no
+        ``DiffAb.invalidate_weight_caches()``.  Raw writes (``flat_param.data``, a pointer handed to a kernel) must bump
+        it themselves (``torch.autograd.graph.increment_version``, as ``FlatAdam`` does) or call that method."""
         flat_p = torch.empty_like(self.flat)
         off = 0
         with torch.no_grad():
@@ -107,6 +113,8 @@ class GradientBucket:
                 off += n
         self.flat_param = torch.nn.Parameter(flat_p, requires_grad=True)
         self.flat_param.grad = self.flat
+        for p in self.params:
+            p._dab_flat_param = self.flat_param
         return self.flat_param
 
     def zero(self):
@@ -160,6 +168,8 @@ class FlatAdam:
                                             _lib.ptr(self.exp_avg_sq), _lib.ptr(self.step_count), float(g["lr"]),
                                             float(g["betas"][0]), float(g["betas"][1]), float(g["eps"]),
                                             float(g["weight_decay"]), p.numel(), _lib.stream_ptr()), "dab_adam_flat")
+        # the kernel writes through a raw pointer: mark the update so weight-derived caches see it (_lib.weight_key)
+        torch.autograd.graph.increment_version(p)
 
     def state_dict(self):
         return {"step": self.step_count.clone(), "exp_avg": self.exp_avg.clone(), "exp_avg_sq": self.exp_avg_sq.clone(),

@@ -130,3 +130,35 @@ def test_flat_parameter_optimizer_equals_the_per_tensor_one():
     # a checkpoint loads in place: the views stay views of the flat buffer
     flat.load_state_dict(ref.state_dict())
     assert flat[0].weight.data_ptr() == fp.data_ptr()
+
+
+def test_weight_key_follows_optimizer_steps_on_the_flat_parameter():
+    """_lib.weight_key decides when packed weights and captured sampling graphs are rebuilt.  An optimizer step on the
+    flat parameter of flatten_parameters() changes every weight but no per-parameter version or data pointer: the key
+    must change all the same, and must stay put while nothing changes."""
+    from diffab_pytorch_b200 import _lib
+    torch.manual_seed(0)
+    model = torch.nn.Sequential(torch.nn.Linear(5, 7), torch.nn.ReLU(), torch.nn.Linear(7, 3))
+    bucket = dd.GradientBucket(model.parameters())
+    fp = bucket.flatten_parameters()
+    opt = torch.optim.Adam([fp], lr=1e-3)
+    params = list(model.parameters())
+    key = _lib.weight_key(params)
+    assert _lib.weight_key(params) == key
+    for _ in range(2):
+        before = [p.detach().clone() for p in params]
+        versions, ptrs = [p._version for p in params], [p.data_ptr() for p in params]
+        dd.ddp_step(lambda: (model(torch.randn(6, 5)).pow(2).sum(), torch.tensor(1.0)), bucket, opt)
+        assert all(not torch.equal(a, p) for a, p in zip(before, params))
+        assert [p._version for p in params] == versions and [p.data_ptr() for p in params] == ptrs
+        new = _lib.weight_key(params)
+        assert new != key
+        assert _lib.weight_key(params) == new
+        key = new
+    # in-place updates of one parameter and declared updates change it too
+    with torch.no_grad():
+        params[0].mul_(2.0)
+    assert _lib.weight_key(params) != key
+    key = _lib.weight_key(params)
+    _lib.bump_weight_generation()
+    assert _lib.weight_key(params) != key
