@@ -152,7 +152,9 @@ static int launch_gemm_tn(const void* A, int64_t lda, const void* Bm, int64_t ld
   if (splits > n_chunks / 4) splits = n_chunks / 4 > 0 ? n_chunks / 4 : 1;
   const int per = (n_chunks + splits - 1) / splits;
   splits = (n_chunks + per - 1) / per;
-  if (!accumulate && cudaMemsetAsync(C, 0, (size_t)M * ldc * sizeof(float), stream) != cudaSuccess)
+  // only the M x N block: with ldc > N the columns N..ldc-1 of each row belong to the caller (C may be a column block)
+  if (!accumulate &&
+      cudaMemset2DAsync(C, (size_t)ldc * sizeof(float), 0, (size_t)N * sizeof(float), (size_t)M, stream) != cudaSuccess)
     return check_launch("gemm_tn memset");
   dim3 grid(N / BN, (M + kTnBM - 1) / kTnBM, splits);
   gemm_tn_bf16_kernel<BN><<<grid, 128, TnSmem<BN>::kTotal, stream>>>(ma, mb, C, ldc, M, per, n_chunks);
@@ -219,7 +221,9 @@ using namespace dab::sm100;
 extern "C" {
 
 /* C[M,N] (fp32, overwritten) = A[K,M]^T B[K,N]: bf16 operands with the contraction index as their ROW index (activations
- * as they lie in memory, one row per residue); K % 64 == 0, N % 64 == 0, M % 8 == 0 (TMA row pitch), any M otherwise.
+ * as they lie in memory, one row per residue); K % 64 == 0, N % 64 == 0, lda % 8 == 0 and ldb % 8 == 0 (TMA row pitch:
+ * a multiple of 16 bytes), ldc % 4 == 0, lda >= M, ldb >= N, ldc >= N, any M > 0 otherwise.  Only the M x N block of C
+ * is written: columns N..ldc-1 are left alone, so C may be a column block of a wider matrix.
  * Split over K across CTAs, partial tiles added with red.global (summation order not fixed: last-bit differences
  * between runs).  Autograd weight gradients of the nn.Linear layers, diffab_pytorch.py:391-408,464. */
 int dab_gemm_bf16_tn(const void* A, int64_t lda, const void* Bm, int64_t ldb, float* C, int64_t ldc, int M, int N, int K,

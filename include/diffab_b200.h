@@ -317,7 +317,7 @@ int dab_pair_zero_masked(void* x_bf16, const uint8_t* res_mask, int B, int L, vo
 int dab_pair_table_grad_sm100(const void* g1_bf16, const int64_t* seq_masked, const int64_t* residue_idx,
                               const int64_t* chain_idx, int B, int L, int max_dist, float* s_type, float* s_rel, void* stream);
 /* out_bf16[n] = sum of n_src (1..8) bf16 tensors, fp32 accumulation, one pass: the pair-tensor gradients of the IPA layers
- * (autograd would add them pairwise, five passes and five bf16 roundings for six layers). */
+ * (autograd would add them pairwise, five passes and five bf16 roundings for six layers).  out may be one of the sources. */
 int dab_sum_bf16(const void* const* src, int n_src, int64_t n, void* out_bf16, void* stream);
 /* ReLU backward of a 64-channel bf16 layer fused with its bias gradient: g_out = g_in where y > 0 else 0 (may alias g_in),
  * colsum[64] += column sums of g_out. */
@@ -365,7 +365,8 @@ int dab_adam_flat(float* p, const float* g, float* m, float* v, const float* ste
 int dab_gemm_bf16(const void* A, const void* Bm, float* C, const float* bias, int M, int N, int K, void* stream);
 /* C[M,N] (fp32, overwritten) = A[K,M]^T B[K,N]: bf16 operands whose ROW index is the contraction index (activations as
  * they lie in memory, one row per residue), read MN-major by tcgen05 - no transposed copies.  Split over K, partial tiles
- * added with red.global (summation order not fixed).  K % 64 == 0, N % 64 == 0, lda / ldb % 8 == 0.  The autograd weight
+ * added with red.global (summation order not fixed).  K % 64 == 0, N % 64 == 0, lda % 8 == 0, ldb % 8 == 0, ldc % 4 == 0,
+ * lda >= M, ldb >= N, ldc >= N, any M > 0; only the M x N block of C is written (C may be a column block).  The autograd weight
  * gradients of the nn.Linear layers of diffab_pytorch.py:391-408,464 (dWout = dy^T cat, dWcat = dproj^T x). */
 int dab_gemm_bf16_tn(const void* A, int64_t lda, const void* Bm, int64_t ldb, float* C, int64_t ldc, int M, int N, int K,
                      void* stream);
