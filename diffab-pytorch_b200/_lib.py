@@ -61,11 +61,12 @@ EXPORTS = {
     "dab_igso3_sample": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p,
                                  c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_void_p]),
     "dab_forward_noise": (c_int, [POINTER(DabSchedule), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
-                                  c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                  c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                                   c_void_p]),
     "dab_seq_probs": (c_int, [POINTER(DabSchedule), c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                               c_void_p, c_void_p]),
-    "dab_reverse_step": (c_int, [POINTER(DabSchedule)] + [c_void_p] * 8 + [c_int, c_int] + [c_void_p] * 8),
+    "dab_reverse_step": (c_int, [POINTER(DabSchedule)] + [c_void_p] * 8 + [c_int, c_int] + [c_void_p] * 3 + [c_int] +
+                         [c_void_p] * 5),
     "dab_ipa_f32_workspace_bytes": (c_size_t, [POINTER(DabIpaDims), c_int]),
     "dab_ipa_fwd_f32": (c_int, [POINTER(DabIpaDims), POINTER(DabIpaWeights), c_void_p, c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
@@ -114,8 +115,8 @@ EXPORTS = {
     "dab_pair_table_grad_sm100": (c_int, [c_void_p] * 4 + [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "dab_pair_mlp_fwd_train_sm100": (c_int, [c_void_p] * 10 + [c_int, c_int, c_int] + [c_void_p] * 6),
     "dab_pair_mlp_bwd_layer_sm100": (c_int, [c_void_p] * 4 + [c_int, c_int] + [c_void_p] * 5),
-    "dab_losses_fwd": (c_int, [c_void_p] * 7 + [c_int64, c_void_p, c_void_p, c_void_p]),
-    "dab_losses_bwd": (c_int, [c_void_p] * 7 + [c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "dab_losses_fwd": (c_int, [c_void_p] * 7 + [c_int64, c_int, c_void_p, c_void_p, c_void_p]),
+    "dab_losses_bwd": (c_int, [c_void_p] * 7 + [c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "dab_adam_flat": (c_int, [c_void_p] * 5 + [c_float] * 5 + [c_int64, c_void_p]),
     "dab_cast_f32_to_bf16": (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
     "dab_out_heads_fwd_sm100": (c_int, [c_void_p] * 5 + [c_int, c_int] + [c_void_p] * 4),

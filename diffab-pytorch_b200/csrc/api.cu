@@ -40,7 +40,7 @@ __global__ void __launch_bounds__(256) cast_bf16_kernel(const float4* __restrict
 
 extern "C" {
 
-int dab_version(void) { return 100; /* 0.1.0 */ }
+int dab_version(void) { return 101; /* 0.1.1: `generate` bits of the diffusion and loss entry points */ }
 
 const char* dab_last_error(void) { return dab::g_error; }
 

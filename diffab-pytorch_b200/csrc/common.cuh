@@ -47,6 +47,13 @@ inline bool aligned32(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
     }                                 \
   } while (0)
 
+// `generate` argument of the diffusion and loss entry points: DAB_GEN_SEQUENCE | DAB_GEN_STRUCTURE, at least one bit
+inline int check_generate(int generate, const char* what) {
+  DAB_REQUIRE(generate >= 1 && generate <= (DAB_GEN_SEQUENCE | DAB_GEN_STRUCTURE), DAB_EINVAL,
+              "%s: generate must be 1 (sequence), 2 (structure) or 3 (both), got %d", what, generate);
+  return DAB_OK;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

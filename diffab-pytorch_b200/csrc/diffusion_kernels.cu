@@ -26,7 +26,7 @@ __device__ __forceinline__ float mix_prob(bool hot, float w_keep, float w_noise,
 __global__ void __launch_bounds__(128) forward_noise_kernel(
     Sched sc, const int64_t* __restrict__ seq0, const float* __restrict__ x0, const float* __restrict__ O0,
     const uint8_t* __restrict__ mask, const int64_t* __restrict__ t, int B, int L,
-    const float* __restrict__ seq_exp, const float* __restrict__ eps, const float* __restrict__ rotvec,
+    const float* __restrict__ seq_exp, const float* __restrict__ eps, const float* __restrict__ rotvec, int generate,
     int64_t* __restrict__ seq_t, float* __restrict__ posterior, float* __restrict__ x_t, float* __restrict__ O_t) {
   __shared__ float s_v[128 * DAB_VOCAB];   // exponential draws in, posterior out
   __shared__ float s_o[128 * 9];           // O_0 in, O_t out
@@ -49,12 +49,13 @@ __global__ void __launch_bounds__(128) forward_noise_kernel(
     int tt = (int)t[b];
   if (tt < 0 || tt > sc.T) asm volatile("trap;");   // out-of-range timestep: the reference raises IndexError
     bool gen = mask[r] != 0;
+    bool gen_seq = gen && (generate & DAB_GEN_SEQUENCE), gen_str = gen && (generate & DAB_GEN_STRUCTURE);
     int s0 = (int)seq0[r];
 
     // ---- sequence: s_t ~ Multinomial(abar_t onehot + (1-abar_t)/21)   diffusion.py:105-158
     float ab = __ldg(sc.alpha_bar + tt);
     float one_m_ab = __fsub_rn(1.0f, ab);
-    int st = argmax_ratio([&](int k) { return mix_prob(k == s0, ab, one_m_ab, gen); }, s_v + tid * DAB_VOCAB);
+    int st = argmax_ratio([&](int k) { return mix_prob(k == s0, ab, one_m_ab, gen_seq); }, s_v + tid * DAB_VOCAB);
     seq_t[r] = st;
     // ---- posterior q(s_{t-1} | s_t, s_0) ∝ p_single(s_t, t) * p_from_t0(s_0, t-1)   diffusion.py:168-192
     float beta = __ldg(sc.beta + tt);
@@ -67,7 +68,7 @@ __global__ void __launch_bounds__(128) forward_noise_kernel(
     float sum = 0.f;
 #pragma unroll
     for (int k = 0; k < DAB_VOCAB; ++k) {
-      p[k] = __fmul_rn(mix_prob(k == st, one_m_beta, beta, gen), mix_prob(k == s0, abm, one_m_abm, gen));
+      p[k] = __fmul_rn(mix_prob(k == st, one_m_beta, beta, gen_seq), mix_prob(k == s0, abm, one_m_abm, gen_seq));
       sum = __fadd_rn(sum, p[k]);
     }
 #pragma unroll
@@ -79,10 +80,10 @@ __global__ void __launch_bounds__(128) forward_noise_kernel(
     for (int c = 0; c < 3; ++c) {
       float v0 = s_x[tid * 3 + c];
       float v = __fadd_rn(__fmul_rn(a, v0), __fmul_rn(s, s_e[tid * 3 + c]));
-      s_x[tid * 3 + c] = gen ? v : v0;
+      s_x[tid * 3 + c] = gen_str ? v : v0;
     }
     // ---- orientations: O_t = scale_rot(O_0, sqrt(abar)) @ exp(rotvec)   diffusion.py:280-292
-    if (gen) {
+    if (gen_str) {
       float R0[9], Rm[9], Rn[9], Ro[9];
 #pragma unroll
       for (int c = 0; c < 9; ++c) R0[c] = s_o[tid * 9 + c];
@@ -143,12 +144,12 @@ __global__ void __launch_bounds__(128) reverse_step_kernel(
     Sched sc, const int64_t* seq_t, const float* x_t, const float* O_t,  // may alias the outputs (in-place)
     const float* __restrict__ eps_theta, const float* __restrict__ v_theta, const float* __restrict__ seq_post,
     const uint8_t* __restrict__ mask, const int64_t* __restrict__ t, int B, int L,
-    const float* __restrict__ seq_exp, const float* __restrict__ z, const float* __restrict__ rotvec,
+    const float* __restrict__ seq_exp, const float* __restrict__ z, const float* __restrict__ rotvec, int generate,
     int64_t* seq_out, float* x_out, float* O_out, float* O0_out) {
   int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= (int64_t)B * L) return;
   reverse_update_residue(sc, r, (int)t[r / L], seq_t, x_t, O_t, eps_theta, v_theta, seq_post, mask, seq_exp, z, rotvec + r * 3,
-                         seq_out, x_out, O_out, O0_out);
+                         generate, seq_out, x_out, O_out, O0_out);
 }
 
 static int check_sched(const DabSchedule* s, Sched& out, const char* name) {
@@ -166,16 +167,18 @@ extern "C" {
 
 int dab_forward_noise(const DabSchedule* sched, const int64_t* seq0, const float* x0, const float* O0,
                       const uint8_t* mask, const int64_t* t, int B, int L, const float* seq_exp, const float* eps,
-                      const float* rotvec, int64_t* seq_t, float* posterior, float* x_t, float* O_t, void* stream) {
+                      const float* rotvec, int generate, int64_t* seq_t, float* posterior, float* x_t, float* O_t,
+                      void* stream) {
   Sched sc;
   if (int rc = check_sched(sched, sc, "dab_forward_noise")) return rc;
+  if (int rc = check_generate(generate, "dab_forward_noise")) return rc;
   DAB_REQUIRE(B >= 0 && L >= 0, DAB_EINVAL, "dab_forward_noise: negative size");
   if ((int64_t)B * L == 0) return DAB_OK;
   DAB_REQUIRE(seq0 && x0 && O0 && mask && t && seq_exp && eps && rotvec && seq_t && posterior && x_t && O_t,
               DAB_EINVAL, "dab_forward_noise: null pointer");
   int64_t n = (int64_t)B * L;
   forward_noise_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
-      sc, seq0, x0, O0, mask, t, B, L, seq_exp, eps, rotvec, seq_t, posterior, x_t, O_t);
+      sc, seq0, x0, O0, mask, t, B, L, seq_exp, eps, rotvec, generate, seq_t, posterior, x_t, O_t);
   count_launch();
   return check_launch("dab_forward_noise");
 }
@@ -197,9 +200,10 @@ int dab_seq_probs(const DabSchedule* sched, int kind, const int64_t* seq, const 
 int dab_reverse_step(const DabSchedule* sched, const int64_t* seq_t, const float* x_t, const float* O_t,
                      const float* eps_theta, const float* v_theta, const float* seq_post, const uint8_t* mask,
                      const int64_t* t, int B, int L, const float* seq_exp, const float* z, const float* rotvec,
-                     int64_t* seq_out, float* x_out, float* O_out, float* O0_out, void* stream) {
+                     int generate, int64_t* seq_out, float* x_out, float* O_out, float* O0_out, void* stream) {
   Sched sc;
   if (int rc = check_sched(sched, sc, "dab_reverse_step")) return rc;
+  if (int rc = check_generate(generate, "dab_reverse_step")) return rc;
   DAB_REQUIRE(B >= 0 && L >= 0, DAB_EINVAL, "dab_reverse_step: negative size");
   if ((int64_t)B * L == 0) return DAB_OK;
   DAB_REQUIRE(seq_t && x_t && O_t && eps_theta && v_theta && seq_post && mask && t && seq_exp && z && rotvec &&
@@ -207,8 +211,8 @@ int dab_reverse_step(const DabSchedule* sched, const int64_t* seq_t, const float
               DAB_EINVAL, "dab_reverse_step: null pointer");
   int64_t n = (int64_t)B * L;
   reverse_step_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
-      sc, seq_t, x_t, O_t, eps_theta, v_theta, seq_post, mask, t, B, L, seq_exp, z, rotvec, seq_out, x_out, O_out,
-      O0_out);
+      sc, seq_t, x_t, O_t, eps_theta, v_theta, seq_post, mask, t, B, L, seq_exp, z, rotvec, generate, seq_out, x_out,
+      O_out, O0_out);
   count_launch();
   return check_launch("dab_reverse_step");
 }

@@ -26,33 +26,37 @@ __device__ __forceinline__ void loss_rot_discrepancy(const float* P, const float
 __global__ void __launch_bounds__(128) losses_fwd_kernel(const float* __restrict__ post_pred, const float* __restrict__ post_tgt,
                                                          const float* __restrict__ eps_pred, const float* __restrict__ eps_tgt,
                                                          const float* __restrict__ O_pred, const float* __restrict__ O_true,
-                                                         const uint8_t* __restrict__ mask, int64_t n, float* __restrict__ acc,
-                                                         float* __restrict__ out) {
+                                                         const uint8_t* __restrict__ mask, int64_t n, int generate,
+                                                         float* __restrict__ acc, float* __restrict__ out) {
   const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   float v[4] = {0.f, 0.f, 0.f, 0.f};
   if (r < n && mask[r]) {
-    float s = 0.f;
-    for (int k = 0; k < LOSS_V; ++k) {
-      const float t = post_tgt[r * LOSS_V + k], p = post_pred[r * LOSS_V + k];
-      s += (t > 0.f ? t * logf(t) : 0.f) - t * logf(p);          // xlogy(t, t) - t * log p
+    if (generate & DAB_GEN_SEQUENCE) {
+      float s = 0.f;
+      for (int k = 0; k < LOSS_V; ++k) {
+        const float t = post_tgt[r * LOSS_V + k], p = post_pred[r * LOSS_V + k];
+        s += (t > 0.f ? t * logf(t) : 0.f) - t * logf(p);          // xlogy(t, t) - t * log p
+      }
+      v[0] = s;
     }
-    v[0] = s;
-    float q = 0.f;
+    if (generate & DAB_GEN_STRUCTURE) {
+      float q = 0.f;
 #pragma unroll
-    for (int c = 0; c < 3; ++c) {
-      const float d = eps_pred[r * 3 + c] - eps_tgt[r * 3 + c];
-      q = fmaf(d, d, q);
+      for (int c = 0; c < 3; ++c) {
+        const float d = eps_pred[r * 3 + c] - eps_tgt[r * 3 + c];
+        q = fmaf(d, d, q);
+      }
+      v[1] = q;
+      float P[9], T[9], D[9];
+#pragma unroll
+      for (int c = 0; c < 9; ++c) { P[c] = O_pred[r * 9 + c]; T[c] = O_true[r * 9 + c]; }
+      loss_rot_discrepancy(P, T, D);
+      float w = 0.f;
+#pragma unroll
+      for (int c = 0; c < 9; ++c) w = fmaf(D[c], D[c], w);
+      v[2] = w;
     }
-    v[1] = q;
-    float P[9], T[9], D[9];
-#pragma unroll
-    for (int c = 0; c < 9; ++c) { P[c] = O_pred[r * 9 + c]; T[c] = O_true[r * 9 + c]; }
-    loss_rot_discrepancy(P, T, D);
-    float w = 0.f;
-#pragma unroll
-    for (int c = 0; c < 9; ++c) w = fmaf(D[c], D[c], w);
-    v[2] = w;
-    v[3] = 1.f;
+    v[3] = 1.f;     // the count is the same in every mode
   }
   __shared__ float s_red[4][4];
   __shared__ bool s_last;
@@ -81,18 +85,20 @@ __global__ void __launch_bounds__(128) losses_fwd_kernel(const float* __restrict
 __global__ void __launch_bounds__(128) losses_bwd_kernel(const float* __restrict__ post_pred, const float* __restrict__ post_tgt,
                                                          const float* __restrict__ eps_pred, const float* __restrict__ eps_tgt,
                                                          const float* __restrict__ O_pred, const float* __restrict__ O_true,
-                                                         const uint8_t* __restrict__ mask, int64_t n, const float* __restrict__ g,
-                                                         const float* __restrict__ fwd_out, float* __restrict__ d_post,
-                                                         float* __restrict__ d_eps, float* __restrict__ d_O) {
+                                                         const uint8_t* __restrict__ mask, int64_t n, int generate,
+                                                         const float* __restrict__ g, const float* __restrict__ fwd_out,
+                                                         float* __restrict__ d_post, float* __restrict__ d_eps,
+                                                         float* __restrict__ d_O) {
   const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= n) return;
   const bool m = mask[r];
+  const bool ms = m && (generate & DAB_GEN_SEQUENCE), mx = m && (generate & DAB_GEN_STRUCTURE);   // launch-uniform bits
   const float inv = m ? 1.f / fwd_out[3] : 0.f;
   const float gs = g[0] * inv, gp = g[1] * inv, gr = g[2] * inv;
   for (int k = 0; k < LOSS_V; ++k)
-    d_post[r * LOSS_V + k] = m ? -gs * post_tgt[r * LOSS_V + k] / post_pred[r * LOSS_V + k] : 0.f;
+    d_post[r * LOSS_V + k] = ms ? -gs * post_tgt[r * LOSS_V + k] / post_pred[r * LOSS_V + k] : 0.f;
 #pragma unroll
-  for (int c = 0; c < 3; ++c) d_eps[r * 3 + c] = m ? 2.f * gp * (eps_pred[r * 3 + c] - eps_tgt[r * 3 + c]) : 0.f;
+  for (int c = 0; c < 3; ++c) d_eps[r * 3 + c] = mx ? 2.f * gp * (eps_pred[r * 3 + c] - eps_tgt[r * 3 + c]) : 0.f;
   float P[9], T[9], D[9];
 #pragma unroll
   for (int c = 0; c < 9; ++c) { P[c] = O_pred[r * 9 + c]; T[c] = O_true[r * 9 + c]; }
@@ -101,7 +107,7 @@ __global__ void __launch_bounds__(128) losses_bwd_kernel(const float* __restrict
   for (int i = 0; i < 3; ++i)
 #pragma unroll
     for (int j = 0; j < 3; ++j)       // d/dP_ij sum D^2 = 2 sum_k D_jk T_ik
-      d_O[r * 9 + i * 3 + j] = m ? 2.f * gr * (D[j * 3] * T[i * 3] + D[j * 3 + 1] * T[i * 3 + 1] + D[j * 3 + 2] * T[i * 3 + 2]) : 0.f;
+      d_O[r * 9 + i * 3 + j] = mx ? 2.f * gr * (D[j * 3] * T[i * 3] + D[j * 3 + 1] * T[i * 3 + 1] + D[j * 3 + 2] * T[i * 3 + 2]) : 0.f;
 }
 
 // Adam on one flat fp32 parameter vector (torch.optim.Adam with capturable=True, diffab_pytorch.py:925-931 of the
@@ -154,14 +160,16 @@ int dab_adam_flat(float* p, const float* g, float* m, float* v, const float* ste
 
 /* out[0..2] = (sequence KL, translation MSE, orientation) losses of DiffAb._shared_step (diffab_pytorch.py:856-880), each the
  * masked sum over the n = B*L residues divided by out[3] = the number of masked residues.  post_*[n,21], eps_*[n,3],
- * O_*[n,3,3] fp32; mask[n] uint8 = generation_mask & residue_mask; acc = 8 zeroed floats of scratch. */
+ * O_*[n,3,3] fp32; mask[n] uint8 = generation_mask & residue_mask; acc = 8 zeroed floats of scratch.  `generate` (DAB_GEN_*
+ * bits): a term of a modality that is not generated is exactly 0; the count is the same in every mode. */
 int dab_losses_fwd(const float* post_pred, const float* post_tgt, const float* eps_pred, const float* eps_tgt, const float* O_pred,
-                   const float* O_true, const uint8_t* mask, int64_t n, float* acc, float* out, void* stream) {
+                   const float* O_true, const uint8_t* mask, int64_t n, int generate, float* acc, float* out, void* stream) {
   DAB_REQUIRE(n > 0, DAB_EINVAL, "dab_losses_fwd: n must be positive");
+  if (int rc = check_generate(generate, "dab_losses_fwd")) return rc;
   DAB_REQUIRE(post_pred && post_tgt && eps_pred && eps_tgt && O_pred && O_true && mask && acc && out, DAB_EINVAL,
               "dab_losses_fwd: null pointer");
   losses_fwd_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(post_pred, post_tgt, eps_pred, eps_tgt, O_pred,
-                                                                                  O_true, mask, n, acc, out);
+                                                                                  O_true, mask, n, generate, acc, out);
   count_launch();
   return check_launch("dab_losses_fwd");
 }
@@ -169,13 +177,15 @@ int dab_losses_fwd(const float* post_pred, const float* post_tgt, const float* e
 /* Gradients of g[0]*seq + g[1]*pos + g[2]*rot with respect to the predicted posterior, epsilon and orientation
  * (d_post[n,21], d_eps[n,3], d_O[n,3,3]); fwd_out = the `out` of dab_losses_fwd (for the count). */
 int dab_losses_bwd(const float* post_pred, const float* post_tgt, const float* eps_pred, const float* eps_tgt, const float* O_pred,
-                   const float* O_true, const uint8_t* mask, int64_t n, const float* g, const float* fwd_out, float* d_post,
-                   float* d_eps, float* d_O, void* stream) {
+                   const float* O_true, const uint8_t* mask, int64_t n, int generate, const float* g, const float* fwd_out,
+                   float* d_post, float* d_eps, float* d_O, void* stream) {
   DAB_REQUIRE(n > 0, DAB_EINVAL, "dab_losses_bwd: n must be positive");
+  if (int rc = check_generate(generate, "dab_losses_bwd")) return rc;
   DAB_REQUIRE(post_pred && post_tgt && eps_pred && eps_tgt && O_pred && O_true && mask && g && fwd_out && d_post && d_eps && d_O,
               DAB_EINVAL, "dab_losses_bwd: null pointer");
   losses_bwd_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(post_pred, post_tgt, eps_pred, eps_tgt, O_pred,
-                                                                                  O_true, mask, n, g, fwd_out, d_post, d_eps, d_O);
+                                                                                  O_true, mask, n, generate, g, fwd_out, d_post, d_eps,
+                                                                                  d_O);
   count_launch();
   return check_launch("dab_losses_bwd");
 }

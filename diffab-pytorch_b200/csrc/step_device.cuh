@@ -25,18 +25,21 @@ __device__ __forceinline__ int argmax_ratio(F prob, const float* __restrict__ q)
 
 // Reverse step of residue r (patch b, timestep tt = t[b]); composition fixed by oracle/sampler.py (the reference has none).
 // `rv` = the residue's IGSO(3) rotation-vector draw (global or shared memory).  seq_t / x_t / O_t may alias the outputs.
+// `generate`: DAB_GEN_* bits.
 __device__ __forceinline__ void reverse_update_residue(
     const Sched& sc, int64_t r, int tt, const int64_t* seq_t, const float* x_t, const float* O_t,
     const float* __restrict__ eps_theta, const float* __restrict__ v_theta, const float* __restrict__ seq_post,
     const uint8_t* __restrict__ mask, const float* __restrict__ seq_exp, const float* __restrict__ z, const float* rv,
-    int64_t* seq_out, float* x_out, float* O_out, float* O0_out) {
+    int generate, int64_t* seq_out, float* x_out, float* O_out, float* O0_out) {
   if (tt < 0 || tt > sc.T) asm volatile("trap;");   // out-of-range timestep: the reference raises IndexError
   bool gen = mask[r] != 0;
+  // a modality the run does not generate keeps its old value (`generate` is uniform over the launch)
+  bool gen_seq = gen && (generate & DAB_GEN_SEQUENCE), gen_str = gen && (generate & DAB_GEN_STRUCTURE);
   bool noisy = tt > 1;
 
   // sequence
   int64_t s_old = seq_t[r];
-  if (gen) {
+  if (gen_seq) {
     const float* p = seq_post + r * DAB_VOCAB;
     seq_out[r] = argmax_ratio([&](int k) { return __ldg(p + k); }, seq_exp + r * DAB_VOCAB);
   } else {
@@ -52,7 +55,7 @@ __device__ __forceinline__ void reverse_update_residue(
     float xo = x_t[r * 3 + c];
     float v = __fadd_rn(__fmul_rn(__fsub_rn(xo, __fmul_rn(c_eps, __ldg(eps_theta + r * 3 + c))), inv_sa),
                         __fmul_rn(sig, __ldg(z + r * 3 + c)));
-    x_out[r * 3 + c] = gen ? v : xo;
+    x_out[r * 3 + c] = gen_str ? v : xo;
   }
   // orientations: O0 = O_t @ exp(v_theta)  (Denoiser tail, diffab_pytorch.py:594-596); O' = O0 @ exp(rotvec)
   float Rt[9], Re[9], R0[9];
@@ -64,7 +67,7 @@ __device__ __forceinline__ void reverse_update_residue(
 #pragma unroll
     for (int c = 0; c < 9; ++c) O0_out[r * 9 + c] = R0[c];
   }
-  if (gen) {
+  if (gen_str) {
     if (noisy) {
       float Rn[9], Ro[9];
       so3_exp(rv[0], rv[1], rv[2], Rn);

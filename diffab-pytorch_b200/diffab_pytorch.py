@@ -1361,7 +1361,7 @@ class _FusedLosses(torch.autograd.Function):
     ``dab_losses_bwd`` (gradients with respect to the three predictions only; targets are data)."""
 
     @staticmethod
-    def forward(ctx, post_pred, post_tgt, eps_pred, eps_tgt, o_pred, o_true, mask):
+    def forward(ctx, post_pred, post_tgt, eps_pred, eps_tgt, o_pred, o_true, mask, generate=3):
         f32 = torch.float32
         tensors = [_lib.dev(t.detach(), f32, n) for t, n in ((post_pred, "seq_posterior"), (post_tgt, "seq_posterior target"),
                                                              (eps_pred, "translations_eps"), (eps_tgt, "translations_eps target"),
@@ -1372,9 +1372,10 @@ class _FusedLosses(torch.autograd.Function):
             raise ValueError("fused losses: shapes must be (B, L, 21), (B, L, 3), (B, L, 3, 3) and a (B, L) mask")
         acc = torch.zeros(8, device=m.device, dtype=f32)
         out = torch.empty(4, device=m.device, dtype=f32)
-        _lib.check(_lib.lib().dab_losses_fwd(*(ptr(t) for t in tensors), ptr(m), n, ptr(acc), ptr(out), _lib.stream_ptr()),
-                   "dab_losses_fwd")
+        _lib.check(_lib.lib().dab_losses_fwd(*(ptr(t) for t in tensors), ptr(m), n, generate, ptr(acc), ptr(out),
+                                             _lib.stream_ptr()), "dab_losses_fwd")
         ctx.save_for_backward(*tensors, m, out)
+        ctx.generate = generate
         return out[0], out[1], out[2]
 
     @staticmethod
@@ -1383,9 +1384,9 @@ class _FusedLosses(torch.autograd.Function):
         zero = out.new_zeros(())
         g = torch.stack([x.to(out.dtype) if x is not None else zero for x in (g_seq, g_pos, g_rot)]).contiguous()
         d_post, d_eps, d_o = torch.empty_like(tensors[0]), torch.empty_like(tensors[2]), torch.empty_like(tensors[4])
-        _lib.check(_lib.lib().dab_losses_bwd(*(ptr(t) for t in tensors), ptr(m), m.numel(), ptr(g), ptr(out), ptr(d_post),
-                                             ptr(d_eps), ptr(d_o), _lib.stream_ptr()), "dab_losses_bwd")
-        return d_post, None, d_eps, None, d_o, None, None
+        _lib.check(_lib.lib().dab_losses_bwd(*(ptr(t) for t in tensors), ptr(m), m.numel(), ctx.generate, ptr(g), ptr(out),
+                                             ptr(d_post), ptr(d_eps), ptr(d_o), _lib.stream_ptr()), "dab_losses_bwd")
+        return d_post, None, d_eps, None, d_o, None, None, None
 
 
 # =============================================================================================
@@ -1393,7 +1394,16 @@ class _FusedLosses(torch.autograd.Function):
 # =============================================================================================
 class DiffAb(nn.Module):
     """diffab_pytorch.py:628-931.  ``device`` is where the schedules / IGSO(3) tables are built; they
-    follow ``.to()`` / ``.cuda()`` and are not part of the state dict (106 keys, as in the reference)."""
+    follow ``.to()`` / ``.cuda()`` and are not part of the state dict (106 keys, as in the reference).
+
+    Design mode: ``generate_sequence`` / ``generate_structure`` (plain attributes, not in the state dict) say which
+    modalities the masked residues generate in training and sampling.  Both True (default) is the reference's
+    sequence-structure co-design; sequence only is fixed-backbone sequence design; structure only is structure
+    prediction.  A modality that is not generated is shown to the context encoders on every residue, is neither noised
+    nor denoised, and adds nothing to the loss."""
+
+    generate_sequence = True
+    generate_structure = True
 
     def __init__(self, d_residue_emb, d_pair_emb, n_ipa_layers, d_scalar_per_head, n_query_point_per_head,
                  n_value_point_per_head, n_head, T=100, s=0.01, beta_max=0.999, n_atoms=15, aa_vocab_size=21,
@@ -1442,6 +1452,10 @@ class DiffAb(nn.Module):
             self._dsched = _lib.Schedule(self.sched, self._device)
         return self._dsched
 
+    def _generate(self):
+        """The ``generate`` bits of the fused kernels for the current design mode (ValueError if it generates nothing)."""
+        return _diffusion.generate_bits(self.generate_sequence, self.generate_structure)
+
     @property
     def so3_reverse(self):
         if self._so3_reverse is None:
@@ -1484,35 +1498,42 @@ class DiffAb(nn.Module):
         return self.denoiser(seq_idx_t, translations_t, orientations_t, res_context_emb, pair_context_emb, beta,
                              generation_mask, residue_mask)
 
-    def _add_noise(self, seq_idx_t0, translations_t0, orientations_t0, generation_mask, t, noise=None):
+    def _add_noise(self, seq_idx_t0, translations_t0, orientations_t0, generation_mask, t, noise=None, generate=3):
         """diffab_pytorch.py:778-806, fused (two launches).  ``noise`` = the six draws of
-        ``diffusion.draw_add_noise_tensors``; drawn on the device in that order when omitted."""
+        ``diffusion.draw_add_noise_tensors``; drawn on the device in that order when omitted (in every design mode).
+        ``generate`` (``diffusion.generate_bits``): a modality that is not generated is returned as given."""
         B, L = seq_idx_t0.shape
         if noise is None:
             noise = _diffusion.draw_add_noise_tensors(B, L, device=seq_idx_t0.device)
         return _diffusion.fused_add_noise(self.dsched, self.orientation_diffuser.so3, seq_idx_t0, translations_t0,
-                                          orientations_t0, generation_mask, t, noise)
+                                          orientations_t0, generation_mask, t, noise, generate=generate)
 
-    def _losses(self, denoised, noised, orientations_t0, generation_mask, residue_mask):
-        """diffab_pytorch.py:856-880.  On the GPU the three masked means are one fused kernel each way (SURVEY §8f N2)."""
+    def _losses(self, denoised, noised, orientations_t0, generation_mask, residue_mask, generate=3):
+        """diffab_pytorch.py:856-880.  On the GPU the three masked means are one fused kernel each way (SURVEY §8f N2).
+        ``generate`` (``diffusion.generate_bits``): the term of a modality that is not generated is exactly 0, with a zero
+        gradient; the denominator is the same in every mode."""
         if denoised["seq_posterior"].is_cuda and denoised["seq_posterior"].dtype == torch.float32:
             return _FusedLosses.apply(denoised["seq_posterior"], noised["seq_posterior"], denoised["translations_eps"],
                                       noised["translations_eps"], denoised["orientations_t0"], orientations_t0,
-                                      generation_mask & residue_mask)
+                                      generation_mask & residue_mask, generate)
         seq_loss = self.aa_loss(denoised["seq_posterior"].log(), noised["seq_posterior"])
         translations_loss = self.coordinate_loss(denoised["translations_eps"], noised["translations_eps"])
         orientations_loss = self.orientation_loss(denoised["orientations_t0"], orientations_t0)
         loss_mask = generation_mask & residue_mask
         denom = loss_mask.sum()
-        return ((seq_loss * loss_mask[..., None]).sum() / denom,
-                (translations_loss * loss_mask[..., None]).sum() / denom,
-                (orientations_loss * loss_mask[..., None, None]).sum() / denom)
+        seq_mask = loss_mask & bool(generate & _diffusion.GEN_SEQUENCE)
+        str_mask = loss_mask & bool(generate & _diffusion.GEN_STRUCTURE)
+        return ((seq_loss * seq_mask[..., None]).sum() / denom,
+                (translations_loss * str_mask[..., None]).sum() / denom,
+                (orientations_loss * str_mask[..., None, None]).sum() / denom)
 
     def _shared_step(self, batch, batch_idx, t=None, noise=None):
         """diffab_pytorch.py:808-880.  ``t`` / ``noise`` may be injected (tests); otherwise drawn on the
         device in the reference's order (#1 t, then the six noising draws).  ``self.train_precision``
         ("fp32" default, "bf16") picks the IPA path: with "bf16" the pair embedding is cast once per step and
-        the six IPA layers run forward and backward on the tensor-core kernels."""
+        the six IPA layers run forward and backward on the tensor-core kernels.  ``generate_sequence`` /
+        ``generate_structure`` pick the design mode (class docstring); the draws are the same in every mode."""
+        generate = self._generate()
         device = batch["generation_mask"].device
         bsz = batch["generation_mask"].size(0)
         if t is None:
@@ -1532,13 +1553,16 @@ class DiffAb(nn.Module):
             main, nside = torch.cuda.current_stream(device), _side_stream(device, 6)
             nside.wait_stream(main)
         with torch.cuda.stream(nside) if fork else contextlib.nullcontext():
-            noised = self._add_noise(seq_idx_t0, translations_t0, orientations_t0, generation_mask, t, noise=noise)
+            noised = self._add_noise(seq_idx_t0, translations_t0, orientations_t0, generation_mask, t, noise=noise,
+                                     generate=generate)
         self.pair_context_embedding.fused_rbf = bf16
         with _tf32_matmuls(bf16), _mixed_glue(bf16):   # mixed-precision step: the context encoders' GEMMs on the tensor cores too
             res_context_emb, pair_context_emb = self.encode_context(
                 seq_idx_t0, xyz_t0, orientations_t0, batch["backbone_dihedrals"], batch["distmat"],
                 batch["pairwise_dihedrals"], batch["atom_mask"], batch["chain_idx"], batch["residue_idx"],
-                batch["generation_mask"], batch["residue_mask"])
+                batch["generation_mask"], batch["residue_mask"],
+                generate_structure=bool(generate & _diffusion.GEN_STRUCTURE),
+                generate_sequence=bool(generate & _diffusion.GEN_SEQUENCE))
         if fork:
             main.wait_stream(nside)
             for v in noised.values():
@@ -1549,7 +1573,8 @@ class DiffAb(nn.Module):
             denoised = self.denoise(noised["seq_idx_t"], noised["translations_t"], noised["orientations_t"],
                                     res_context_emb, pair_context_emb, beta, batch["generation_mask"],
                                     batch["residue_mask"])
-        return self._losses(denoised, noised, batch["orientations"], batch["generation_mask"], batch["residue_mask"])
+        return self._losses(denoised, noised, batch["orientations"], batch["generation_mask"], batch["residue_mask"],
+                            generate=generate)
 
     def training_step(self, batch, batch_idx):
         seq_loss, translations_loss, orientations_loss = self._shared_step(batch, batch_idx)
@@ -1607,10 +1632,11 @@ class DiffAb(nn.Module):
 
     @torch.no_grad()
     def reverse_step(self, seq_idx_t, translations_t, orientations_t, res_context_emb, pair_context_emb,
-                     generation_mask, t, noise, inplace=False, pair_bias=None, glue_cache=None, beta=None):
+                     generation_mask, t, noise, inplace=False, pair_bias=None, glue_cache=None, beta=None, generate=3):
         """One reverse-diffusion step: epsilon network + fused update kernel.  ``t`` is (B,) int64.
         ``glue_cache`` (``Denoiser.sampling_cache``) switches the dense glue to its regrouped form; ``beta`` = the
-        schedule's beta at ``t`` when the caller has already gathered it."""
+        schedule's beta at ``t`` when the caller has already gathered it.  ``generate`` (``diffusion.generate_bits``):
+        a modality that is not generated keeps its value."""
         if beta is None:
             beta = self.dsched.tensors["beta"][t]
         rotvec = None
@@ -1631,7 +1657,7 @@ class DiffAb(nn.Module):
                                                    pair_context_emb, beta, pair_bias)
         return _diffusion.fused_reverse_step(self.dsched, self.so3_reverse, seq_idx_t, translations_t,
                                              orientations_t, eps, v_eps, post, generation_mask, t, noise,
-                                             inplace=inplace, rotvec=rotvec)
+                                             inplace=inplace, rotvec=rotvec, generate=generate)
 
     @torch.no_grad()
     def sample_from_context(self, seq_idx, translations, orientations, res_context_emb, pair_context_emb,
@@ -1639,7 +1665,9 @@ class DiffAb(nn.Module):
                             use_cuda_graph=False, _valid_len=None):
         """The reverse loop t_start..t_stop on resident tensors (this is what bench.py's ``value`` times).
         ``pair_context_emb`` may be fp32 (exact path) or bf16 (tensor-core path).  ``noises`` = {t: draws of step t}
-        (``draw_step_noise``) injects every random draw (parity tests); it works with and without CUDA graphs."""
+        (``draw_step_noise``) injects every random draw (parity tests); it works with and without CUDA graphs.
+        Only the modalities of the design mode (``generate_sequence`` / ``generate_structure``) change."""
+        generate = self._generate()
         T = self.T
         t_start = T if t_start is None else t_start
         L0 = seq_idx.shape[1]
@@ -1672,7 +1700,7 @@ class DiffAb(nn.Module):
         with _tf32_matmuls(pair_context_emb.dtype == torch.bfloat16):
             if use_cuda_graph and generator is None:
                 return self._sample_graphed(s, x, O, res_context_emb, pair_context_emb, generation_mask, t_start,
-                                            t_stop, noises, _valid_len)
+                                            t_stop, noises, _valid_len, generate)
             pair_bias = self._pair_bias_planes(pair_context_emb)
             if pair_bias is not None and _valid_len is not None:
                 _mask_padded_keys(pair_bias, _valid_len)
@@ -1681,7 +1709,7 @@ class DiffAb(nn.Module):
                 t = torch.full((B,), step, device=dev, dtype=torch.int64)
                 noise = noises[step] if noises is not None else self.draw_step_noise(B, L, dev, generator=generator)
                 out = self.reverse_step(s, x, O, res_context_emb, pair_context_emb, generation_mask, t, noise,
-                                        inplace=True, pair_bias=pair_bias, glue_cache=glue)
+                                        inplace=True, pair_bias=pair_bias, glue_cache=glue, generate=generate)
                 s, x, O = out["seq_idx"], out["translations"], out["orientations"]
             return {"seq_idx": s, "translations": x, "orientations": O}
 
@@ -1698,18 +1726,20 @@ class DiffAb(nn.Module):
         bufs["seq_exp"].exponential_(); bufs["z"].normal_(); bufs["axis"].normal_()
         bufs["hist_exp"].exponential_(); bufs["jitter"].uniform_(); bufs["gauss"].normal_()
 
-    def _sample_graphed(self, s, x, O, res_ctx, pair_ctx, generation_mask, t_start, t_stop, noises=None, valid_len=None):
+    def _sample_graphed(self, s, x, O, res_ctx, pair_ctx, generation_mask, t_start, t_stop, noises=None, valid_len=None,
+                        generate=3):
         """Reverse steps captured in CUDA graphs and replayed; the step index lives in a device tensor.
         The graphs work on static buffers (state, context, mask, pair-bias planes, noise) and are cached per shape and
         ``_lib.weight_key``, so repeated ``sample()`` calls only copy their context in (~1 GB device-to-device, well
         under a millisecond).  Two step graphs: one reverse step, and a block of ``graph_block_steps`` consecutive
         steps; each reads its random draws from static buffers that a small companion graph redraws before every
-        replay - or that the caller's ``noises`` are copied into (injected draws, parity tests)."""
+        replay - or that the caller's ``noises`` are copied into (injected draws, parity tests).  The ``generate`` bits of
+        the design mode are baked into the captured update kernels, so they are part of the cache key."""
         B, L = s.shape
         dev = s.device
         # the captured graphs bake in packed weights and per-run weight products: recapture when any parameter may have
         # changed (see _lib.weight_key for which updates are noticed on their own)
-        key = (B, L, tuple(res_ctx.shape), tuple(pair_ctx.shape), pair_ctx.dtype, str(dev),
+        key = (B, L, tuple(res_ctx.shape), tuple(pair_ctx.shape), pair_ctx.dtype, str(dev), generate,
                _lib.weight_key(self.denoiser.parameters()))
         cache = getattr(self, "_graph_cache", None)
         fresh = cache is None or cache["key"] != key
@@ -1738,14 +1768,15 @@ class DiffAb(nn.Module):
                 for _ in range(2):  # warm-up outside capture (allocator, lazy init, weight packing)
                     self._fill_noise_(st["noise1"])
                     self.reverse_step(st["s"].clone(), st["x"].clone(), st["O"].clone(), st["res"], st["pair"],
-                                      st["mask"], st["t"], st["noise1"], pair_bias=st["bias"], glue_cache=st["glue"])
+                                      st["mask"], st["t"], st["noise1"], pair_bias=st["bias"], glue_cache=st["glue"],
+                                      generate=generate)
             torch.cuda.current_stream(dev).wait_stream(side)
             draw, graph = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
             with torch.cuda.graph(draw):
                 self._fill_noise_(st["noise1"])
             with torch.cuda.graph(graph, pool=draw.pool()):
                 self.reverse_step(st["s"], st["x"], st["O"], st["res"], st["pair"], st["mask"], st["t"], st["noise1"],
-                                  inplace=True, pair_bias=st["bias"], glue_cache=st["glue"])
+                                  inplace=True, pair_bias=st["bias"], glue_cache=st["glue"], generate=generate)
                 st["t"].sub_(1)
             st["graph"], st["draw"] = graph, draw
             self._graph_cache = st
@@ -1769,7 +1800,7 @@ class DiffAb(nn.Module):
                 for u in range(U):
                     self.reverse_step(st["s"], st["x"], st["O"], st["res"], st["pair"], st["mask"], t_blk[u],
                                       {k: v[u] for k, v in noiseU.items()}, inplace=True, pair_bias=st["bias"],
-                                      glue_cache=st["glue"], beta=beta_blk[u])
+                                      glue_cache=st["glue"], beta=beta_blk[u], generate=generate)
                 st["t"].sub_(U)
             st["graph_block"] = (U, block, draw_block)
         st["s"].copy_(s); st["x"].copy_(x); st["O"].copy_(O)
@@ -1811,13 +1842,28 @@ class DiffAb(nn.Module):
     @torch.no_grad()
     def sample(self, seq_idx, xyz, orientations, backbone_dihedrals=None, distmat=None, pairwise_dihedrals=None,
                atom_mask=None, chain_idx=None, residue_idx=None, generation_mask=None, residue_mask=None,
-               generator=None, precision="bf16", use_cuda_graph=True, context_chunk=32, t_start=None, t_stop=1):
+               generator=None, precision="bf16", use_cuda_graph=True, context_chunk=32, t_start=None, t_stop=1,
+               init="prior"):
         """Reverse-diffusion sampling of the masked residues (the reference's stub, made real).
 
         Accepts host or device tensors (host tensors are copied to the model's device; pinned memory
         makes that asynchronous).  Features not given are derived: ``distmat`` from ``xyz`` on the
         device, masks default to "all residues valid / generation mask required".  Returns a dict
-        ``{seq_idx, translations, orientations}`` on the model's device."""
+        ``{seq_idx, translations, orientations}`` on the model's device.
+
+        Only the modalities of the design mode (``generate_sequence`` / ``generate_structure``) are generated; the
+        other one is context on every residue and comes back unchanged.  ``init="prior"`` starts the generated
+        residues from the t = T prior; ``init="native"`` (optimisation of an existing antibody) starts from the given
+        sequence and structure noised to step ``t_start`` (in [1, T], default T) by the forward process, then
+        denoises from there."""
+        generate = self._generate()
+        gen_seq, gen_str = bool(generate & _diffusion.GEN_SEQUENCE), bool(generate & _diffusion.GEN_STRUCTURE)
+        if init not in ("prior", "native"):
+            raise ValueError(f"sample(): init must be 'prior' or 'native', got {init!r}")
+        if init == "native":
+            t_start = self.T if t_start is None else t_start
+            if not 1 <= t_start <= self.T:
+                raise ValueError(f"sample(init='native'): t_start must be in [1, {self.T}], got {t_start}")
         dev = self._device
         mv = lambda v: None if v is None else v.to(dev, non_blocking=True)
         seq_idx, xyz, orientations = mv(seq_idx), mv(xyz), mv(orientations)
@@ -1847,37 +1893,49 @@ class DiffAb(nn.Module):
                 # pair context from one fused tcgen05 kernel (bf16, distances from xyz inside the kernel); the small
                 # residue encoder stays a PyTorch module
                 ctx_mask = residue_mask & (~generation_mask)
+                seq_ctx = ctx_mask if gen_seq else None        # encode_context's generate_* flags
                 res_ctx = self.residue_context_embedding(seq_idx, xyz, orientations, backbone_dihedrals, chain_idx,
-                                                         atom_mask, ctx_mask, ctx_mask)
+                                                         atom_mask, ctx_mask if gen_str else None, seq_ctx)
                 if L < Lp:    # ragged length: the fused kernel works on 128 / 256 residues - pad with absent residues, cut back
                     n = Lp - L
                     pad1 = lambda v: F.pad(v, (0, n))
                     pair_ctx = self.pair_context_embedding.forward_fused_bf16(
                         pad1(seq_idx), F.pad(xyz, (0, 0, 0, 0, 0, n)), F.pad(pairwise_dihedrals, (0, 0, 0, n, 0, n)),
-                        pad1(residue_idx), pad1(chain_idx), F.pad(atom_mask, (0, 0, 0, n)), pad1(ctx_mask))
+                        pad1(residue_idx), pad1(chain_idx), F.pad(atom_mask, (0, 0, 0, n)),
+                        None if seq_ctx is None else pad1(seq_ctx))
                     pair_ctx = pair_ctx[:, :L, :L].contiguous()
                 else:
                     pair_ctx = self.pair_context_embedding.forward_fused_bf16(seq_idx, xyz, pairwise_dihedrals, residue_idx,
-                                                                              chain_idx, atom_mask, ctx_mask)
+                                                                              chain_idx, atom_mask, seq_ctx)
             else:
                 for lo in range(0, B, context_chunk):
                     sl = slice(lo, min(B, lo + context_chunk))
                     dm = distmat[sl] if distmat is not None else derive(xyz[sl])
                     r, p = self.encode_context(seq_idx[sl], xyz[sl], orientations[sl], backbone_dihedrals[sl], dm,
                                                pairwise_dihedrals[sl], atom_mask[sl], chain_idx[sl], residue_idx[sl],
-                                               generation_mask[sl], residue_mask[sl], distmat_is_squared=distmat is None)
+                                               generation_mask[sl], residue_mask[sl], generate_structure=gen_str,
+                                               generate_sequence=gen_seq, distmat_is_squared=distmat is None)
                     res_parts.append(r)
                     pair_parts.append(cast_pair_to_bf16(p) if use_bf16 else p)
                 res_ctx, pair_ctx = torch.cat(res_parts), torch.cat(pair_parts)
-        # t = T prior on generated residues: s ~ U{0..20}, x ~ N(0, I), O ~ uniform SO(3)
-        from .synth import uniform_rotations
         m = generation_mask
-        sT = torch.randint(0, 21, (B, L), device=dev, generator=generator)
-        xT = torch.randn(B, L, 3, device=dev, generator=generator)
-        OT = uniform_rotations(B, L, generator=generator, device=dev)
         x0 = xyz[:, :, CA_IDX]
-        s = torch.where(m, sT, seq_idx)
-        x = torch.where(m[..., None], xT, x0)
-        O = torch.where(m[..., None, None], OT, orientations)
+        if init == "native":
+            # the native state noised to t_start on the generated modalities (the forward process of training)
+            noise = _diffusion.draw_add_noise_tensors(B, L, device=dev, generator=generator)
+            t = torch.full((B,), t_start, device=dev, dtype=torch.int64)
+            noised = self._add_noise(seq_idx, x0, orientations, m, t, noise=noise, generate=generate)
+            s, x, O = noised["seq_idx_t"], noised["translations_t"], noised["orientations_t"]
+        else:
+            # t = T prior on generated residues: s ~ U{0..20}, x ~ N(0, I), O ~ uniform SO(3); drawn in every mode,
+            # a modality that is not generated starts (and stays) at its native value
+            from .synth import uniform_rotations
+            sT = torch.randint(0, 21, (B, L), device=dev, generator=generator)
+            xT = torch.randn(B, L, 3, device=dev, generator=generator)
+            OT = uniform_rotations(B, L, generator=generator, device=dev)
+            ms, mx = m & gen_seq, m & gen_str
+            s = torch.where(ms, sT, seq_idx)
+            x = torch.where(mx[..., None], xT, x0)
+            O = torch.where(mx[..., None, None], OT, orientations)
         return self.sample_from_context(s, x, O, res_ctx, pair_ctx, m, generator=generator, t_start=t_start,
                                         t_stop=t_stop, use_cuda_graph=use_cuda_graph and generator is None)

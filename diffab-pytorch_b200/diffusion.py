@@ -14,6 +14,15 @@ from . import so3
 from ._lib import ptr
 
 V = 21  # diffusion.py:47 (``aa_vocab_size`` is ignored there)
+GEN_SEQUENCE, GEN_STRUCTURE = 1, 2   # ``generate`` bits of the fused kernels (DAB_GEN_* in include/diffab_b200.h)
+
+
+def generate_bits(generate_sequence, generate_structure):
+    """The ``generate`` argument of the fused kernels for a design mode: 3 co-design, 1 fixed-backbone sequence design,
+    2 structure prediction.  Generating neither modality is refused."""
+    if not (generate_sequence or generate_structure):
+        raise ValueError("generate_sequence and generate_structure are both False: nothing to generate")
+    return (GEN_SEQUENCE if generate_sequence else 0) | (GEN_STRUCTURE if generate_structure else 0)
 
 
 def cosine_variance_schedule(T, s=8e-3, beta_max=0.999):
@@ -150,9 +159,9 @@ def draw_add_noise_tensors(bsz, L, n_bins=8192, device="cuda", generator=None):
     }
 
 
-def fused_add_noise(dsched, so3_table, seq0, x0, O0, generation_mask, t, noise):
+def fused_add_noise(dsched, so3_table, seq0, x0, O0, generation_mask, t, noise, generate=3):
     """``DiffAb._add_noise`` (diffab_pytorch.py:778-806) as two launches: IGSO(3) sampler + one fused
-    per-residue kernel."""
+    per-residue kernel.  ``generate`` (``generate_bits``): a modality that is not generated comes back as its input."""
     seq0 = _lib.dev(seq0, torch.int64, "seq_idx_t0")
     x0 = _lib.dev(x0, torch.float32, "translations_t0")
     O0 = _lib.dev(O0, torch.float32, "orientations_t0")
@@ -168,16 +177,17 @@ def fused_add_noise(dsched, so3_table, seq0, x0, O0, generation_mask, t, noise):
     x_t = torch.empty(B, L, 3, device=dev, dtype=torch.float32)
     O_t = torch.empty(B, L, 3, 3, device=dev, dtype=torch.float32)
     _lib.check(_lib.lib().dab_forward_noise(dsched.ref(), ptr(seq0), ptr(x0), ptr(O0), ptr(m), ptr(t), B, L,
-                                            ptr(seq_exp), ptr(eps), ptr(rotvec), ptr(seq_t), ptr(post), ptr(x_t),
+                                            ptr(seq_exp), ptr(eps), ptr(rotvec), generate, ptr(seq_t), ptr(post), ptr(x_t),
                                             ptr(O_t), _lib.stream_ptr()), "dab_forward_noise")
     return {"seq_idx_t": seq_t, "seq_posterior": post, "translations_t": x_t, "translations_eps": eps,
             "orientations_t": O_t}
 
 
 def fused_reverse_step(dsched, so3_rev, seq_t, x_t, O_t, eps_theta, v_theta, seq_post, generation_mask, t, noise,
-                       inplace=False, return_O0=False, rotvec=None):
+                       inplace=False, return_O0=False, rotvec=None, generate=3):
     """Reverse step (oracle/sampler.py; not in the reference): IGSO(3) sampler + one fused kernel.  ``rotvec``: the step's
-    IGSO(3) draw when the caller has already made it (it depends on t and the noise only, not on the network)."""
+    IGSO(3) draw when the caller has already made it (it depends on t and the noise only, not on the network).
+    ``generate`` (``generate_bits``): a modality that is not generated keeps its old value."""
     seq_t = _lib.dev(seq_t, torch.int64, "seq_idx_t")
     x_t = _lib.dev(x_t, torch.float32, "translations_t")
     O_t = _lib.dev(O_t, torch.float32, "orientations_t")
@@ -199,7 +209,7 @@ def fused_reverse_step(dsched, so3_rev, seq_t, x_t, O_t, eps_theta, v_theta, seq
     O0 = torch.empty_like(O_t) if return_O0 else None
     _lib.check(_lib.lib().dab_reverse_step(dsched.ref(), ptr(seq_t), ptr(x_t), ptr(O_t), ptr(eps_theta), ptr(v_theta),
                                            ptr(seq_post), ptr(m), ptr(t), B, L, ptr(seq_exp), ptr(z), ptr(rotvec),
-                                           ptr(s_out), ptr(x_out), ptr(O_out), ptr(O0), _lib.stream_ptr()),
+                                           generate, ptr(s_out), ptr(x_out), ptr(O_out), ptr(O0), _lib.stream_ptr()),
                "dab_reverse_step")
     out = {"seq_idx": s_out, "translations": x_out, "orientations": O_out}
     if return_O0:

@@ -38,6 +38,12 @@ extern "C" {
 
 #define DAB_VOCAB 21 /* diffusion.py:47 (hard-coded there) */
 
+/* `generate` bits of dab_forward_noise, dab_reverse_step and dab_losses_fwd/bwd: which modalities the masked
+ * residues generate.  3 = co-design (the reference's training task), 1 = fixed-backbone sequence design,
+ * 2 = structure prediction; any other value is refused with DAB_EINVAL. */
+#define DAB_GEN_SEQUENCE 1
+#define DAB_GEN_STRUCTURE 2
+
 int dab_version(void);
 const char* dab_last_error(void);
 /* Number of kernels this library has launched in this process (bench.py's "gpu_launches" claim). */
@@ -83,10 +89,12 @@ typedef struct DabSchedule {
  * posterior_single_step (diffusion.py:137-192), CoordinateDiffuser.diffuse_from_t0 (:199-236),
  * OrientationDiffuser.diffuse_from_t0 (:262-294; `rotvec` is dab_igso3_sample's output).
  * mask[B,L] uint8 (bool); t[B] int64; seq_exp[B*L,21] Exp(1); eps[B,L,3] randn.
- * Outputs: seq_t[B,L] int64, posterior[B,L,21], x_t[B,L,3], O_t[B,L,3,3]. */
+ * Outputs: seq_t[B,L] int64, posterior[B,L,21], x_t[B,L,3], O_t[B,L,3,3].
+ * A modality whose DAB_GEN_* bit is clear is left as its input on every residue (s_t = s_0 with a
+ * one-hot posterior, x_t = x_0, O_t = O_0); the draws are read all the same. */
 int dab_forward_noise(const DabSchedule* sched, const int64_t* seq0, const float* x0, const float* O0,
                       const uint8_t* mask, const int64_t* t, int B, int L, const float* seq_exp,
-                      const float* eps, const float* rotvec, int64_t* seq_t, float* posterior,
+                      const float* eps, const float* rotvec, int generate, int64_t* seq_t, float* posterior,
                       float* x_t, float* O_t, void* stream);
 
 /* SequenceDiffuser.forward_prob_single_step / forward_prob_from_t0 / posterior_single_step
@@ -100,12 +108,13 @@ int dab_seq_probs(const DabSchedule* sched, int kind, const int64_t* seq, const 
  * (diffab_pytorch.py:594-596: O0 = O_t @ exp(v_theta)) with the three updates:
  *   s' = argmax(seq_post / seq_exp); x' = (x - beta/sqrt(1-abar) eps_theta)/sqrt(alpha) + sqrt(beta) z;
  *   O' = O0 @ exp(rotvec) (no noise at t = 1); each under where(mask, new, old).
- * O0_out may be NULL.  In-place (seq_out == seq_t etc.) is allowed. */
+ * A modality whose DAB_GEN_* bit in `generate` is clear keeps its old value on every residue, bit for bit
+ * (O0_out is written in every mode).  O0_out may be NULL.  In-place (seq_out == seq_t etc.) is allowed. */
 int dab_reverse_step(const DabSchedule* sched, const int64_t* seq_t, const float* x_t, const float* O_t,
                      const float* eps_theta, const float* v_theta, const float* seq_post,
                      const uint8_t* mask, const int64_t* t, int B, int L, const float* seq_exp,
-                     const float* z, const float* rotvec, int64_t* seq_out, float* x_out, float* O_out,
-                     float* O0_out, void* stream);
+                     const float* z, const float* rotvec, int generate, int64_t* seq_out, float* x_out,
+                     float* O_out, float* O0_out, void* stream);
 
 /* ------------------------------------------------------------------ invariant point attention */
 /* One InvariantPointAttentionLayer (diffab_pytorch.py:339-465, use_pair_bias=True).
@@ -348,12 +357,15 @@ int dab_pair_mlp_bwd_layer_sm100(const void* g_bf16, const void* a_bf16, const v
  * OrientationLoss :610-625, reduction "none", then masked mean; csrc/loss_kernels.cu).  n = B*L residues; post_*[n,21],
  * eps_*[n,3], O_*[n,3,3] fp32, mask[n] uint8 = generation_mask & residue_mask.  Forward: acc = 8 zeroed floats of scratch,
  * out[0..2] = sequence / translation / orientation loss, out[3] = number of masked residues.  Backward: g[3] = upstream
- * gradients of the three losses, fwd_out = the forward's out; writes d_post[n,21], d_eps[n,3], d_O[n,3,3]. */
+ * gradients of the three losses, fwd_out = the forward's out; writes d_post[n,21], d_eps[n,3], d_O[n,3,3].
+ * `generate` (DAB_GEN_* bits): the sequence term needs DAB_GEN_SEQUENCE, the translation and orientation terms need
+ * DAB_GEN_STRUCTURE; a term whose bit is clear is exactly 0 and so is its gradient.  The count out[3] is the same in
+ * every mode. */
 int dab_losses_fwd(const float* post_pred, const float* post_tgt, const float* eps_pred, const float* eps_tgt, const float* O_pred,
-                   const float* O_true, const uint8_t* mask, int64_t n, float* acc, float* out, void* stream);
+                   const float* O_true, const uint8_t* mask, int64_t n, int generate, float* acc, float* out, void* stream);
 int dab_losses_bwd(const float* post_pred, const float* post_tgt, const float* eps_pred, const float* eps_tgt, const float* O_pred,
-                   const float* O_true, const uint8_t* mask, int64_t n, const float* g, const float* fwd_out, float* d_post,
-                   float* d_eps, float* d_O, void* stream);
+                   const float* O_true, const uint8_t* mask, int64_t n, int generate, const float* g, const float* fwd_out,
+                   float* d_post, float* d_eps, float* d_O, void* stream);
 /* One Adam step (torch.optim.Adam semantics, the reference's configure_optimizers diffab_pytorch.py:925-931) on a FLAT fp32
  * parameter vector: p, m, v [n] updated in place from the gradient g [n] (n % 4 == 0, 16-byte aligned); `step` = device
  * scalar (float) with the step count including this step, incremented by the caller - no host state, graph-capturable. */

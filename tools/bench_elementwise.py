@@ -63,13 +63,13 @@ seq_t = torch.empty_like(seq); post = torch.empty(B, L, 21, device=dev); x_t = t
 sched = model.dsched
 m8 = mask.to(torch.uint8)
 fn = lambda: lib.dab_forward_noise(sched.ref(), ptr(seq), ptr(x0), ptr(O0), ptr(m8), ptr(t), B, L, ptr(noise["seq_exp"]),
-                                   ptr(noise["eps"]), ptr(rotvec), ptr(seq_t), ptr(post), ptr(x_t), ptr(O_t), _lib.stream_ptr())
+                                   ptr(noise["eps"]), ptr(rotvec), 3, ptr(seq_t), ptr(post), ptr(x_t), ptr(O_t), _lib.stream_ptr())
 rows.append(("forward_noise (DiffAb._add_noise, fused)", 317 * B * L, timed(fn)))
 eps = torch.randn(B, L, 3, device=dev, generator=g); vth = 0.1 * torch.randn(B, L, 3, device=dev, generator=g)
 z = torch.randn(B, L, 3, device=dev, generator=g)
 so = torch.empty_like(seq); xo = torch.empty_like(x0); Oo = torch.empty_like(O0)
 fn = lambda: lib.dab_reverse_step(sched.ref(), ptr(seq), ptr(x0), ptr(O0), ptr(eps), ptr(vth), ptr(post), ptr(m8), ptr(t), B, L,
-                                  ptr(noise["seq_exp"]), ptr(z), ptr(rotvec), ptr(so), ptr(xo), ptr(Oo), None, _lib.stream_ptr())
+                                  ptr(noise["seq_exp"]), ptr(z), ptr(rotvec), 3, ptr(so), ptr(xo), ptr(Oo), None, _lib.stream_ptr())
 rows.append(("reverse_step (fused update)", 330 * B * L, timed(fn)))
 
 print(f"{'kernel':44s} {'GB moved':>9s} {'ms':>8s} {'GB/s':>8s} {'of measured HBM peak':>22s}")
