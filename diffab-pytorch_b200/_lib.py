@@ -76,19 +76,13 @@ EXPORTS = {
     "dab_ipa_pack_weights": (c_int, [POINTER(DabIpaDims), POINTER(DabIpaWeights), c_void_p, c_void_p]),
     "dab_ipa_packed_layout": (c_int, [POINTER(DabIpaDims), POINTER(c_size_t)]),
     "dab_ipa_sm100_workspace_bytes": (c_size_t, [POINTER(DabIpaDims)]),
-    "dab_ipa_pair_bias": (c_int, [POINTER(DabIpaDims), c_void_p, c_void_p, c_void_p, c_void_p]),
     "dab_ipa_pair_bias_multi": (c_int, [POINTER(DabIpaDims), c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
-    "dab_ipa_fwd_sm100": (c_int, [POINTER(DabIpaDims), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
-                                  c_void_p, c_void_p, c_size_t, c_void_p]),
-    "dab_ipa_fwd_sm100_io": (c_int, [POINTER(DabIpaDims)] + [c_void_p] * 10 + [c_size_t, c_void_p]),
     "dab_ipa_mid_sm100": (c_int, [POINTER(DabIpaDims), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "dab_ipa_fwd_sm100_stages": (c_int, [POINTER(DabIpaDims)] + [c_void_p] * 10 + [c_size_t, c_int, c_void_p]),
     "dab_ipa_fwd_sm100_train": (c_int, [POINTER(DabIpaDims), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                         c_void_p, c_void_p, c_size_t, c_void_p]),
     "dab_ipa_sm100_workspace_layout": (c_int, [POINTER(DabIpaDims), POINTER(c_size_t)]),
     "dab_ipa_bwd_sm100_workspace_bytes": (c_size_t, [POINTER(DabIpaDims)]),
-    "dab_ipa_bwd_sm100": (c_int, [POINTER(DabIpaDims), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
-                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "dab_ipa_bwd_sm100_main": (c_int, [POINTER(DabIpaDims), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "dab_ipa_bwd_sm100_finish": (c_int, [POINTER(DabIpaDims), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
@@ -121,7 +115,6 @@ EXPORTS = {
     "dab_cast_f32_to_bf16": (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
     "dab_out_heads_fwd_sm100": (c_int, [c_void_p] * 5 + [c_int, c_int] + [c_void_p] * 4),
     "dab_ipa_front_proj_sm100": (c_int, [c_void_p] * 10 + [c_size_t, c_void_p]),
-    "dab_gemm_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "dab_gemm_bf16_tn": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int, c_int, c_int, c_void_p]),
     "dab_gemm_bf16_tn_acc": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int, c_int, c_int, c_void_p]),
     "dab_linear_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),

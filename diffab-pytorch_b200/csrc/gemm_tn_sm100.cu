@@ -220,6 +220,18 @@ using namespace dab::sm100;
 
 extern "C" {
 
+// dab_gemm_bf16_tn (accumulate = false) and dab_gemm_bf16_tn_acc (true); `fn` names the one called in the messages
+static int gemm_tn(const char* fn, const void* A, int64_t lda, const void* Bm, int64_t ldb, float* C, int64_t ldc, int M, int N,
+                   int K, void* stream, bool accumulate) {
+  DAB_REQUIRE(A && Bm && C, DAB_EINVAL, "%s: null pointer", fn);
+  DAB_REQUIRE(M > 0 && N > 0 && K > 0 && K % kTnKC == 0 && N % 64 == 0 && lda % 8 == 0 && ldb % 8 == 0 && ldc % 4 == 0 &&
+                  lda >= M && ldb >= N && ldc >= N,
+              DAB_EUNSUPPORTED, "%s: K %% 64, N %% 64, lda/ldb %% 8, ldc %% 4 required (M=%d N=%d K=%d)", fn, M, N, K);
+  DAB_REQUIRE(aligned16(A) && aligned16(Bm) && aligned16(C), DAB_EINVAL, "%s: misaligned pointer", fn);
+  if (N % 128 == 0) return launch_gemm_tn<128>(A, lda, Bm, ldb, C, ldc, M, N, K, (cudaStream_t)stream, accumulate);
+  return launch_gemm_tn<64>(A, lda, Bm, ldb, C, ldc, M, N, K, (cudaStream_t)stream, accumulate);
+}
+
 /* C[M,N] (fp32, overwritten) = A[K,M]^T B[K,N]: bf16 operands with the contraction index as their ROW index (activations
  * as they lie in memory, one row per residue); K % 64 == 0, N % 64 == 0, lda % 8 == 0 and ldb % 8 == 0 (TMA row pitch:
  * a multiple of 16 bytes), ldc % 4 == 0, lda >= M, ldb >= N, ldc >= N, any M > 0 otherwise.  Only the M x N block of C
@@ -228,26 +240,14 @@ extern "C" {
  * between runs).  Autograd weight gradients of the nn.Linear layers, diffab_pytorch.py:391-408,464. */
 int dab_gemm_bf16_tn(const void* A, int64_t lda, const void* Bm, int64_t ldb, float* C, int64_t ldc, int M, int N, int K,
                      void* stream) {
-  DAB_REQUIRE(A && Bm && C, DAB_EINVAL, "dab_gemm_bf16_tn: null pointer");
-  DAB_REQUIRE(M > 0 && N > 0 && K > 0 && K % kTnKC == 0 && N % 64 == 0 && lda % 8 == 0 && ldb % 8 == 0 && ldc % 4 == 0 &&
-                  lda >= M && ldb >= N && ldc >= N,
-              DAB_EUNSUPPORTED, "dab_gemm_bf16_tn: K %% 64, N %% 64, lda/ldb %% 8, ldc %% 4 required (M=%d N=%d K=%d)", M, N, K);
-  DAB_REQUIRE(aligned16(A) && aligned16(Bm) && aligned16(C), DAB_EINVAL, "dab_gemm_bf16_tn: misaligned pointer");
-  if (N % 128 == 0) return launch_gemm_tn<128>(A, lda, Bm, ldb, C, ldc, M, N, K, (cudaStream_t)stream);
-  return launch_gemm_tn<64>(A, lda, Bm, ldb, C, ldc, M, N, K, (cudaStream_t)stream);
+  return gemm_tn("dab_gemm_bf16_tn", A, lda, Bm, ldb, C, ldc, M, N, K, stream, false);
 }
 
 /* C[M,N] += A[K,M]^T B[K,N]: dab_gemm_bf16_tn without the fill of C - the caller zeroes (or pre-loads) C, e.g. on a side
  * stream long before the operands exist, so that no fill sits between the producer of the operands and this GEMM. */
 int dab_gemm_bf16_tn_acc(const void* A, int64_t lda, const void* Bm, int64_t ldb, float* C, int64_t ldc, int M, int N, int K,
                          void* stream) {
-  DAB_REQUIRE(A && Bm && C, DAB_EINVAL, "dab_gemm_bf16_tn_acc: null pointer");
-  DAB_REQUIRE(M > 0 && N > 0 && K > 0 && K % kTnKC == 0 && N % 64 == 0 && lda % 8 == 0 && ldb % 8 == 0 && ldc % 4 == 0 &&
-                  lda >= M && ldb >= N && ldc >= N,
-              DAB_EUNSUPPORTED, "dab_gemm_bf16_tn_acc: K %% 64, N %% 64, lda/ldb %% 8, ldc %% 4 required (M=%d N=%d K=%d)", M, N, K);
-  DAB_REQUIRE(aligned16(A) && aligned16(Bm) && aligned16(C), DAB_EINVAL, "dab_gemm_bf16_tn_acc: misaligned pointer");
-  if (N % 128 == 0) return launch_gemm_tn<128>(A, lda, Bm, ldb, C, ldc, M, N, K, (cudaStream_t)stream, true);
-  return launch_gemm_tn<64>(A, lda, Bm, ldb, C, ldc, M, N, K, (cudaStream_t)stream, true);
+  return gemm_tn("dab_gemm_bf16_tn_acc", A, lda, Bm, ldb, C, ldc, M, N, K, stream, true);
 }
 
 /* out[cols] (fp32, overwritten) = column sums of x[rows, cols] (fp32, contiguous): bias gradients (sum over residues).

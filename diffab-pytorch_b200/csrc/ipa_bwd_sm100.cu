@@ -14,7 +14,7 @@
 //   dgamma_h = (1/gamma_h) sum_ij dl_ij,h lp_ij,h,  lp = l - ls - lb, each sum obtained from quantities at hand:
 //              sum dl l from the logits in registers, sum dl ls = <qs, dqs>, sum dl lb = <st Wpb, sum dl e>.
 //
-// Launch sequence (dab_ipa_bwd_sm100):
+// Launch sequence (dab_ipa_bwd_sm100_main: 1 and 2, dab_ipa_bwd_sm100_finish: 3):
 //   1. ipa_bwd_core_kernel  : per CTA = (patch, 16 query rows), thread = key j = TMEM lane (as the forward core):
 //        prologue: dcat, cat rows of the tile -> dO (fp16 with a per-row power-of-two scale, in shared memory; bf16 copy to
 //                  HBM for the key side), dopair (bf16, shared memory), Delta   (a separate launch until round 2)
@@ -881,33 +881,33 @@ size_t dab_ipa_bwd_sm100_workspace_bytes(const DabIpaDims* d) { return shape_ok(
 
 static int bwd_sm100_impl(const DabIpaDims* d, const void* packed, const void* e_bf16, const float* R, const float* dcat,
                           void* saved, size_t saved_bytes, void* dproj_bf16, void* de_bf16, float* d_w_pair_bias, float* d_gamma,
-                          void* workspace, size_t workspace_bytes, void* stream, int parts) {
-  DAB_REQUIRE(shape_ok(d), DAB_EUNSUPPORTED,
-              "dab_ipa_bwd_sm100: the sm_100a fast path needs L=128, D=128, C=64, H=8, ds=32, Pq=Pv=8");
+                          void* workspace, size_t workspace_bytes, void* stream, bool finish) {
+  const char* fn = finish ? "dab_ipa_bwd_sm100_finish" : "dab_ipa_bwd_sm100_main";
+  DAB_REQUIRE(shape_ok(d), DAB_EUNSUPPORTED, "%s: the sm_100a fast path needs L=128, D=128, C=64, H=8, ds=32, Pq=Pv=8", fn);
   if (d->B == 0) return DAB_OK;
   DAB_REQUIRE(packed && e_bf16 && R && dcat && saved && dproj_bf16 && de_bf16 && d_w_pair_bias && d_gamma && workspace,
-              DAB_EINVAL, "dab_ipa_bwd_sm100: null pointer");
+              DAB_EINVAL, "%s: null pointer", fn);
   DAB_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0 && (reinterpret_cast<uintptr_t>(saved) & 1023) == 0 &&
                   (reinterpret_cast<uintptr_t>(e_bf16) & 127) == 0 && (reinterpret_cast<uintptr_t>(de_bf16) & 127) == 0 &&
                   aligned16(dcat) && aligned32(dproj_bf16),
-              DAB_EINVAL, "dab_ipa_bwd_sm100: misaligned pointer (workspaces 1024 B, e/de 128 B, dcat 16 B, dproj 32 B)");
+              DAB_EINVAL, "%s: misaligned pointer (workspaces 1024 B, e/de 128 B, dcat 16 B, dproj 32 B)", fn);
   const int B = d->B, M = B * L;
   Ws ws = carve_ws(B, saved);
   BwdWs bw = carve_bwd(B, workspace);
-  DAB_REQUIRE(saved_bytes >= ws.bytes, DAB_EWORKSPACE, "dab_ipa_bwd_sm100: saved workspace %zu < %zu", saved_bytes, ws.bytes);
-  DAB_REQUIRE(workspace_bytes >= bw.bytes, DAB_EWORKSPACE, "dab_ipa_bwd_sm100: workspace %zu < %zu", workspace_bytes, bw.bytes);
+  DAB_REQUIRE(saved_bytes >= ws.bytes, DAB_EWORKSPACE, "%s: saved workspace %zu < %zu", fn, saved_bytes, ws.bytes);
+  DAB_REQUIRE(workspace_bytes >= bw.bytes, DAB_EWORKSPACE, "%s: workspace %zu < %zu", fn, workspace_bytes, bw.bytes);
   const PackedOffsets po = packed_offsets();
   const uint8_t* pk = reinterpret_cast<const uint8_t*>(packed);
   const float* wpb = reinterpret_cast<const float*>(pk + po.wpb);
   const float* gamma = reinterpret_cast<const float*>(pk + po.gamma);
   cudaStream_t s = (cudaStream_t)stream;
 
-  if (!(parts & 1)) {   // only the final reductions: d_w_pair_bias / d_gamma from the partial sums of an earlier main pass
+  if (finish) {   // only the final reductions: d_w_pair_bias / d_gamma from the partial sums of an earlier main pass
     bwd_reduce_kernel<<<kRedBlocks, 512, 0, s>>>(bw.p_wpb, B * 8, bw.p_g1, bw.p_g2, B, bw.r_part);
     count_launch();
     bwd_finalize_kernel<<<1, 512, 0, s>>>(bw.r_part, wpb, gamma, d_w_pair_bias, d_gamma);
     count_launch();
-    return check_launch("dab_ipa_bwd_sm100_finish");
+    return check_launch(fn);
   }
   CUtensorMap mv, me;
   {
@@ -942,23 +942,10 @@ static int bwd_sm100_impl(const DabIpaDims* d, const void* packed, const void* e
                                                             reinterpret_cast<__nv_bfloat16*>(dproj_bf16), bw.p_g2,
                                                             g_bwd_keep_qkv ? bw.dQ : nullptr);
   count_launch();
-  if (parts & 2) {
-    bwd_reduce_kernel<<<kRedBlocks, 512, 0, s>>>(bw.p_wpb, B * 8, bw.p_g1, bw.p_g2, B, bw.r_part);
-    count_launch();
-    bwd_finalize_kernel<<<1, 512, 0, s>>>(bw.r_part, wpb, gamma, d_w_pair_bias, d_gamma);
-    count_launch();
-  }
-  return check_launch("dab_ipa_bwd_sm100");
+  return check_launch(fn);
 }
 
-int dab_ipa_bwd_sm100(const DabIpaDims* d, const void* packed, const void* e_bf16, const float* R, const float* dcat,
-                      void* saved, size_t saved_bytes, void* dproj_bf16, void* de_bf16, float* d_w_pair_bias, float* d_gamma,
-                      void* workspace, size_t workspace_bytes, void* stream) {
-  return bwd_sm100_impl(d, packed, e_bf16, R, dcat, saved, saved_bytes, dproj_bf16, de_bf16, d_w_pair_bias, d_gamma, workspace,
-                        workspace_bytes, stream, 3);
-}
-
-/* The same backward in two calls, so that a caller can overlap what depends only on dproj (dx, dWcat) with the final
+/* The backward in two calls, so that a caller can overlap what depends only on dproj (dx, dWcat) with the final
  * reductions: `_main` = everything up to dproj / de and the per-CTA partial sums, `_finish` = d_w_pair_bias / d_gamma from
  * those partial sums (same arguments; it reads only packed, d_w_pair_bias, d_gamma and the workspace).  May run on
  * different streams if the caller orders _finish after _main. */
@@ -966,13 +953,13 @@ int dab_ipa_bwd_sm100_main(const DabIpaDims* d, const void* packed, const void* 
                            void* saved, size_t saved_bytes, void* dproj_bf16, void* de_bf16, float* d_w_pair_bias,
                            float* d_gamma, void* workspace, size_t workspace_bytes, void* stream) {
   return bwd_sm100_impl(d, packed, e_bf16, R, dcat, saved, saved_bytes, dproj_bf16, de_bf16, d_w_pair_bias, d_gamma, workspace,
-                        workspace_bytes, stream, 1);
+                        workspace_bytes, stream, false);
 }
 int dab_ipa_bwd_sm100_finish(const DabIpaDims* d, const void* packed, const void* e_bf16, const float* R, const float* dcat,
                              void* saved, size_t saved_bytes, void* dproj_bf16, void* de_bf16, float* d_w_pair_bias,
                              float* d_gamma, void* workspace, size_t workspace_bytes, void* stream) {
   return bwd_sm100_impl(d, packed, e_bf16, R, dcat, saved, saved_bytes, dproj_bf16, de_bf16, d_w_pair_bias, d_gamma, workspace,
-                        workspace_bytes, stream, 2);
+                        workspace_bytes, stream, true);
 }
 
 #ifdef DAB_DEBUG_HOOKS
@@ -988,7 +975,7 @@ int dab_debug_set_bwd_timeline(long long* buf) {
   return DAB_OK;
 }
 
-/* Test hook: the intermediate buffers of the last dab_ipa_bwd_sm100 call on `workspace` (device pointers). */
+/* Test hook: the intermediate buffers of the last dab_ipa_bwd_sm100_main call on `workspace` (device pointers). */
 int dab_debug_bwd_sm100_buffers(const DabIpaDims* d, void* workspace, void** out /* 10 pointers */) {
   DAB_REQUIRE(shape_ok(d) && workspace && out, DAB_EINVAL, "dab_debug_bwd_sm100_buffers: bad argument");
   BwdWs bw = carve_bwd(d->B, workspace);

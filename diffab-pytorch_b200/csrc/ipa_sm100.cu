@@ -1,14 +1,14 @@
 // sm_100a fast path of one InvariantPointAttentionLayer (train.py configuration: L=128, D=128, C=64, H=8, ds=32,
 // Pq=Pv=8).  Replaces diffab_pytorch.py:389-465 of the reference.
 //
-// Three launches per layer (dab_ipa_fwd_sm100 / _io / _train / _stages):
+// Three launches per layer (dab_ipa_fwd_sm100_train / _stages):
 //   1. ipa_proj_kernel (ipa_proj_sm100.cuh): x -> bf16 -> the six projections on tcgen05 -> frame transform (x R + t,
 //      centred on the patch centroid), logit scales folded into q, split-bf16 (hi + lo) point coordinates,
 //      -0.5 c |k|^2 as extra K columns -> packed operands Qp, Kp, Vp (TMA stores)
 //   2. ipa_core_kernel (this file): one persistent CTA per SM with two tile contexts (tile = patch x 16 query rows);
 //      TMA-staged tiles, tcgen05.mma with TMEM accumulators; j (keys) sits on the 128 TMEM lanes:
 //        S^T_h = K_h Q_h^T          (M=128 j, N=16 i, K=32+3*32)   scalar + expanded point-distance logits
-//        + precomputed pair bias (dab_ipa_pair_bias*), softmax over j in fp32 (warp butterflies + one exchange per row pair)
+//        + precomputed pair bias (dab_ipa_pair_bias_multi), fp32 softmax over j (warp butterflies, one exchange per row pair)
 //        [pair_2p ; pair_2p+1]^T = [e[2p] | e[2p+1]]^T [P_2p ; P_2p+1]^T   (M=128, N=16, K=128 j)  same e tiles, MN-major
 //        [O_2m ; O_2m+1]^T = [V_2m | V_2m+1]^T [P_2m ; P_2m+1]^T          (M=128, N=32, K=128 j)  fp16 operands
 //      epilogue: normalise, inverse frame, norms -> concat features (bf16)
@@ -242,7 +242,7 @@ __device__ __forceinline__ void tmem_ld_x4(uint32_t taddr, float (&v)[4]) {
 // issues the context's tcgen05.mma; warp 18 lane 0 issues the K / Q loads of both contexts, warp 19 lane 0 the pair-row
 // and value loads.  The roles meet only at mbarriers.
 // `bias` is the layer's precomputed pair bias, fp16 [B*L rows i][128 j][8 h], already scaled by
-// scale_total * log2(e) (dab_ipa_pair_bias): e is constant over the six layers and the T steps, so the
+// scale_total * log2(e) (dab_ipa_pair_bias_multi): e is constant over the six layers and the T steps, so the
 // e . Wpb contraction is hoisted out of the sampling loop entirely.
 constexpr int kCoreThreads = 640;
 template <bool KB2>     // KB2: key-block mode for patches of 256 residues (see `decode` below); false: the L = 128 kernel
@@ -988,20 +988,8 @@ int dab_ipa_sm100_workspace_layout(const DabIpaDims* d, size_t* offsets /* 8 */)
   return DAB_OK;
 }
 
-int dab_ipa_pair_bias(const DabIpaDims* d, const void* e_bf16, const float* w_pair_bias, void* bias_f16, void* stream) {
-  DAB_REQUIRE(shape_ok_fwd(d), DAB_EUNSUPPORTED,
-              "dab_ipa_pair_bias: the sm_100a fast path needs L=128 (or 256), D=128, C=64, H=8, ds=32, Pq=Pv=8");
-  if (d->B == 0) return DAB_OK;
-  DAB_REQUIRE(e_bf16 && w_pair_bias && bias_f16 && (reinterpret_cast<uintptr_t>(e_bf16) & 127) == 0 &&
-                  aligned16(bias_f16),
-              DAB_EINVAL, "dab_ipa_pair_bias: null or misaligned pointer (e 128 B, bias 16 B)");
-  const int64_t n_pairs = (int64_t)d->B * d->L * d->L;
-  if (int rc = launch_pair_bias(e_bf16, w_pair_bias, 1, bias_f16, n_pairs, (cudaStream_t)stream)) return rc;
-  return check_launch("dab_ipa_pair_bias");
-}
-
-/* Same for n_layers <= 6 layers in one pass over the pair tensor: w_pair_bias[n_layers][8][64] fp32 (contiguous),
- * planes_f16[n_layers][B*L*L][8] fp16 (contiguous). */
+/* Pair-bias planes of n_layers <= 6 layers in one pass over the pair tensor: w_pair_bias[n_layers][8][64] fp32
+ * (contiguous), planes_f16[n_layers][B*L*L][8] fp16 (contiguous). */
 int dab_ipa_pair_bias_multi(const DabIpaDims* d, const void* e_bf16, const float* w_pair_bias, int n_layers,
                             void* planes_f16, void* stream) {
   DAB_REQUIRE(shape_ok_fwd(d), DAB_EUNSUPPORTED,
@@ -1018,11 +1006,13 @@ int dab_ipa_pair_bias_multi(const DabIpaDims* d, const void* e_bf16, const float
 
 // Projection launch of a layer (weights `pk`), packed operands into `ws`.  With `pk_prev` the kernel first computes the
 // PREVIOUS layer's to_out, y = cat Wout^T + b (cat = ws.cat, weights pk_prev), straight into its A tile: x is not read.
+// With `w2` (patches of 256 residues, B = 2 x patches) the patch centroids are computed first and the projections are
+// centred on them.
 // the epsilon network's front MLP as the input of layer 0 (mode 2 of the projection kernel): y = relu(c[row] + t1[seq[row]]) W2^T + b2
 struct FrontIn { const float* c; const float* t1; const int64_t* seq; const void* w2_bf16; const float* b2; };
 static int launch_proj(int B, const uint8_t* pk, const float* x, const __nv_bfloat16* x16, const float* R, const float* t,
-                       const Ws& ws, const uint8_t* pk_prev, cudaStream_t s, const float* cen_ext = nullptr,
-                       const FrontIn* front = nullptr) {
+                       const Ws& ws, const Ws2* w2, const uint8_t* pk_prev, cudaStream_t s, const FrontIn* front = nullptr) {
+  if (w2) { centroid256_kernel<<<B / 2, 256, 0, s>>>(t, w2->cen); count_launch(); }
   const PackedOffsets po = packed_offsets();
   const int M = B * L;
   CUtensorMap mw64, mw48;
@@ -1059,42 +1049,68 @@ static int launch_proj(int B, const uint8_t* pk, const float* x, const __nv_bflo
   }
   ipa_proj_kernel<<<dim3(n_split, B), 288, ProjSmem::kTotal, s>>>(
       mw64, mw48, msq, msk, msv, x, R, t, reinterpret_cast<const float*>(pk + po.gamma), ws.Qp, ws.Kp, ws.Vp, ws.tc,
-      g_core_dbg ? g_core_dbg + (1 << 20) : nullptr, x16, mcat, mwout, b_out, pk_prev ? 1 : (front ? 2 : 0), cen_ext,
+      g_core_dbg ? g_core_dbg + (1 << 20) : nullptr, x16, mcat, mwout, b_out, pk_prev ? 1 : (front ? 2 : 0),
+      w2 ? w2->cen : nullptr,
       front ? reinterpret_cast<const float4*>(front->c) : nullptr, front ? reinterpret_cast<const float4*>(front->t1) : nullptr,
       front ? front->seq : nullptr);
   count_launch();
   return DAB_OK;
 }
 
-// x / y: fp32, or (x_bf16 / y_bf16 non-null) bf16 - the residue stream handed from layer to layer already rounded
-static int fwd_sm100_impl(const DabIpaDims* d, const void* packed, const float* x, const void* e_bf16,
-                          const void* bias_f16, const float* R, const float* t, float* y, void* workspace,
-                          size_t workspace_bytes, bool save_for_bwd, void* stream, const void* x_bf16 = nullptr,
-                          void* y_bf16 = nullptr, int phases = 7) {
-  DAB_REQUIRE(save_for_bwd ? shape_ok(d) : shape_ok_fwd(d), DAB_EUNSUPPORTED,
-              "dab_ipa_fwd_sm100: the sm_100a fast path needs D=128, C=64, H=8, ds=32, Pq=Pv=8 and L=128 (inference: 128 or 256)");
+// Workspace views of a forward call.  A patch of 256 residues = two blocks of 128: everything row-wise (projections,
+// to_out) runs on nblk = 2 B blocks, the attention core once per (query block, key block) pair, and the two key blocks'
+// results are merged by their softmax statistics (w2).
+struct FwdWs {
+  bool two;
+  int nblk;   // 0: empty batch, nothing to launch
+  Ws ws;
+  Ws2 w2;
+};
+
+// Prologue shared by the forward entry points (`fn`: the one the caller called, for the messages): the shape, the
+// pointers (`args_ok` / `args_aligned`: the caller's own operands), the workspace size, and the workspace views.
+static int fwd_prologue(const char* fn, const DabIpaDims* d, bool train, bool args_ok, bool args_aligned, const void* packed,
+                        void* workspace, size_t workspace_bytes, FwdWs& f) {
+  DAB_REQUIRE(train ? shape_ok(d) : shape_ok_fwd(d), DAB_EUNSUPPORTED,
+              "%s: the sm_100a fast path needs the train.py configuration (D=128, C=64, H=8, ds=32, Pq=Pv=8) and L=128 "
+              "(inference: 128 or 256)", fn);
+  f = {};
+  f.two = d->L == 2 * L;
   if (d->B == 0) return DAB_OK;
-  DAB_REQUIRE(packed && (x || x_bf16) && e_bf16 && R && t && (y || y_bf16) && workspace, DAB_EINVAL,
-              "dab_ipa_fwd_sm100: null pointer");
-  DAB_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0 && (reinterpret_cast<uintptr_t>(packed) & 1023) == 0 &&
-                  (reinterpret_cast<uintptr_t>(e_bf16) & 127) == 0 && aligned16(x) && aligned16(y) && aligned16(x_bf16) &&
-                  aligned16(y_bf16),
-              DAB_EINVAL, "dab_ipa_fwd_sm100: misaligned pointer (workspace/packed 1024 B, e 128 B, x/y 16 B)");
-  // A patch of 256 residues = two blocks of 128: everything row-wise (projections, to_out) runs on 2 B blocks, the attention
-  // core once per (query block, key block) pair, and the two key blocks' results are merged by their softmax statistics.
-  const bool two = d->L == 2 * L;
-  const int Lp = d->L, B = two ? 2 * d->B : d->B, M = B * L;
-  Ws ws = carve_ws(B, workspace);
-  Ws2 w2 = {};
-  size_t need = ws.bytes;
-  if (two) { w2 = carve_ws2(d->B, workspace); need = w2.bytes; }
-  DAB_REQUIRE(workspace_bytes >= need, DAB_EWORKSPACE, "dab_ipa_fwd_sm100: workspace %zu < %zu", workspace_bytes, need);
+  DAB_REQUIRE(args_ok && packed && workspace, DAB_EINVAL, "%s: null pointer", fn);
+  DAB_REQUIRE(args_aligned && (reinterpret_cast<uintptr_t>(workspace) & 1023) == 0 &&
+                  (reinterpret_cast<uintptr_t>(packed) & 1023) == 0,
+              DAB_EINVAL, "%s: misaligned pointer (workspace / packed weights 1024 B, e 128 B, other arrays 16 B)", fn);
+  f.nblk = f.two ? 2 * d->B : d->B;
+  f.ws = carve_ws(f.nblk, workspace);
+  size_t need = f.ws.bytes;
+  if (f.two) { f.w2 = carve_ws2(d->B, workspace); need = f.w2.bytes; }
+  DAB_REQUIRE(workspace_bytes >= need, DAB_EWORKSPACE, "%s: workspace %zu < %zu", fn, workspace_bytes, need);
+  return DAB_OK;
+}
+
+// x / y: fp32, or (x_bf16 / y_bf16 non-null) bf16 - the residue stream handed from layer to layer already rounded
+static int fwd_sm100_impl(const char* fn, const DabIpaDims* d, const void* packed, const float* x, const void* e_bf16,
+                          const void* bias_f16, const float* R, const float* t, float* y, void* workspace,
+                          size_t workspace_bytes, bool save_for_bwd, void* stream, const void* x_bf16, void* y_bf16,
+                          int phases) {
+  FwdWs f;
+  if (int rc = fwd_prologue(fn, d, save_for_bwd, (x || x_bf16) && e_bf16 && R && t && (y || y_bf16),
+                            (reinterpret_cast<uintptr_t>(e_bf16) & 127) == 0 && aligned16(x) && aligned16(y) &&
+                                aligned16(x_bf16) && aligned16(y_bf16),
+                            packed, workspace, workspace_bytes, f))
+    return rc;
+  if (f.nblk == 0) return DAB_OK;
+  const bool two = f.two;
+  const int Lp = d->L, B = f.nblk, M = B * L;
+  const Ws& ws = f.ws;
+  const Ws2& w2 = f.w2;
   const PackedOffsets po = packed_offsets();
   const uint8_t* pk = reinterpret_cast<const uint8_t*>(packed);
   cudaStream_t s = (cudaStream_t)stream;
   if (phases & 1) {
-    if (two) { centroid256_kernel<<<d->B, 256, 0, s>>>(t, w2.cen); count_launch(); }
-    if (int rc = launch_proj(B, pk, x, reinterpret_cast<const __nv_bfloat16*>(x_bf16), R, t, ws, nullptr, s, two ? w2.cen : nullptr))
+    if (int rc = launch_proj(B, pk, x, reinterpret_cast<const __nv_bfloat16*>(x_bf16), R, t, ws, two ? &w2 : nullptr,
+                             nullptr, s))
       return rc;
   }
   if (phases & 2) {
@@ -1146,13 +1162,7 @@ static int fwd_sm100_impl(const DabIpaDims* d, const void* packed, const float* 
                                       : launch_gemm_bf16<32>(ws.cat, NCAT, pk + po.wout, NCAT, y, D, bo, M, D, NCAT, s, y_bf16))
       return rc;
   }
-  return check_launch("dab_ipa_fwd_sm100");
-}
-
-int dab_ipa_fwd_sm100(const DabIpaDims* d, const void* packed, const float* x, const void* e_bf16,
-                      const void* bias_f16, const float* R, const float* t, float* y, void* workspace,
-                      size_t workspace_bytes, void* stream) {
-  return fwd_sm100_impl(d, packed, x, e_bf16, bias_f16, R, t, y, workspace, workspace_bytes, false, stream);
+  return check_launch(fn);
 }
 
 /* Byte offsets inside the packed weights: offs[0..6] = Wcat bf16 [1344][128] (rows: to_q_scalar, to_k_scalar, to_v_scalar,
@@ -1167,62 +1177,46 @@ int dab_ipa_packed_layout(const DabIpaDims* d, size_t* offs) {
   return DAB_OK;
 }
 
-/* Same layer with the residue stream in bf16 on either side: exactly one of x / x_bf16 and one of y / y_bf16 is given.
- * Between the layers of a stack the stream is consumed as bf16 anyway (the projections' A operand), so handing it over
- * already rounded changes no bit of the result and halves its HBM traffic. */
-int dab_ipa_fwd_sm100_io(const DabIpaDims* d, const void* packed, const float* x, const void* x_bf16, const void* e_bf16,
-                         const void* bias_f16, const float* R, const float* t, float* y, void* y_bf16, void* workspace,
-                         size_t workspace_bytes, void* stream) {
-  DAB_REQUIRE((x == nullptr) != (x_bf16 == nullptr) && (y == nullptr) != (y_bf16 == nullptr), DAB_EINVAL,
-              "dab_ipa_fwd_sm100_io: give exactly one of x / x_bf16 and one of y / y_bf16");
-  return fwd_sm100_impl(d, packed, x, e_bf16, bias_f16, R, t, y, workspace, workspace_bytes, false, stream, x_bf16, y_bf16);
-}
-
-/* Training forward: same launches; the workspace additionally keeps what dab_ipa_bwd_sm100 needs (packed operands,
+/* Training forward: same launches; the workspace additionally keeps what dab_ipa_bwd_sm100_main needs (packed operands,
  * concat features, un-normalised probabilities and the softmax statistics) and must be handed to it untouched. */
 int dab_ipa_fwd_sm100_train(const DabIpaDims* d, const void* packed, const float* x, const void* e_bf16,
                             const void* bias_f16, const float* R, const float* t, float* y, void* saved,
                             size_t saved_bytes, void* stream) {
-  return fwd_sm100_impl(d, packed, x, e_bf16, bias_f16, R, t, y, saved, saved_bytes, true, stream);
+  return fwd_sm100_impl("dab_ipa_fwd_sm100_train", d, packed, x, e_bf16, bias_f16, R, t, y, saved, saved_bytes, true, stream,
+                        nullptr, nullptr, 7);
 }
 
-/* The same layer launch by launch: `stages` = bit0 projections + frame transform, bit1 attention core, bit2 to_out.  The
- * workspace must hold the products of the earlier stages (a previous call with the lower bits).  Lets a caller bracket one
- * stage with its own events (bench.py's roofline of the attention core) or interleave its own work between the stages. */
+/* The inference forward, whole (stages = 7) or launch by launch: `stages` = bit0 projections + frame transform, bit1
+ * attention core, bit2 to_out.  The workspace must hold the products of the earlier stages (a previous call with the lower
+ * bits).  Lets a caller bracket one stage with its own events (bench.py's roofline of the attention core) or interleave its
+ * own work between the stages.  The residue stream is fp32 or bf16 on either side: exactly one of x / x_bf16 and one of
+ * y / y_bf16 is given.  Between the layers of a stack the stream is consumed as bf16 anyway (the projections' A operand),
+ * so handing it over already rounded changes no bit of the result and halves its HBM traffic. */
 int dab_ipa_fwd_sm100_stages(const DabIpaDims* d, const void* packed, const float* x, const void* x_bf16, const void* e_bf16,
                              const void* bias_f16, const float* R, const float* t, float* y, void* y_bf16, void* workspace,
                              size_t workspace_bytes, int stages, void* stream) {
   DAB_REQUIRE((x == nullptr) != (x_bf16 == nullptr) && (y == nullptr) != (y_bf16 == nullptr), DAB_EINVAL,
               "dab_ipa_fwd_sm100_stages: give exactly one of x / x_bf16 and one of y / y_bf16");
   DAB_REQUIRE(stages > 0 && stages <= 7, DAB_EINVAL, "dab_ipa_fwd_sm100_stages: stages must be a non-empty subset of bits 0..2");
-  return fwd_sm100_impl(d, packed, x, e_bf16, bias_f16, R, t, y, workspace, workspace_bytes, false, stream, x_bf16, y_bf16,
-                        stages);
+  return fwd_sm100_impl("dab_ipa_fwd_sm100_stages", d, packed, x, e_bf16, bias_f16, R, t, y, workspace, workspace_bytes, false,
+                        stream, x_bf16, y_bf16, stages);
 }
 
 /* Between two layers of a stack (inference): the previous layer's to_out (y = cat Wout^T + b, `packed_prev`; `cat` = the
  * concat features its attention core left in `workspace`) fused with this layer's projections (`packed`): y is rounded to
- * bf16 exactly as dab_ipa_fwd_sm100_io would hand it over, but goes straight into the projection kernel's operand tile
- * and never exists in HBM; the packed Q / K / V of this layer replace those of the previous one in `workspace`.
+ * bf16 exactly as dab_ipa_fwd_sm100_stages would hand it over (y_bf16), but goes straight into the projection kernel's
+ * operand tile and never exists in HBM; the packed Q / K / V of this layer replace those of the previous one in `workspace`.
  * Sequence for a stack: stages(1) of layer 0, then per layer stages(2) followed by dab_ipa_mid_sm100 (or stages(4) after
  * the last layer).  Bit-identical to the unfused sequence. */
 int dab_ipa_mid_sm100(const DabIpaDims* d, const void* packed_prev, const void* packed, const float* R, const float* t,
                       void* workspace, size_t workspace_bytes, void* stream) {
-  DAB_REQUIRE(shape_ok_fwd(d), DAB_EUNSUPPORTED, "dab_ipa_mid_sm100: the sm_100a fast path needs the train.py configuration");
-  if (d->B == 0) return DAB_OK;
-  DAB_REQUIRE(packed_prev && packed && R && t && workspace, DAB_EINVAL, "dab_ipa_mid_sm100: null pointer");
-  DAB_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0 && (reinterpret_cast<uintptr_t>(packed) & 1023) == 0 &&
-                  (reinterpret_cast<uintptr_t>(packed_prev) & 1023) == 0,
-              DAB_EINVAL, "dab_ipa_mid_sm100: workspace / packed weights must be 1024-byte aligned");
-  const bool two = d->L == 2 * L;
-  const int nblk = two ? 2 * d->B : d->B;
-  Ws ws = carve_ws(nblk, workspace);
-  Ws2 w2 = {};
-  size_t need = ws.bytes;
-  if (two) { w2 = carve_ws2(d->B, workspace); need = w2.bytes; }
-  DAB_REQUIRE(workspace_bytes >= need, DAB_EWORKSPACE, "dab_ipa_mid_sm100: workspace %zu < %zu", workspace_bytes, need);
-  if (two) { centroid256_kernel<<<d->B, 256, 0, (cudaStream_t)stream>>>(t, w2.cen); count_launch(); }
-  if (int rc = launch_proj(nblk, reinterpret_cast<const uint8_t*>(packed), nullptr, nullptr, R, t, ws,
-                           reinterpret_cast<const uint8_t*>(packed_prev), (cudaStream_t)stream, two ? w2.cen : nullptr))
+  FwdWs f;
+  if (int rc = fwd_prologue("dab_ipa_mid_sm100", d, false, packed_prev && R && t,
+                            (reinterpret_cast<uintptr_t>(packed_prev) & 1023) == 0, packed, workspace, workspace_bytes, f))
+    return rc;
+  if (f.nblk == 0) return DAB_OK;
+  if (int rc = launch_proj(f.nblk, reinterpret_cast<const uint8_t*>(packed), nullptr, nullptr, R, t, f.ws,
+                           f.two ? &f.w2 : nullptr, reinterpret_cast<const uint8_t*>(packed_prev), (cudaStream_t)stream))
     return rc;
   return check_launch("dab_ipa_mid_sm100");
 }
@@ -1235,48 +1229,29 @@ int dab_ipa_mid_sm100(const DabIpaDims* d, const void* packed_prev, const void* 
 int dab_ipa_front_proj_sm100(const DabIpaDims* d, const void* packed, const float* c, const float* t1, const int64_t* seq,
                              const void* w2_bf16, const float* b2, const float* R, const float* t, void* workspace,
                              size_t workspace_bytes, void* stream) {
-  DAB_REQUIRE(shape_ok_fwd(d), DAB_EUNSUPPORTED, "dab_ipa_front_proj_sm100: the sm_100a fast path needs the train.py configuration");
-  if (d->B == 0) return DAB_OK;
-  DAB_REQUIRE(packed && c && t1 && seq && w2_bf16 && b2 && R && t && workspace, DAB_EINVAL, "dab_ipa_front_proj_sm100: null pointer");
-  DAB_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0 && (reinterpret_cast<uintptr_t>(packed) & 1023) == 0 &&
-                  aligned16(c) && aligned16(t1) && aligned16(w2_bf16),
-              DAB_EINVAL, "dab_ipa_front_proj_sm100: misaligned pointer (workspace / packed 1024 B, c / t1 / w2 16 B)");
-  const bool two = d->L == 2 * L;
-  const int nblk = two ? 2 * d->B : d->B;
-  Ws ws = carve_ws(nblk, workspace);
-  Ws2 w2s = {};
-  size_t need = ws.bytes;
-  if (two) { w2s = carve_ws2(d->B, workspace); need = w2s.bytes; }
-  DAB_REQUIRE(workspace_bytes >= need, DAB_EWORKSPACE, "dab_ipa_front_proj_sm100: workspace %zu < %zu", workspace_bytes, need);
-  if (two) { centroid256_kernel<<<d->B, 256, 0, (cudaStream_t)stream>>>(t, w2s.cen); count_launch(); }
+  FwdWs f;
+  if (int rc = fwd_prologue("dab_ipa_front_proj_sm100", d, false, c && t1 && seq && w2_bf16 && b2 && R && t,
+                            aligned16(c) && aligned16(t1) && aligned16(w2_bf16), packed, workspace, workspace_bytes, f))
+    return rc;
+  if (f.nblk == 0) return DAB_OK;
   const FrontIn fr = {c, t1, seq, w2_bf16, b2};
-  if (int rc = launch_proj(nblk, reinterpret_cast<const uint8_t*>(packed), nullptr, nullptr, R, t, ws, nullptr,
-                           (cudaStream_t)stream, two ? w2s.cen : nullptr, &fr))
+  if (int rc = launch_proj(f.nblk, reinterpret_cast<const uint8_t*>(packed), nullptr, nullptr, R, t, f.ws,
+                           f.two ? &f.w2 : nullptr, nullptr, (cudaStream_t)stream, &fr))
     return rc;
   return check_launch("dab_ipa_front_proj_sm100");
 }
 
-/* C[M,N] = A[M,K] B[N,K]^T + bias on the tcgen05 GEMM (bf16 operands, fp32 result; M % 128 == 0, N % 64 == 0, K % 64 == 0):
- * the nn.Linear of diffab_pytorch.py:464 as a stand-alone entry point. */
-int dab_gemm_bf16(const void* A, const void* Bm, float* Cm, const float* bias, int M, int N, int K, void* stream) {
-  DAB_REQUIRE(A && Bm && Cm, DAB_EINVAL, "dab_gemm_bf16: null pointer");
-  // narrow N tiles and a deep ring when 64-wide tiles would leave most SMs idle (e.g. dx = dproj Wcat: N = 128, K = 1344);
-  // wide tiles when there are more than two waves of them (e.g. dcat = dy Wout: N = 1024, K = 128)
-  if (M > 0 && N % 64 == 0 && (M / kGemmBM) * (N / 64) < 148)
-    return launch_gemm_bf16<32>(A, K, Bm, K, Cm, N, bias, M, N, K, (cudaStream_t)stream);
-  if (N % 128 == 0 && (M / kGemmBM) * (N / 128) >= 2 * 148)
-    return launch_gemm_bf16<128>(A, K, Bm, K, Cm, N, bias, M, N, K, (cudaStream_t)stream);
-  return launch_gemm_bf16<64>(A, K, Bm, K, Cm, N, bias, M, N, K, (cudaStream_t)stream);
-}
-
-/* nn.Linear (+ ReLU) of the dense glue on the same GEMM: C = act(A[M,K] W[N,K]^T + bias), bf16 operands, fp32 accumulation;
- * the result as fp32 (C_f32) or rounded to bf16 (C_bf16) - exactly one of the two.  M % 128 == 0, N % 64 == 0, K % 64 == 0.
- * Forward of the MLPs of diffab_pytorch.py:57-183,572-599 in mixed-precision training, and (W transposed) their data gradients. */
+/* nn.Linear (+ ReLU) on the tcgen05 GEMM: C = act(A[M,K] W[N,K]^T + bias), bf16 operands, fp32 accumulation; the result as
+ * fp32 (C_f32) or rounded to bf16 (C_bf16) - exactly one of the two.  M % 128 == 0, N % 64 == 0, K % 64 == 0.
+ * Forward of the MLPs of diffab_pytorch.py:57-183,572-599 in mixed-precision training, and (W transposed) their data
+ * gradients and those of the IPA layer's nn.Linear layers (dcat = dy Wout, dx = dproj Wcat). */
 int dab_linear_bf16(const void* A, const void* W, const float* bias, int relu, int M, int N, int K, float* C_f32, void* C_bf16,
                     void* stream) {
   DAB_REQUIRE(A && W && ((C_f32 == nullptr) != (C_bf16 == nullptr)), DAB_EINVAL,
               "dab_linear_bf16: null pointer (exactly one of C_f32 / C_bf16 must be given)");
   cudaStream_t s = (cudaStream_t)stream;
+  // narrow N tiles and a deep ring when 64-wide tiles would leave most SMs idle (e.g. dx = dproj Wcat: N = 128, K = 1344);
+  // wide tiles when there are more than two waves of them (e.g. dcat = dy Wout: N = 1024, K = 128)
   if (M > 0 && N % 64 == 0 && (M / kGemmBM) * (N / 64) < 148)
     return launch_gemm_bf16<32>(A, K, W, K, C_f32, N, bias, M, N, K, s, C_bf16, relu);
   if (N % 128 == 0 && (M / kGemmBM) * (N / 128) >= 2 * 148)

@@ -571,15 +571,20 @@ def _fast_len(L, inference):
     return FAST_L2 if inference and L <= FAST_L2 else None
 
 
-def _pad_patch(x, e, r, t, L_to=FAST_L):
-    """Pad a patch batch of L < 128 residues to the tensor-core kernels' length: zero residues / pair rows, identity
-    frames.  Differentiable (F.pad / cat), so gradients reach the unpadded tensors."""
+def _pad_patch(x, e, r, t, planes, L_to, make_planes):
+    """Pad a patch batch of L < L_to residues to the tensor-core kernels' length: zero residues / pair rows, identity
+    frames, and the pair-bias planes (one per layer; None: ``make_planes`` builds them from the padded pair tensor) with
+    the padded keys masked.  Differentiable (F.pad / cat), so gradients reach the unpadded tensors."""
     L = x.shape[1]
     n = L_to - L
     xp = F.pad(x, (0, 0, 0, n))
     ep = F.pad(e, (0, 0, 0, n, 0, n))
     eye = torch.eye(3, device=r.device, dtype=r.dtype).expand(r.shape[0], n, 3, 3)
-    return xp, ep, torch.cat([r, eye], dim=1), F.pad(t, (0, 0, 0, n))
+    rp, tp = torch.cat([r, eye], dim=1), F.pad(t, (0, 0, 0, n))
+    with torch.no_grad():
+        planes = make_planes(ep.detach()) if planes is None else [F.pad(p_, (0, 0, 0, n, 0, n)) for p_ in planes]
+        _mask_padded_keys(planes, L)
+    return xp, ep, rp, tp, planes
 
 
 def _mask_padded_keys(planes, L):
@@ -609,6 +614,27 @@ def _ipa_structs(layer, B, L):
 
 def _weights_struct(tensors):
     return _lib.DabIpaWeights(*(t.data_ptr() for t in tensors))
+
+
+def _fwd_stages(dims, packed, x, e, bias, r, t, y, ws, stages, st):
+    """``dab_ipa_fwd_sm100_stages`` with the residue stream x / y in fp32, or in bf16 when that is their dtype."""
+    x32, x16 = (None, x) if x.dtype == torch.bfloat16 else (x, None)
+    y32, y16 = (None, y) if y.dtype == torch.bfloat16 else (y, None)
+    _lib.check(_lib.lib().dab_ipa_fwd_sm100_stages(ctypes.byref(dims), ptr(packed), ptr(x32), ptr(x16), ptr(e), ptr(bias),
+                                                   ptr(r), ptr(t), ptr(y32), ptr(y16), ptr(ws), ws.numel(), stages, st),
+               "dab_ipa_fwd_sm100_stages")
+
+
+def _pair_bias_planes(layers, e, out):
+    """The pair-bias planes of ``layers`` into ``out`` (fp16 (n_layers, B, L, L, H), contiguous) from the bf16 pair
+    tensor ``e``: one pass over it per six layers."""
+    dims = _ipa_structs(layers[0], e.shape[0], e.shape[1])
+    for lo in range(0, len(layers), 6):   # the kernel takes up to six layers per pass
+        hi = min(len(layers), lo + 6)
+        ws = [_lib.dev(l.to_pair_bias.weight.detach(), torch.float32, "to_pair_bias.weight") for l in layers[lo:hi]]
+        w = ws[0] if len(ws) == 1 else torch.stack(ws)
+        _lib.check(_lib.lib().dab_ipa_pair_bias_multi(ctypes.byref(dims), ptr(e), ptr(w), hi - lo, ptr(out[lo:hi]),
+                                                      _lib.stream_ptr()), "dab_ipa_pair_bias_multi")
 
 
 class _IpaFunction(torch.autograd.Function):
@@ -688,9 +714,9 @@ class _PairFanOut(torch.autograd.Function):
 
 
 class _IpaFastFunction(torch.autograd.Function):
-    """bf16 tensor-core IPA layer with gradients: ``dab_ipa_fwd_sm100_train`` / ``dab_ipa_bwd_sm100``.
+    """bf16 tensor-core IPA layer with gradients: ``dab_ipa_fwd_sm100_train`` / ``dab_ipa_bwd_sm100_main`` + ``_finish``.
     Every GEMM of the backward runs in the library's tcgen05 kernels too: the data gradients through ``to_out`` and the
-    six projections on the K-major GEMM (``dab_gemm_bf16``), the weight gradients on the MN-major split-K GEMM
+    six projections on the K-major GEMM (``dab_linear_bf16``), the weight gradients on the MN-major split-K GEMM
     (``dab_gemm_bf16_tn``) - bf16 operands, fp32 accumulation."""
 
     @staticmethod
@@ -788,7 +814,8 @@ class _IpaFastFunction(torch.autograd.Function):
             _lib.check(lib.dab_gemm_bf16_tn_acc(ptr(dy_bf), D, ptr(cat), ncat, ptr(d_w_out), ncat, D, ncat, M, sst),
                        "dab_gemm_bf16_tn_acc (dWout)")
         dcat = torch.empty(M, ncat, device=dev_, dtype=f32)
-        _lib.check(lib.dab_gemm_bf16(ptr(dy_bf), ptr(w_out_t), ptr(dcat), None, M, ncat, D, st), "dab_gemm_bf16 (dcat)")
+        _lib.check(lib.dab_linear_bf16(ptr(dy_bf), ptr(w_out_t), None, 0, M, ncat, D, ptr(dcat), None, st),
+                   "dab_linear_bf16 (dcat)")
         dproj = torch.empty(M, n_proj, device=dev_, dtype=bf)
         de = torch.empty_like(e)
         bws = _lib.aligned_empty(max(lib.dab_ipa_bwd_sm100_workspace_bytes(ctypes.byref(dims)), 16), dev_)
@@ -803,8 +830,8 @@ class _IpaFastFunction(torch.autograd.Function):
         # the longer of the two GEMMs (dWcat, split over K) continues on the main stream without a stream hand-over
         dx = torch.empty(B, L, D, device=dev_, dtype=f32)
         with torch.cuda.stream(side):
-            _lib.check(lib.dab_gemm_bf16(ptr(dproj), ptr(w_cat_t), ptr(dx), None, M, D, n_proj, _lib.stream_ptr()),
-                       "dab_gemm_bf16 (dx)")
+            _lib.check(lib.dab_linear_bf16(ptr(dproj), ptr(w_cat_t), None, 0, M, D, n_proj, ptr(dx), None,
+                                           _lib.stream_ptr()), "dab_linear_bf16 (dx)")
         with torch.cuda.stream(side2):
             _lib.check(lib.dab_ipa_bwd_sm100_finish(*bwd_args, _lib.stream_ptr()), "dab_ipa_bwd_sm100_finish")
         main.wait_event(ev_fill)        # the fill of d_w_cat and the bf16 copy of x: long done
@@ -891,23 +918,19 @@ class InvariantPointAttentionLayer(nn.Module):
             no_grad = not (torch.is_grad_enabled() and (x.requires_grad or e.requires_grad or
                                                         any(w.requires_grad for w in self._weights())))
             Lp = _fast_len(L, no_grad)
-            if Lp is not None and L < Lp and self.fast_path_supported(Lp, no_grad):
+            if Lp is None or not self.fast_path_supported(Lp, no_grad):
+                raise RuntimeError("bf16 pair tensor given but the sm_100a path only supports the train.py configuration "
+                                   "(D=128, C=64, H=8, ds=32, Pq=Pv=8; L <= 128, without gradients L <= 256)")
+            if L < Lp:
                 # shorter patch on the tensor-core kernels: padded to 128 (without gradients: 256) residues, padded keys
                 # masked through the bias plane
-                xp, ep, rp, tp = _pad_patch(x, e, r, t, Lp)
-                with torch.no_grad():
-                    if pair_bias is None:
-                        bias = self.pair_bias(ep.detach())
-                    else:
-                        bias = F.pad(pair_bias, (0, 0, 0, Lp - L, 0, Lp - L))
-                    _mask_padded_keys([bias], L)
-                if Lp == FAST_L2:
-                    return self.forward_fast_io(xp, ep, rp, tp, bias, torch.float32)[:, :L]
-                return self.forward_fast(xp, ep, rp, tp, bias)[:, :L]
-            if L == FAST_L2 and no_grad and self.fast_path_supported(L, True):
-                return self.forward_fast_io(x, e, r, t, pair_bias if pair_bias is not None else self.pair_bias(e),
-                                            torch.float32)
-            return self.forward_fast(x, e, r, t, pair_bias)
+                x, e, r, t, (pair_bias,) = _pad_patch(x, e, r, t, None if pair_bias is None else [pair_bias], Lp,
+                                                      lambda ep: [self.pair_bias(ep)])
+            if no_grad:
+                y = self.forward_fast_io(x, e, r, t, pair_bias, torch.float32)
+            else:
+                y = _IpaFastFunction.apply(self, pair_bias, x, e, r, t, *self._weights())
+            return y[:, :L] if L < Lp else y
         ws = self._weights()
         need_bwd = torch.is_grad_enabled() and (x.requires_grad or e.requires_grad or r.requires_grad or
                                                 t.requires_grad or any(w.requires_grad for w in ws))
@@ -957,50 +980,18 @@ class InvariantPointAttentionLayer(nn.Module):
         The pair tensor is constant over the sampling loop, so ``DiffAb.sample`` computes this once per run."""
         e = _lib.dev(e_bf16, torch.bfloat16, "e")
         B, L = e.shape[0], e.shape[1]
-        dims = _ipa_structs(self, B, L)
         if out is None:
             out = torch.empty(B, L, L, self.n_head, device=e.device, dtype=torch.float16)
         elif out.dtype != torch.float16 or tuple(out.shape) != (B, L, L, self.n_head) or not out.is_contiguous():
             raise ValueError("pair_bias: `out` must be a contiguous fp16 (B, L, L, H) tensor")
-        w = _lib.dev(self.to_pair_bias.weight.detach(), torch.float32, "to_pair_bias.weight")
-        _lib.check(_lib.lib().dab_ipa_pair_bias(ctypes.byref(dims), ptr(e), ptr(w), ptr(out), _lib.stream_ptr()),
-                   "dab_ipa_pair_bias")
+        _pair_bias_planes([self], e, out[None])
         return out
-
-    def forward_fast(self, x, e_bf16, r, t, pair_bias=None):
-        if torch.is_grad_enabled() and (x.requires_grad or e_bf16.requires_grad or
-                                        any(w.requires_grad for w in self._weights())):
-            if not self.fast_path_supported(x.shape[1]):
-                raise RuntimeError("bf16 pair tensor given but the sm_100a path only supports the train.py "
-                                   "configuration (L=128, D=128, C=64, H=8, ds=32, Pq=Pv=8)")
-            return _IpaFastFunction.apply(self, pair_bias, x, e_bf16, r, t, *self._weights())
-        x = _lib.dev(x, torch.float32, "x")
-        e = _lib.dev(e_bf16, torch.bfloat16, "e")
-        r = _lib.dev(r, torch.float32, "r")
-        t = _lib.dev(t, torch.float32, "t")
-        B, L, D = x.shape
-        if not self.fast_path_supported(L):
-            raise RuntimeError("bf16 pair tensor given but the sm_100a fast path only supports the train.py "
-                               "configuration (L=128, D=128, C=64, H=8, ds=32, Pq=Pv=8)")
-        dims = _ipa_structs(self, B, L)
-        lib = _lib.lib()
-        packed = self._packed_weights(dims)
-        nbytes = lib.dab_ipa_sm100_workspace_bytes(ctypes.byref(dims))
-        ws = self._workspace(max(nbytes, 16), x.device)
-        y = torch.empty(B, L, D, device=x.device, dtype=torch.float32)
-        if pair_bias is not None:
-            pair_bias = _lib.dev(pair_bias, torch.float16, "pair_bias")
-            if tuple(pair_bias.shape) != (B, L, L, self.n_head):
-                raise ValueError(f"pair_bias shape {tuple(pair_bias.shape)} != {(B, L, L, self.n_head)}")
-        _lib.check(lib.dab_ipa_fwd_sm100(ctypes.byref(dims), ptr(packed), ptr(x), ptr(e), ptr(pair_bias), ptr(r), ptr(t),
-                                         ptr(y), ptr(ws), ws.numel(), _lib.stream_ptr()), "dab_ipa_fwd_sm100")
-        return y
 
     @torch.no_grad()
     def forward_fast_io(self, x, e_bf16, r, t, pair_bias, out_dtype):
         """Inference on the sm_100a path with the residue stream in fp32 or bf16 on either side (``x.dtype`` /
         ``out_dtype``): the layers of a stack hand it over already rounded to bf16 - what the next layer's projections
-        consume anyway, so no bit of the result changes - via ``dab_ipa_fwd_sm100_io``."""
+        consume anyway, so no bit of the result changes.  ``pair_bias`` None: the library builds this layer's plane."""
         B, L, D = x.shape
         if not self.fast_path_supported(L, True):
             raise RuntimeError("the sm_100a fast path only supports the train.py configuration")
@@ -1009,16 +1000,14 @@ class InvariantPointAttentionLayer(nn.Module):
         r = _lib.dev(r, torch.float32, "r")
         t = _lib.dev(t, torch.float32, "t")
         bias = None if pair_bias is None else _lib.dev(pair_bias, torch.float16, "pair_bias")
+        if bias is not None and tuple(bias.shape) != (B, L, L, self.n_head):
+            raise ValueError(f"pair_bias shape {tuple(bias.shape)} != {(B, L, L, self.n_head)}")
         dims = _ipa_structs(self, B, L)
-        lib = _lib.lib()
         packed = self._packed_weights(dims)
-        ws = self._workspace(max(lib.dab_ipa_sm100_workspace_bytes(ctypes.byref(dims)), 16), x.device)
+        ws = self._workspace(max(_lib.lib().dab_ipa_sm100_workspace_bytes(ctypes.byref(dims)), 16), x.device)
         y = torch.empty(B, L, D, device=x.device, dtype=out_dtype)
-        x32, x16 = (None, x) if x.dtype == torch.bfloat16 else (x, None)
-        y32, y16 = (None, y) if out_dtype == torch.bfloat16 else (y, None)
-        _lib.check(lib.dab_ipa_fwd_sm100_io(ctypes.byref(dims), ptr(packed), ptr(x32), ptr(x16), ptr(e), ptr(bias), ptr(r),
-                                            ptr(t), ptr(y32), ptr(y16), ptr(ws), ws.numel(), _lib.stream_ptr()),
-                   "dab_ipa_fwd_sm100_io")
+        if B > 0:   # (an empty tensor's data pointer is NULL: the library would read x / y as not given)
+            _fwd_stages(dims, packed, x, e, bias, r, t, y, ws, 7, _lib.stream_ptr())
         return y
 
 
@@ -1041,14 +1030,8 @@ class InvariantPointAttentionModule(nn.Module):
                 self.layers[0].fast_path_supported(Lp, not needs_grad)):
             # shorter patches on the tensor-core kernels: pad once for the whole stack (to 128, without gradients to 256
             # residues), mask the padded keys in every layer's bias plane, slice the result
-            xp, ep, rp, tp = _pad_patch(res_emb, pair_emb, orientations, translations, Lp)
-            with torch.no_grad():
-                if pair_bias is None:
-                    planes = self.precompute_pair_bias(ep.detach())
-                else:
-                    planes = [F.pad(p_, (0, 0, 0, Lp - L, 0, Lp - L)) for p_ in pair_bias]
-                _mask_padded_keys(planes, L)
-            return self.forward(xp, ep, rp, tp, planes)[:, :L]
+            padded = _pad_patch(res_emb, pair_emb, orientations, translations, pair_bias, Lp, self.precompute_pair_bias)
+            return self.forward(*padded)[:, :L]
         if (pair_bias is None and pair_emb.dtype == torch.bfloat16 and
                 self.layers[0].fast_path_supported(pair_emb.shape[1], not needs_grad)):
             # tensor-core path: the bias planes of all layers in one pass over the pair tensor (their gradient
@@ -1105,15 +1088,13 @@ class InvariantPointAttentionModule(nn.Module):
         packed = [layer._packed_weights(dims) for layer in layers]
         ws = layers[0]._workspace(max(lib.dab_ipa_sm100_workspace_bytes(ctypes.byref(dims)), 16), e.device)
         y = torch.empty(B, L, D, device=e.device, dtype=torch.float32)
-        x32 = x16 = None
         if front is None:
             x = _lib.dev(res_emb, res_emb.dtype if res_emb.dtype == torch.bfloat16 else torch.float32, "x")
-            x32, x16 = (None, x) if x.dtype == torch.bfloat16 else (x, None)
+        else:
+            x = ws                  # (stages 2 / 4 do not read x: any non-null pointer satisfies the argument check)
 
         def stage(k, stages):     # (x is read by stage 1 only, y written by stage 4 only)
-            _lib.check(lib.dab_ipa_fwd_sm100_stages(
-                ctypes.byref(dims), ptr(packed[k]), ptr(x32), ptr(x16), ptr(e), ptr(bias[k]), ptr(r), ptr(t), ptr(y), None,
-                ptr(ws), ws.numel(), stages, st), "dab_ipa_fwd_sm100_stages")
+            _fwd_stages(dims, packed[k], x, e, bias[k], r, t, y, ws, stages, st)
 
         if front is None:
             stage(0, 1)
@@ -1122,7 +1103,6 @@ class InvariantPointAttentionModule(nn.Module):
             _lib.check(lib.dab_ipa_front_proj_sm100(
                 ctypes.byref(dims), ptr(packed[0]), ptr(cache["c"]), ptr(cache["t1"]), ptr(_lib.dev(seq, torch.int64, "seq_idx")),
                 ptr(cache["w2_bf16"]), ptr(cache["b2"]), ptr(r), ptr(t), ptr(ws), ws.numel(), st), "dab_ipa_front_proj_sm100")
-            x16 = ws                # (stages 2 / 4 do not read x: any non-null pointer satisfies the argument check)
         for k in range(n):
             stage(k, 2)
             if k + 1 < n:
@@ -1159,14 +1139,7 @@ class InvariantPointAttentionModule(nn.Module):
             out = torch.empty(n, B, L, L, H, device=e.device, dtype=torch.float16)
         elif out.dtype != torch.float16 or tuple(out.shape) != (n, B, L, L, H) or not out.is_contiguous():
             raise ValueError("precompute_pair_bias: `out` must be a contiguous fp16 (n_layers, B, L, L, H) tensor")
-        lib = _lib.lib()
-        dims = _ipa_structs(self.layers[0], B, L)
-        for lo in range(0, n, 6):   # the kernel takes up to six layers per pass
-            hi = min(n, lo + 6)
-            w = torch.stack([_lib.dev(l.to_pair_bias.weight.detach(), torch.float32, "to_pair_bias.weight")
-                             for l in self.layers[lo:hi]]).contiguous()
-            _lib.check(lib.dab_ipa_pair_bias_multi(ctypes.byref(dims), ptr(e), ptr(w), hi - lo, ptr(out[lo:hi]),
-                                                   _lib.stream_ptr()), "dab_ipa_pair_bias_multi")
+        _pair_bias_planes(self.layers, e, out)
         return list(out.unbind(0))
 
 
@@ -1227,8 +1200,6 @@ class Denoiser(nn.Module):
                 o.record_stream(main)
         return tuple(outs)
 
-    fuse_out_into_heads = True     # False: to_out of the last layer as its own GEMM in front of the heads kernel (timing A/B)
-
     # ---- sampling fast path of the dense glue (same arithmetic, regrouped; inference only) ----
     @torch.no_grad()
     def sampling_cache(self, res_context_emb, cache=None):
@@ -1285,7 +1256,7 @@ class Denoiser(nn.Module):
                 self.ipa.fused_stack_applicable(B, L, pair_context_emb, pair_bias)):
             # large batches: the front MLP runs inside the first layer's projection kernel (same bits as the branch below)
             front = (cache, seq_idx_t.contiguous())
-            if cache.get("heads_packed") is not None and self.fuse_out_into_heads:
+            if cache.get("heads_packed") is not None:
                 # ... and the last layer's to_out inside the heads kernel: the stack's output never exists in HBM either
                 nb = L // FAST_L
                 beta_blk = beta.contiguous() if nb == 1 else beta.repeat_interleave(nb)

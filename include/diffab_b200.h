@@ -162,12 +162,13 @@ int dab_ipa_bwd_f32(const DabIpaDims* d, const DabIpaWeights* w, const float* x,
  * split-bf16 point-distance logits, fp32 softmax.  `packed` is produced once per layer by
  * dab_ipa_pack_weights (weights are constant during sampling).  x[B,L,D] fp32 in, y[B,L,D] fp32
  * out, e_bf16[B,L,L,C] bf16.
- * The inference entry points (dab_ipa_fwd_sm100, _io, _stages, dab_ipa_mid_sm100, dab_ipa_pair_bias*, the packing and
- * workspace functions) also take L = 256 - the reference's preprocessed patches have 128..256 residues
- * (preprocess_pdb.py:48-58; shorter ones are padded by the caller with -inf in the padded keys' bias columns): a patch is
- * then two blocks of 128 residues - block-wise projections centred on the patch centroid, the attention core once per
- * (query block, key block) pair, the two key blocks' results merged by their softmax statistics (exact for the scalar,
- * pair and local-frame point features; point norms recomputed).  The training pair (_train / dab_ipa_bwd_sm100) is L = 128. */
+ * The inference entry points (dab_ipa_fwd_sm100_stages, dab_ipa_mid_sm100, dab_ipa_front_proj_sm100,
+ * dab_ipa_pair_bias_multi, the packing and workspace functions) also take L = 256 - the reference's preprocessed patches
+ * have 128..256 residues (preprocess_pdb.py:48-58; shorter ones are padded by the caller with -inf in the padded keys'
+ * bias columns): a patch is then two blocks of 128 residues - block-wise projections centred on the patch centroid, the
+ * attention core once per (query block, key block) pair, the two key blocks' results merged by their softmax statistics
+ * (exact for the scalar, pair and local-frame point features; point norms recomputed).  The training pair
+ * (dab_ipa_fwd_sm100_train / dab_ipa_bwd_sm100_main + _finish) is L = 128. */
 size_t dab_ipa_packed_bytes(const DabIpaDims* d);
 int dab_ipa_pack_weights(const DabIpaDims* d, const DabIpaWeights* w, void* packed, void* stream);
 /* offs[0..6]: byte offsets of Wcat bf16 [1344][128] (rows in the order to_q_scalar, to_k_scalar, to_v_scalar, to_q_point,
@@ -175,34 +176,26 @@ int dab_ipa_pack_weights(const DabIpaDims* d, const DabIpaWeights* w, void* pack
  * `packed` - the caller's own backward GEMMs reuse the bf16 copies instead of casting the weights again. */
 int dab_ipa_packed_layout(const DabIpaDims* d, size_t* offs);
 size_t dab_ipa_sm100_workspace_bytes(const DabIpaDims* d);
-/* Pair bias of one layer, hoisted out of the sampling loop: bias_f16[B*L*L*8] (fp16, [b][i][j][h]) =
- * scale_total * log2(e) * e . w_pair_bias^T (to_pair_bias, diffab_pytorch.py:423,439).  The pair tensor is
- * constant over the T reverse steps, so this is computed once per sampling run per layer. */
-int dab_ipa_pair_bias(const DabIpaDims* d, const void* e_bf16, const float* w_pair_bias, void* bias_f16, void* stream);
-/* Same for n_layers <= 6 layers in ONE pass over the pair tensor (the six layers of the epsilon network share it):
- * w_pair_bias[n_layers][8][64] fp32 contiguous, planes_f16[n_layers][B*L*L][8] fp16 contiguous. */
+/* Pair bias of n_layers <= 6 layers in ONE pass over the pair tensor (the six layers of the epsilon network share it),
+ * hoisted out of the sampling loop: planes_f16[n_layers][B*L*L][8] (fp16, [b][i][j][h] per layer) =
+ * scale_total * log2(e) * e . w_pair_bias^T (to_pair_bias, diffab_pytorch.py:423,439), w_pair_bias[n_layers][8][64] fp32
+ * contiguous.  The pair tensor is constant over the T reverse steps, so this is computed once per sampling run. */
 int dab_ipa_pair_bias_multi(const DabIpaDims* d, const void* e_bf16, const float* w_pair_bias, int n_layers,
                             void* planes_f16, void* stream);
-/* bias_f16: the layer's plane from dab_ipa_pair_bias, or NULL (then it is rebuilt inside the call). */
-int dab_ipa_fwd_sm100(const DabIpaDims* d, const void* packed, const float* x, const void* e_bf16,
-                      const void* bias_f16, const float* R, const float* t, float* y, void* workspace,
-                      size_t workspace_bytes, void* stream);
-/* dab_ipa_fwd_sm100 with the residue stream in bf16 on either side (exactly one of x / x_bf16 and one of y / y_bf16 non-NULL):
- * used between the layers of InvariantPointAttentionModule (diffab_pytorch.py:494-498), where the next layer's projections
- * consume x as bf16 anyway - same bits, half the traffic. */
-int dab_ipa_fwd_sm100_io(const DabIpaDims* d, const void* packed, const float* x, const void* x_bf16, const void* e_bf16,
-                         const void* bias_f16, const float* R, const float* t, float* y, void* y_bf16, void* workspace,
-                         size_t workspace_bytes, void* stream);
-/* The same layer launch by launch: `stages` = bit0 projections + frame transform, bit1 attention core, bit2 to_out; the
- * workspace must hold the products of the lower stages (an earlier call).  For callers that bracket one stage with their
- * own events (bench.py's roofline of the attention core) - there is no process-global measurement state in the library. */
+/* Inference forward of one layer, whole (stages = 7) or launch by launch: `stages` = bit0 projections + frame transform,
+ * bit1 attention core, bit2 to_out; the workspace must hold the products of the lower stages (an earlier call).  For
+ * callers that bracket one stage with their own events (bench.py's roofline of the attention core) - there is no
+ * process-global measurement state in the library.  bias_f16: the layer's plane from dab_ipa_pair_bias_multi, or NULL
+ * (then it is rebuilt inside the call).  The residue stream is fp32 or bf16 on either side (exactly one of x / x_bf16 and
+ * one of y / y_bf16 non-NULL): between the layers of InvariantPointAttentionModule (diffab_pytorch.py:494-498) the next
+ * layer's projections consume x as bf16 anyway - same bits, half the traffic. */
 int dab_ipa_fwd_sm100_stages(const DabIpaDims* d, const void* packed, const float* x, const void* x_bf16, const void* e_bf16,
                              const void* bias_f16, const float* R, const float* t, float* y, void* y_bf16, void* workspace,
                              size_t workspace_bytes, int stages, void* stream);
 /* Between two layers of a stack (inference): the previous layer's to_out (`packed_prev`; input = the concat features its
  * attention core left in `workspace`) fused into this layer's projection kernel (`packed`): y is rounded to bf16 as
- * dab_ipa_fwd_sm100_io would hand it over but never exists in HBM.  Stack = stages(1) of layer 0, then per layer stages(2)
- * + dab_ipa_mid_sm100 (stages(4) after the last layer); bit-identical to the unfused sequence
+ * dab_ipa_fwd_sm100_stages would hand it over (y_bf16) but never exists in HBM.  Stack = stages(1) of layer 0, then per
+ * layer stages(2) + dab_ipa_mid_sm100 (stages(4) after the last layer); bit-identical to the unfused sequence
  * (InvariantPointAttentionModule.forward, diffab_pytorch.py:494-498). */
 int dab_ipa_mid_sm100(const DabIpaDims* d, const void* packed_prev, const void* packed, const float* R, const float* t,
                       void* workspace, size_t workspace_bytes, void* stream);
@@ -213,8 +206,8 @@ int dab_ipa_mid_sm100(const DabIpaDims* d, const void* packed_prev, const void* 
 int dab_ipa_front_proj_sm100(const DabIpaDims* d, const void* packed, const float* c, const float* t1, const int64_t* seq,
                              const void* w2_bf16, const float* b2, const float* R, const float* t, void* workspace,
                              size_t workspace_bytes, void* stream);
-/* Training pair of the sm_100a path (bf16 pair tensor, fp32 x / y).  The forward is dab_ipa_fwd_sm100 (the pair
- * bias is rebuilt inside the call when bias_f16 is NULL); `saved` (dab_ipa_sm100_workspace_bytes) additionally keeps
+/* Training pair of the sm_100a path (bf16 pair tensor, fp32 x / y).  The forward is dab_ipa_fwd_sm100_stages(.., 7) (the
+ * pair bias is rebuilt inside the call when bias_f16 is NULL); `saved` (dab_ipa_sm100_workspace_bytes) additionally keeps
  * the packed operands, the concat features, the un-normalised probabilities and the softmax statistics, and must
  * reach the backward untouched. */
 int dab_ipa_fwd_sm100_train(const DabIpaDims* d, const void* packed, const float* x, const void* e_bf16,
@@ -230,10 +223,7 @@ int dab_ipa_fwd_sm100_train(const DabIpaDims* d, const void* packed, const float
  * R and t are treated as constants, as in dab_ipa_bwd_f32. */
 int dab_ipa_sm100_workspace_layout(const DabIpaDims* d, size_t* offsets /* 8: Qp, Kp, Vp, tc, cat, bias, stats, pu */);
 size_t dab_ipa_bwd_sm100_workspace_bytes(const DabIpaDims* d);
-int dab_ipa_bwd_sm100(const DabIpaDims* d, const void* packed, const void* e_bf16, const float* R, const float* dcat,
-                      void* saved, size_t saved_bytes, void* dproj_bf16, void* de_bf16, float* d_w_pair_bias, float* d_gamma,
-                      void* workspace, size_t workspace_bytes, void* stream);
-/* The same backward in two calls (same arguments): `_main` = everything up to dproj / de and the per-CTA partial sums,
+/* The backward in two calls (same arguments): `_main` = everything up to dproj / de and the per-CTA partial sums,
  * `_finish` = d_w_pair_bias / d_gamma from those sums - lets the caller overlap the final reductions with the GEMMs that
  * depend only on dproj (dx, dWcat). */
 int dab_ipa_bwd_sm100_main(const DabIpaDims* d, const void* packed, const void* e_bf16, const float* R, const float* dcat,
@@ -273,7 +263,7 @@ int dab_out_heads_fwd_sm100(const void* packed, const void* cat_bf16, const void
  * x0[n_rows,128] = relu(c[row] + t1[seq[row]]) . w2^T + b2, where c = res_ctx . W1[:, :128]^T + b1 (per-run constant,
  * fp32 [n_rows,128]) and t1 = emb . W1[:, 128:]^T (fp32 [25,128]) are computed once per run by the caller;
  * w2_bf16 = to_res_emb.2.weight in bf16 [128][128]; a_scratch holds n_rows*128 bf16.  Exactly one of x0 (fp32) and
- * x0_bf16 (the same values rounded to bf16, the form dab_ipa_fwd_sm100_io takes) is non-NULL. */
+ * x0_bf16 (the same values rounded to bf16, the form dab_ipa_fwd_sm100_stages takes as x_bf16) is non-NULL. */
 int dab_front_fwd_sm100(const float* c, const float* t1, const int64_t* seq, int64_t n_rows, const void* w2_bf16,
                         const float* b2, void* a_scratch, float* x0, void* x0_bf16, void* stream);
 
@@ -372,9 +362,6 @@ int dab_losses_bwd(const float* post_pred, const float* post_tgt, const float* e
 int dab_adam_flat(float* p, const float* g, float* m, float* v, const float* step, float lr, float beta1, float beta2,
                   float eps, float weight_decay, int64_t n, void* stream);
 
-/* The tcgen05 GEMM C[M,N] = A[M,K] B[N,K]^T + bias (bf16 in, fp32 out; M % 128 == 0, N % 64 == 0, K % 64 == 0): nn.Linear
- * (diffab_pytorch.py:464) as a stand-alone entry point. */
-int dab_gemm_bf16(const void* A, const void* Bm, float* C, const float* bias, int M, int N, int K, void* stream);
 /* C[M,N] (fp32, overwritten) = A[K,M]^T B[K,N]: bf16 operands whose ROW index is the contraction index (activations as
  * they lie in memory, one row per residue), read MN-major by tcgen05 - no transposed copies.  Split over K, partial tiles
  * added with red.global (summation order not fixed).  K % 64 == 0, N % 64 == 0, lda % 8 == 0, ldb % 8 == 0, ldc % 4 == 0,
@@ -392,7 +379,8 @@ int dab_colsum_f32(const float* x, int64_t rows, int cols, float* out, void* x_b
  * diffab_pytorch.py:57-183,572-599) on the library's tcgen05 GEMM.
  * dab_linear_bf16: C = act(A[M,K] W[N,K]^T + bias), bf16 operands, fp32 accumulation; act = ReLU when relu != 0; the result as
  *   fp32 (C_f32) or rounded to bf16 (C_bf16), exactly one of the two non-NULL.  M % 128 == 0, N % 64 == 0, K % 64 == 0.
- *   Forward y = x W^T + b, and with W transposed the data gradient dx = g W.
+ *   Forward y = x W^T + b, and with W transposed the data gradient dx = g W (also of the IPA layer's nn.Linear layers,
+ *   diffab_pytorch.py:391-408,464).
  * dab_bias_grad: g' = g * (y > 0) (y_bf16 = the layer's ReLU output, NULL: no mask), db[cols] (fp32, overwritten) = column
  *   sums of g', g_out_bf16 (optional) = g' rounded to bf16 (the operand of dx = g' W and dW = g'^T x, dab_gemm_bf16_tn).
  *   g: fp32 (g_is_bf16 = 0) or bf16, [rows, cols] contiguous; cols % 4 == 0 (8 for bf16 input), <= 1024. */

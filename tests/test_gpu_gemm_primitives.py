@@ -1,6 +1,6 @@
 """The small primitives every gradient of a mixed-precision training step passes through, called directly and compared
 with float64 references computed from the exact values each kernel was given:
-  dab_gemm_bf16 / dab_linear_bf16 (K-major tcgen05 GEMM, every epilogue), dab_gemm_bf16_tn / _acc (MN-major split-K
+  dab_linear_bf16 (K-major tcgen05 GEMM, every epilogue), dab_gemm_bf16_tn / _acc (MN-major split-K
   weight-gradient GEMM), dab_colsum_f32 / dab_bias_grad (column sums, ReLU mask, bf16 copy), dab_cast_f32_to_bf16,
   dab_sum_bf16, dab_relu_bwd_colsum, dab_pair_zero_masked;
 and the to_out gradients of the bf16 IPA training layer, which are plain products and sums of what the layer holds.
@@ -72,7 +72,8 @@ def _gemm(A, W, bias=None):
     M, K = A.shape
     N = W.shape[0]
     C = torch.full((M, N), NAN, device=DEV)
-    _lib.check(_lib.lib().dab_gemm_bf16(ptr(A), ptr(W), ptr(C), ptr(bias), M, N, K, _lib.stream_ptr()), "dab_gemm_bf16")
+    _lib.check(_lib.lib().dab_linear_bf16(ptr(A), ptr(W), ptr(bias), 0, M, N, K, ptr(C), None, _lib.stream_ptr()),
+               "dab_linear_bf16")
     return C
 
 
@@ -129,8 +130,6 @@ def test_kmajor_gemm_rejects_unsupported_shapes(M, N, K):
     C = torch.zeros(Mp, 128, device=DEV)
     msg = rf"gemm_bf16: M % 128, N % \d+, K % 64 required \(M={M} N={N} K={K}\)"
     lib = _lib.lib()
-    with pytest.raises(RuntimeError, match=msg):
-        _lib.check(lib.dab_gemm_bf16(ptr(A), ptr(W), ptr(C), None, M, N, K, _lib.stream_ptr()), "dab_gemm_bf16")
     with pytest.raises(RuntimeError, match=msg):
         _lib.check(lib.dab_linear_bf16(ptr(A), ptr(W), None, 0, M, N, K, ptr(C), None, _lib.stream_ptr()), "dab_linear_bf16")
     torch.cuda.synchronize()

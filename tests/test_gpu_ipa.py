@@ -126,8 +126,8 @@ def test_tensor_core_path_vs_fp32_kernel_and_reference():
 
 
 def test_tensor_core_backward_vs_reference_autograd():
-    """bf16 tcgen05 training path (dab_ipa_fwd_sm100_train / dab_ipa_bwd_sm100): every gradient against the fp64
-    autograd of the oracle evaluated on the bf16-rounded pair tensor.  Tolerance: 2e-2 max-normalised per tensor
+    """bf16 tcgen05 training path (dab_ipa_fwd_sm100_train / dab_ipa_bwd_sm100_main + _finish): every gradient against
+    the fp64 autograd of the oracle evaluated on the bf16-rounded pair tensor.  Tolerance: 2e-2 max-normalised per tensor
     (north_star's bound for the bf16 path); measured ~1e-2 on the point-projection weights, ~5e-3 elsewhere."""
     g, c, layer, x, e, R, t, gy = _case("train")
     e16 = e.to(torch.bfloat16)
@@ -210,8 +210,8 @@ def test_tensor_core_layer_full_size_properties():
 
 def test_layer_stack_bf16_handoff_changes_no_bit():
     """Inference through InvariantPointAttentionModule hands the residue stream from layer to layer as bf16
-    (dab_ipa_fwd_sm100_io: the to_out GEMM rounds, the next projections copy); the projections round their fp32 input
-    the same way, so the result must equal the layer-by-layer fp32 hand-off bit for bit."""
+    (dab_ipa_fwd_sm100_stages with y_bf16: the to_out GEMM rounds, the next projections copy); the projections round
+    their fp32 input the same way, so the result must equal the layer-by-layer fp32 hand-off bit for bit."""
     torch.manual_seed(2)
     B = 4
     mod = InvariantPointAttentionModule(4, 128, 64, 32, 8, 8, 8).to(DEV)

@@ -101,8 +101,5 @@ with torch.no_grad():
     parts = [timed(front, "front MLP (act + GEMM)"), timed(stack, "IPA stack (6 layers)"), timed(heads, "heads"),
              timed(update, "IGSO(3) draw + reverse-step update")]
     e = timed(eps_net, "epsilon network (front+stack+heads)")
-    type(den).fuse_out_into_heads = False
-    timed(eps_net, "  ... last to_out as its own GEMM")
-    type(den).fuse_out_into_heads = True
     w = timed(whole, "whole reverse step")
     print(f"  sum of the four parts {sum(parts):.1f} us; epsilon network {e:.1f}; whole step {w:.1f}")
