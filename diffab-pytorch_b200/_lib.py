@@ -79,6 +79,7 @@ EXPORTS = {
     "dab_ipa_pair_bias_multi": (c_int, [POINTER(DabIpaDims), c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "dab_ipa_mid_sm100": (c_int, [POINTER(DabIpaDims), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "dab_ipa_fwd_sm100_stages": (c_int, [POINTER(DabIpaDims)] + [c_void_p] * 10 + [c_size_t, c_int, c_void_p]),
+    "dab_ipa_core_sm100_live": (c_int, [POINTER(DabIpaDims)] + [c_void_p] * 6 + [c_size_t, c_void_p, c_void_p, c_void_p]),
     "dab_ipa_fwd_sm100_train": (c_int, [POINTER(DabIpaDims), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                         c_void_p, c_void_p, c_size_t, c_void_p]),
     "dab_ipa_sm100_workspace_layout": (c_int, [POINTER(DabIpaDims), POINTER(c_size_t)]),
@@ -113,7 +114,7 @@ EXPORTS = {
     "dab_losses_bwd": (c_int, [c_void_p] * 7 + [c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "dab_adam_flat": (c_int, [c_void_p] * 5 + [c_float] * 5 + [c_int64, c_void_p]),
     "dab_cast_f32_to_bf16": (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
-    "dab_out_heads_fwd_sm100": (c_int, [c_void_p] * 5 + [c_int, c_int] + [c_void_p] * 4),
+    "dab_out_heads_fwd_sm100": (c_int, [c_void_p] * 5 + [c_int, c_int] + [c_void_p] * 6),
     "dab_ipa_front_proj_sm100": (c_int, [c_void_p] * 10 + [c_size_t, c_void_p]),
     "dab_gemm_bf16_tn": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int, c_int, c_int, c_void_p]),
     "dab_gemm_bf16_tn_acc": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int, c_int, c_int, c_void_p]),

@@ -40,8 +40,9 @@ struct HeadsSmem {
   static constexpr int kA2 = 32768;            // layer-2 activations of the current head
   static constexpr int kW = 65536;             // ring of two [2 kb][128 rows][128 B] weight tiles
   static constexpr int kW3 = kW + 2 * 32768;   // three [2 kb][32 rows][128 B] last-layer tiles
-  static constexpr int kPb = kW3 + 3 * 8192;   // fp32 [384]: b1 + Wt1 . (beta, sin beta, cos beta)
-  static constexpr int kBars = kPb + 384 * 4;
+  static constexpr int kPb = kW3 + 3 * 8192;   // fp32 [8 slots][384]: b1 + Wt1 . (beta, sin beta, cos beta) per block
+  static constexpr int kTile = kPb + 8 * 384 * 4;   // int [8]: the tile of each 16-row slot (live-tile mode)
+  static constexpr int kBars = kTile + 8 * 4;
   static constexpr int kTmemSlot = kBars + 32 * 8;
   static constexpr int kTotal = kTmemSlot + 16;
 };
@@ -91,12 +92,17 @@ __global__ void pack_heads_kernel(DabHeadWeights w, uint8_t* packed) {
 
 // grid = patches (128 residues each); 288 threads: warps 0-7 = epilogue (thread = residue row x column half),
 // warp 8 lane 0 = TMA producer + tcgen05.mma issuer.
+// Live-tile mode (fuse_out only; `tiles` = ascending ids of 16-row tiles, global row / 16, `tile_count` = their number):
+// CTA b takes tiles 8 b .. 8 b + 7 of the list - still 128 MMA rows, the cat rows arrive as eight 16-row boxes (map_cat
+// has a 16-row box then) - and writes only their rows; a short last group repeats its last tile in the unused slots and
+// masks their writes, CTAs past the end of the list exit.  Every MMA row depends on its own A row only: the same bits.
 __global__ void __launch_bounds__(288, 1)
 denoiser_heads_kernel(const __grid_constant__ CUtensorMap map_w128, const __grid_constant__ CUtensorMap map_w32,
                       const float* __restrict__ x, const float* __restrict__ beta, const uint8_t* __restrict__ packed,
                       float* __restrict__ eps, float* __restrict__ rotvec, float* __restrict__ post,
                       const __grid_constant__ CUtensorMap map_cat, const __grid_constant__ CUtensorMap map_wout,
-                      const float* __restrict__ b_out, int fuse_out) {
+                      const float* __restrict__ b_out, int fuse_out, const int* __restrict__ tiles,
+                      const int* __restrict__ tile_count) {
   extern __shared__ __align__(1024) uint8_t smem[];
   using S = HeadsSmem;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + S::kBars);
@@ -104,6 +110,9 @@ denoiser_heads_kernel(const __grid_constant__ CUtensorMap map_w128, const __grid
   float* s_pb = reinterpret_cast<float*>(smem + S::kPb);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int b = blockIdx.x;
+  const int n_live = tiles ? __ldg(tile_count) - 8 * b : 8;    // slots of this CTA that hold a tile of the list
+  if (n_live <= 0) return;
+  int* s_tile = reinterpret_cast<int*>(smem + S::kTile);
   const uint32_t smem_base = smem_u32(smem);
   if ((smem_base & 1023u) != 0) asm volatile("trap;");
   const float* b2 = reinterpret_cast<const float*>(packed + HeadsPacked::kB2);
@@ -128,12 +137,7 @@ denoiser_heads_kernel(const __grid_constant__ CUtensorMap map_w128, const __grid
             make_uint2(hpk(v.x, v.y), hpk(v.z, v.w));
       }
     }
-    // per-patch bias of the first layers: the three time columns of [x | beta, sin beta, cos beta]
-    const float* wt1 = reinterpret_cast<const float*>(packed + HeadsPacked::kWt1);
-    const float* b1 = reinterpret_cast<const float*>(packed + HeadsPacked::kB1);
-    const float bt = __ldg(beta + b), sb = sinf(bt), cb = cosf(bt);
-    for (int i = tid; i < 384; i += 256)
-      s_pb[i] = __ldg(b1 + i) + __ldg(wt1 + i * 3) * bt + __ldg(wt1 + i * 3 + 1) * sb + __ldg(wt1 + i * 3 + 2) * cb;
+    if (tiles && tid < 8) s_tile[tid] = __ldg(tiles + 8 * b + min(tid, n_live - 1));
     fence_proxy_async_smem();
   }
   tcgen05_fence_before_sync();
@@ -153,7 +157,12 @@ denoiser_heads_kernel(const __grid_constant__ CUtensorMap map_w128, const __grid
         auto load_g = [&](int kc) {
           const int st = kc % 3;
           mbar_arrive_expect_tx(&bars[HG_FULL + st], 32768);
-          tma_load_2d(smem + g_off[st], &map_cat, &bars[HG_FULL + st], kc * 64, b * 128);
+          if (tiles) {
+            for (int sl = 0; sl < 8; ++sl)     // 2 KB boxes: the 128B swizzle repeats every 8 rows, the layout is unchanged
+              tma_load_2d(smem + g_off[st] + sl * 2048, &map_cat, &bars[HG_FULL + st], kc * 64, s_tile[sl] * 16);
+          } else {
+            tma_load_2d(smem + g_off[st], &map_cat, &bars[HG_FULL + st], kc * 64, b * 128);
+          }
           tma_load_2d(smem + g_off[st] + 16384, &map_wout, &bars[HG_FULL + st], kc * 64, 0);
         };
         for (int kc = 0; kc < 3; ++kc) load_g(kc);
@@ -241,7 +250,10 @@ denoiser_heads_kernel(const __grid_constant__ CUtensorMap map_w128, const __grid
   } else {
     const int row = tid & 127, chalf = tid >> 7;           // column half = K block of the next layer's A operand
     const uint32_t tmem_lane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-    const int64_t grow = (int64_t)b * 128 + row;
+    const int slot = row >> 4;
+    const int64_t grow = tiles ? (int64_t)s_tile[slot] * 16 + (row & 15) : (int64_t)b * 128 + row;
+    const bool write = slot < n_live;
+    const float* pb = s_pb + (tiles ? slot * 384 : 0);
     // bias + relu on 64 accumulator columns -> bf16 -> row `row` of K block `chalf` of an A operand
     auto relu_to_smem = [&](uint32_t col0, const float* bias, bool bias_in_smem, uint8_t* dst) {
 #pragma unroll
@@ -263,6 +275,18 @@ denoiser_heads_kernel(const __grid_constant__ CUtensorMap map_w128, const __grid
         }
       }
     };
+    {
+      // per-block bias of the first layers: the three time columns of [x | beta, sin beta, cos beta]; one vector per
+      // 16-row slot in live-tile mode (the slots may come from different blocks)
+      const float* wt1 = reinterpret_cast<const float*>(packed + HeadsPacked::kWt1);
+      const float* b1 = reinterpret_cast<const float*>(packed + HeadsPacked::kB1);
+      for (int sl = 0; sl < (tiles ? 8 : 1); ++sl) {
+        const float bt = __ldg(beta + (tiles ? s_tile[sl] >> 3 : b)), sb = sinf(bt), cb = cosf(bt);
+        for (int i = tid; i < 384; i += 256)
+          s_pb[sl * 384 + i] = __ldg(b1 + i) + __ldg(wt1 + i * 3) * bt + __ldg(wt1 + i * 3 + 1) * sb + __ldg(wt1 + i * 3 + 2) * cb;
+      }
+      asm volatile("bar.sync 1, 256;" ::: "memory");    // the epilogue warps read each other's entries
+    }
     if (fuse_out) {
       // y = acc + b_out of the last IPA layer, rounded to bf16 exactly as the heads would round its fp32 output, goes
       // straight into the A tile: this thread converts its row of K block `chalf`
@@ -289,7 +313,7 @@ denoiser_heads_kernel(const __grid_constant__ CUtensorMap map_w128, const __grid
     tcgen05_fence_after_sync();
     for (int k = 0; k < 3; ++k) {
       // layer-1 activations of head k (its A1 buffer is free: the previous head's second layer has completed)
-      relu_to_smem(k * 128 + chalf * 64, s_pb + k * 128 + chalf * 64, true, smem + S::kA);
+      relu_to_smem(k * 128 + chalf * 64, pb + k * 128 + chalf * 64, true, smem + S::kA);
       fence_proxy_async_smem();
       tcgen05_fence_before_sync();
       mbar_arrive(&bars[HA1_READY]);
@@ -305,11 +329,11 @@ denoiser_heads_kernel(const __grid_constant__ CUtensorMap map_w128, const __grid
         float v[32];
         tmem_ld_x32(tmem_lane + 384 + k * HN3, v);
         tmem_wait_ld();
-        if (k < 2) {
+        if (write && k < 2) {
           float* dst = (k == 0 ? eps : rotvec) + grow * 3;
 #pragma unroll
           for (int c = 0; c < 3; ++c) dst[c] = v[c] + __ldg(b3 + k * HN3 + c);
-        } else {                                   // nn.Softmax(dim=-1) over the 21 classes (:599)
+        } else if (write) {                        // nn.Softmax(dim=-1) over the 21 classes (:599)
           float mx = -INFINITY;
 #pragma unroll
           for (int c = 0; c < DAB_VOCAB; ++c) { v[c] += __ldg(b3 + 2 * HN3 + c); mx = fmaxf(mx, v[c]); }
@@ -380,7 +404,7 @@ int dab_heads_fwd_sm100(const void* packed, const float* x, const float* beta, i
   if (int rc = make_tensor_map_bf16(&m32, pk + HeadsPacked::kW, 2, dims, strides, b32, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
   DAB_ENSURE_SMEM(denoiser_heads_kernel, HeadsSmem::kTotal);
   denoiser_heads_kernel<<<n_patches, 288, HeadsSmem::kTotal, (cudaStream_t)stream>>>(m128, m32, x, beta, pk, eps, rotvec, post,
-                                                                                      m128, m128, nullptr, 0);
+                                                                                      m128, m128, nullptr, 0, nullptr, nullptr);
   count_launch();
   return check_launch("dab_heads_fwd_sm100");
 }
@@ -388,14 +412,16 @@ int dab_heads_fwd_sm100(const void* packed, const float* x, const float* beta, i
 /* The same heads with the LAST IPA layer's to_out (diffab_pytorch.py:464: y = cat Wout^T + b) fused in front: cat_bf16
  * [n_patches*128, 1024] = the concat features the layer's attention core left in its workspace, wout_bf16 [128][1024] and
  * b_out [128] from the layer's packed weights (dab_ipa_packed_layout).  The stack's output never exists in HBM; the same bits
- * as dab_ipa_fwd_sm100_stages(.., 4) followed by dab_heads_fwd_sm100. */
+ * as dab_ipa_fwd_sm100_stages(.., 4) followed by dab_heads_fwd_sm100.  With tiles / n_tiles (device memory: ascending ids
+ * of 16-row tiles, global row / 16, and their number) only the rows of those tiles are computed and written. */
 int dab_out_heads_fwd_sm100(const void* packed, const void* cat_bf16, const void* wout_bf16, const float* b_out, const float* beta,
-                            int n_patches, int L_, float* eps, float* rotvec, float* post, void* stream) {
+                            int n_patches, int L_, float* eps, float* rotvec, float* post, const int* tiles,
+                            const int* n_tiles, void* stream) {
   DAB_REQUIRE(L_ == 128, DAB_EUNSUPPORTED, "dab_out_heads_fwd_sm100: the fused heads kernel needs L = 128 (one block per CTA)");
   DAB_REQUIRE(n_patches >= 0, DAB_EINVAL, "dab_out_heads_fwd_sm100: negative batch");
   if (n_patches == 0) return DAB_OK;
-  DAB_REQUIRE(packed && cat_bf16 && wout_bf16 && b_out && beta && eps && rotvec && post, DAB_EINVAL,
-              "dab_out_heads_fwd_sm100: null pointer");
+  DAB_REQUIRE(packed && cat_bf16 && wout_bf16 && b_out && beta && eps && rotvec && post && (tiles == nullptr) == (n_tiles == nullptr),
+              DAB_EINVAL, "dab_out_heads_fwd_sm100: null pointer (tiles and n_tiles: both or neither)");
   DAB_REQUIRE((reinterpret_cast<uintptr_t>(packed) & 1023) == 0 && aligned16(cat_bf16) && aligned16(wout_bf16), DAB_EINVAL,
               "dab_out_heads_fwd_sm100: misaligned pointer (packed 1024 B, cat / Wout 16 B)");
   CUtensorMap m128, m32, mcat, mwout;
@@ -405,11 +431,12 @@ int dab_out_heads_fwd_sm100(const void* packed, const void* cat_bf16, const void
   if (int rc = make_tensor_map_bf16(&m128, pk + HeadsPacked::kW, 2, dims, strides, b128, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
   if (int rc = make_tensor_map_bf16(&m32, pk + HeadsPacked::kW, 2, dims, strides, b32, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
   uint64_t dc[2] = {1024, (uint64_t)n_patches * 128}, dwo[2] = {1024, (uint64_t)HD}, sc[1] = {1024 * 2};
-  if (int rc = make_tensor_map_bf16(&mcat, cat_bf16, 2, dc, sc, b128, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+  uint32_t b16[2] = {64, 16};        // live tiles: one box per 16-row tile
+  if (int rc = make_tensor_map_bf16(&mcat, cat_bf16, 2, dc, sc, tiles ? b16 : b128, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
   if (int rc = make_tensor_map_bf16(&mwout, wout_bf16, 2, dwo, sc, b128, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
   DAB_ENSURE_SMEM(denoiser_heads_kernel, HeadsSmem::kTotal);
   denoiser_heads_kernel<<<n_patches, 288, HeadsSmem::kTotal, (cudaStream_t)stream>>>(m128, m32, nullptr, beta, pk, eps, rotvec, post,
-                                                                                      mcat, mwout, b_out, 1);
+                                                                                      mcat, mwout, b_out, 1, tiles, n_tiles);
   count_launch();
   return check_launch("dab_out_heads_fwd_sm100");
 }

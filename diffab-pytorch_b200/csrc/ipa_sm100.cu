@@ -244,14 +244,19 @@ __device__ __forceinline__ void tmem_ld_x4(uint32_t taddr, float (&v)[4]) {
 // `bias` is the layer's precomputed pair bias, fp16 [B*L rows i][128 j][8 h], already scaled by
 // scale_total * log2(e) (dab_ipa_pair_bias_multi): e is constant over the six layers and the T steps, so the
 // e . Wpb contraction is hoisted out of the sampling loop entirely.
+// `live` (optional): ascending ids of the query tiles to compute (query tile = global row / 16), their count in
+// live_count[0]; the rows of the other tiles are left as they are.  n_tiles is then the upper bound of the kernel tiles.
 constexpr int kCoreThreads = 640;
-template <bool KB2>     // KB2: key-block mode for patches of 256 residues (see `decode` below); false: the L = 128 kernel
+// KB2: key-block mode for patches of 256 residues (see `decode` below); false: the L = 128 kernel.  LIVE: `live` is given
+// (a template argument so that the full-grid kernels stay exactly as they were)
+template <bool KB2, bool LIVE>
 __global__ void __launch_bounds__(kCoreThreads, 1)
 ipa_core_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                 const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_e,
                 const uint4* __restrict__ bias, const float* __restrict__ tc, const float* __restrict__ R,
                 __nv_bfloat16* __restrict__ cat, float* __restrict__ stats, uint4* __restrict__ pu,
-                int n_tiles, long long* __restrict__ dbg, int64_t out_stride) {
+                int n_tiles, long long* __restrict__ dbg, int64_t out_stride, const int* __restrict__ live,
+                const int* __restrict__ live_count) {
   extern __shared__ __align__(1024) uint8_t smem[];
   // optional per-tile timeline: slot k of tile c at dbg[c * 64 + k]
   long long* dbg_cta = nullptr;
@@ -266,13 +271,22 @@ ipa_core_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t smem_base = smem_u32(smem);
   if ((smem_base & 1023u) != 0) asm volatile("trap;");
+  // with a live-tile list: each live query tile is one kernel tile (two in key-block mode, one per key block); a CTA
+  // left without tiles falls straight through to the teardown
+  if (LIVE) n_tiles = min(n_tiles, (KB2 ? 2 : 1) * __ldg(live_count));
   // local tiles of this CTA: k = 0, 1, ... -> global tile blockIdx.x + k * gridDim.x, context k & 1
   const int n_local = (n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
   // Tiles are walked from the LAST patch down: the projection kernel has just written the packed operands in ascending
   // patch order, so the highest patches are the ones still resident in L2 (and the to_out GEMM, which starts with patch
   // 0, finds the concat features this kernel wrote last).  The pair rows are streamed with an evict-first policy so that
   // they do not push those operands out of L2.
-  auto tile_of = [&](int k) { return n_tiles - 1 - ((int)blockIdx.x + k * (int)gridDim.x); };
+  auto tile_of = [&](int k) {
+    const int x = n_tiles - 1 - ((int)blockIdx.x + k * (int)gridDim.x);
+    if (!LIVE) return x;
+    if (!KB2) return __ldg(live + x);
+    const int q = __ldg(live + (x >> 1));          // query tile -> (query block, key block x & 1), same row group
+    return ((((q >> 3) << 1) | (x & 1)) << 3) | (q & 7);
+  };
   // A tile = 16 query rows against one block of 128 keys.  Plain mode (KB2 = false): tile >> 3 = patch, keys = the patch.
   // Key-block mode (KB2, patches of 256 residues = two blocks): tile >> 3 = (query block, key block) pair; the pair
   // tensor / bias rows are 256 pairs long and the key block starts at pair 128 kb of the row; the (normalised) result and
@@ -947,6 +961,27 @@ static int launch_pair_bias(const void* e_bf16, const float* wpb, int nl, void* 
   return DAB_OK;
 }
 
+struct CoreArgs {
+  CUtensorMap mq, mk, mv, me;
+  const uint4* bias;
+  const float *tc, *R;
+  __nv_bfloat16* cat;
+  float* stats;
+  uint4* pu;
+  int n_tiles;
+  int64_t out_stride;
+  const int *live, *live_count;
+};
+// (a function template: DAB_ENSURE_SMEM keeps one flag per instantiation, i.e. per kernel)
+template <bool KB2, bool LIVE>
+static int launch_core_kernel(const CoreArgs& a, int grid, cudaStream_t s) {
+  DAB_ENSURE_SMEM((ipa_core_kernel<KB2, LIVE>), CoreSmem::kTotal);
+  ipa_core_kernel<KB2, LIVE><<<grid, kCoreThreads, CoreSmem::kTotal, s>>>(a.mq, a.mk, a.mv, a.me, a.bias, a.tc, a.R, a.cat, a.stats,
+                                                                          a.pu, a.n_tiles, g_core_dbg, a.out_stride, a.live,
+                                                                          a.live_count);
+  return DAB_OK;
+}
+
 }  // namespace sm100
 }  // namespace dab
 
@@ -1089,6 +1124,53 @@ static int fwd_prologue(const char* fn, const DabIpaDims* d, bool train, bool ar
   return DAB_OK;
 }
 
+// Attention-core launch of a layer (stage 2) on the packed operands in the workspace; `live` / `live_count` (device
+// memory, optional): only these query tiles (see ipa_core_kernel).
+static int launch_core(const FwdWs& f, int Lp, const uint8_t* pk, const void* e_bf16, const void* bias_f16, const float* R,
+                       bool save_for_bwd, const int* live, const int* live_count, cudaStream_t s) {
+  const bool two = f.two;
+  const int B = f.nblk, M = B * L;
+  const Ws& ws = f.ws;
+  const Ws2& w2 = f.w2;
+  const PackedOffsets po = packed_offsets();
+  const uint4* bias = reinterpret_cast<const uint4*>(bias_f16);
+  if (bias == nullptr) {   // one-off call without a precomputed bias: build this layer's plane now
+    uint4* plane = two ? w2.bias2 : ws.bias;
+    if (int rc = launch_pair_bias(e_bf16, reinterpret_cast<const float*>(pk + po.wpb), 1, plane, (int64_t)M * Lp, s)) return rc;
+    bias = plane;
+  }
+  CUtensorMap mq, mk, mv, me;
+  uint64_t dqk[2] = {(uint64_t)H * QK_W, (uint64_t)M}, sqk[1] = {(uint64_t)H * QK_W * 2};
+  uint32_t bq[2] = {32, IB}, bk[2] = {32, L};
+  if (int rc = make_tensor_map_bf16(&mq, ws.Qp, 2, dqk, sqk, bq, CU_TENSOR_MAP_SWIZZLE_64B)) return rc;
+  if (int rc = make_tensor_map_bf16(&mk, ws.Kp, 2, dqk, sqk, bk, CU_TENSOR_MAP_SWIZZLE_64B)) return rc;
+  uint64_t dv[2] = {(uint64_t)H * V_W, (uint64_t)M}, sv[1] = {(uint64_t)H * V_W * 2};
+  uint32_t bv[2] = {V_W, L};
+  if (int rc = make_tensor_map_bf16(&mv, ws.Vp, 2, dv, sv, bv, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+  uint64_t de[2] = {(uint64_t)C, (uint64_t)M * Lp}, se[1] = {(uint64_t)C * 2};
+  uint32_t be[2] = {C, L};
+  if (int rc = make_tensor_map_bf16(&me, e_bf16, 2, de, se, be, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+  const int n_tiles = (two ? 2 * B : B) * (L / IB);      // 256: one tile set per (query block, key block) pair
+  int n_sm = 148;
+  {
+    int dev_id = 0;
+    cudaGetDevice(&dev_id);
+    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev_id);
+  }
+  const int grid = n_tiles < n_sm ? n_tiles : n_sm;     // persistent: one CTA per SM, two tile contexts each
+  const CoreArgs a = {mq, mk, mv, me, bias, ws.tc, R, two ? w2.cat2 : ws.cat, two ? w2.stats2 : (save_for_bwd ? ws.stats : nullptr),
+                      two || !save_for_bwd ? nullptr : ws.pu, n_tiles, two ? (int64_t)M : 0, live, live_count};
+  if (int rc = two ? (live ? launch_core_kernel<true, true>(a, grid, s) : launch_core_kernel<true, false>(a, grid, s))
+                   : (live ? launch_core_kernel<false, true>(a, grid, s) : launch_core_kernel<false, false>(a, grid, s)))
+    return rc;
+  count_launch();
+  if (two) {   // (all rows: those of tiles left out are merged from stale inputs and never read)
+    merge_kb2_kernel<<<(unsigned)(((int64_t)M * H + 255) / 256), 256, 0, s>>>(w2.cat2, w2.stats2, (int64_t)M, ws.cat);
+    count_launch();
+  }
+  return DAB_OK;
+}
+
 // x / y: fp32, or (x_bf16 / y_bf16 non-null) bf16 - the residue stream handed from layer to layer already rounded
 static int fwd_sm100_impl(const char* fn, const DabIpaDims* d, const void* packed, const float* x, const void* e_bf16,
                           const void* bias_f16, const float* R, const float* t, float* y, void* workspace,
@@ -1114,46 +1196,7 @@ static int fwd_sm100_impl(const char* fn, const DabIpaDims* d, const void* packe
       return rc;
   }
   if (phases & 2) {
-    const uint4* bias = reinterpret_cast<const uint4*>(bias_f16);
-    if (bias == nullptr) {   // one-off call without a precomputed bias: build this layer's plane now
-      uint4* plane = two ? w2.bias2 : ws.bias;
-      if (int rc = launch_pair_bias(e_bf16, reinterpret_cast<const float*>(pk + po.wpb), 1, plane, (int64_t)M * Lp, s)) return rc;
-      bias = plane;
-    }
-    CUtensorMap mq, mk, mv, me;
-    uint64_t dqk[2] = {(uint64_t)H * QK_W, (uint64_t)M}, sqk[1] = {(uint64_t)H * QK_W * 2};
-    uint32_t bq[2] = {32, IB}, bk[2] = {32, L};
-    if (int rc = make_tensor_map_bf16(&mq, ws.Qp, 2, dqk, sqk, bq, CU_TENSOR_MAP_SWIZZLE_64B)) return rc;
-    if (int rc = make_tensor_map_bf16(&mk, ws.Kp, 2, dqk, sqk, bk, CU_TENSOR_MAP_SWIZZLE_64B)) return rc;
-    uint64_t dv[2] = {(uint64_t)H * V_W, (uint64_t)M}, sv[1] = {(uint64_t)H * V_W * 2};
-    uint32_t bv[2] = {V_W, L};
-    if (int rc = make_tensor_map_bf16(&mv, ws.Vp, 2, dv, sv, bv, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
-    uint64_t de[2] = {(uint64_t)C, (uint64_t)M * Lp}, se[1] = {(uint64_t)C * 2};
-    uint32_t be[2] = {C, L};
-    if (int rc = make_tensor_map_bf16(&me, e_bf16, 2, de, se, be, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
-    const int n_tiles = (two ? 2 * B : B) * (L / IB);      // 256: one tile set per (query block, key block) pair
-    int n_sm = 148;
-    {
-      int dev_id = 0;
-      cudaGetDevice(&dev_id);
-      cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev_id);
-    }
-    const int grid = n_tiles < n_sm ? n_tiles : n_sm;     // persistent: one CTA per SM, two tile contexts each
-    if (two) {
-      DAB_ENSURE_SMEM(ipa_core_kernel<true>, CoreSmem::kTotal);
-      ipa_core_kernel<true><<<grid, kCoreThreads, CoreSmem::kTotal, s>>>(mq, mk, mv, me, bias, ws.tc, R, w2.cat2, w2.stats2, nullptr,
-                                                                         n_tiles, g_core_dbg, (int64_t)M);
-    } else {
-      DAB_ENSURE_SMEM(ipa_core_kernel<false>, CoreSmem::kTotal);
-      ipa_core_kernel<false><<<grid, kCoreThreads, CoreSmem::kTotal, s>>>(mq, mk, mv, me, bias, ws.tc, R, ws.cat,
-                                                                          save_for_bwd ? ws.stats : nullptr,
-                                                                          save_for_bwd ? ws.pu : nullptr, n_tiles, g_core_dbg, 0);
-    }
-    count_launch();
-    if (two) {
-      merge_kb2_kernel<<<(unsigned)(((int64_t)M * H + 255) / 256), 256, 0, s>>>(w2.cat2, w2.stats2, (int64_t)M, ws.cat);
-      count_launch();
-    }
+    if (int rc = launch_core(f, Lp, pk, e_bf16, bias_f16, R, save_for_bwd, nullptr, nullptr, s)) return rc;
   }
   if (phases & 4) {
     // y = cat Wout^T + b: one 128-wide N tile per CTA when the batch fills the GPU, four 32-wide ones otherwise
@@ -1200,6 +1243,23 @@ int dab_ipa_fwd_sm100_stages(const DabIpaDims* d, const void* packed, const floa
   DAB_REQUIRE(stages > 0 && stages <= 7, DAB_EINVAL, "dab_ipa_fwd_sm100_stages: stages must be a non-empty subset of bits 0..2");
   return fwd_sm100_impl("dab_ipa_fwd_sm100_stages", d, packed, x, e_bf16, bias_f16, R, t, y, workspace, workspace_bytes, false,
                         stream, x_bf16, y_bf16, stages);
+}
+
+/* The attention core (stages(.., 2)) on a list of query tiles only: live_tiles = ascending ids of 16-row tiles (global
+ * row / 16 of the B*L rows), live_count[0] = their number; both in device memory, read by the kernel (no host sync, so the
+ * list may change between replays of a captured graph).  The concat features of the other rows are left as they were. */
+int dab_ipa_core_sm100_live(const DabIpaDims* d, const void* packed, const void* e_bf16, const void* bias_f16, const float* R,
+                            const float* t, void* workspace, size_t workspace_bytes, const int* live_tiles,
+                            const int* live_count, void* stream) {
+  FwdWs f;
+  if (int rc = fwd_prologue("dab_ipa_core_sm100_live", d, false, e_bf16 && R && t && live_tiles && live_count,
+                            (reinterpret_cast<uintptr_t>(e_bf16) & 127) == 0, packed, workspace, workspace_bytes, f))
+    return rc;
+  if (f.nblk == 0) return DAB_OK;
+  if (int rc = launch_core(f, d->L, reinterpret_cast<const uint8_t*>(packed), e_bf16, bias_f16, R, false, live_tiles,
+                           live_count, (cudaStream_t)stream))
+    return rc;
+  return check_launch("dab_ipa_core_sm100_live");
 }
 
 /* Between two layers of a stack (inference): the previous layer's to_out (y = cat Wout^T + b, `packed_prev`; `cat` = the

@@ -45,43 +45,47 @@ __device__ __forceinline__ void reverse_update_residue(
   } else {
     seq_out[r] = s_old;
   }
+  // The network outputs are read only where they are used: sampling computes them for the tiles of generated residues
+  // only (DiffAb.sample_from_context), the rows of the other tiles are undefined.
   // positions: (x_t - beta/sqrt(1-abar) eps_theta) * (1/sqrt(alpha)) + sqrt(beta) z
-  float beta = __ldg(sc.beta + tt);
-  float c_eps = __fdiv_rn(beta, __ldg(sc.one_minus_alpha_bar_sqrt + tt));
-  float inv_sa = __fdiv_rn(1.0f, __fsqrt_rn(__ldg(sc.alpha + tt)));
-  float sig = noisy ? __fsqrt_rn(beta) : 0.f;
-#pragma unroll
-  for (int c = 0; c < 3; ++c) {
-    float xo = x_t[r * 3 + c];
-    float v = __fadd_rn(__fmul_rn(__fsub_rn(xo, __fmul_rn(c_eps, __ldg(eps_theta + r * 3 + c))), inv_sa),
-                        __fmul_rn(sig, __ldg(z + r * 3 + c)));
-    x_out[r * 3 + c] = gen_str ? v : xo;
-  }
-  // orientations: O0 = O_t @ exp(v_theta)  (Denoiser tail, diffab_pytorch.py:594-596); O' = O0 @ exp(rotvec)
-  float Rt[9], Re[9], R0[9];
-#pragma unroll
-  for (int c = 0; c < 9; ++c) Rt[c] = O_t[r * 9 + c];
-  so3_exp(__ldg(v_theta + r * 3), __ldg(v_theta + r * 3 + 1), __ldg(v_theta + r * 3 + 2), Re);
-  mat3_mul(Rt, Re, R0);
-  if (O0_out) {
-#pragma unroll
-    for (int c = 0; c < 9; ++c) O0_out[r * 9 + c] = R0[c];
-  }
   if (gen_str) {
-    if (noisy) {
-      float Rn[9], Ro[9];
-      so3_exp(rv[0], rv[1], rv[2], Rn);
-      mat3_mul(R0, Rn, Ro);
+    float beta = __ldg(sc.beta + tt);
+    float c_eps = __fdiv_rn(beta, __ldg(sc.one_minus_alpha_bar_sqrt + tt));
+    float inv_sa = __fdiv_rn(1.0f, __fsqrt_rn(__ldg(sc.alpha + tt)));
+    float sig = noisy ? __fsqrt_rn(beta) : 0.f;
 #pragma unroll
-      for (int c = 0; c < 9; ++c) O_out[r * 9 + c] = Ro[c];
-    } else {
-#pragma unroll
-      for (int c = 0; c < 9; ++c) O_out[r * 9 + c] = R0[c];
-    }
+    for (int c = 0; c < 3; ++c)
+      x_out[r * 3 + c] = __fadd_rn(__fmul_rn(__fsub_rn(x_t[r * 3 + c], __fmul_rn(c_eps, __ldg(eps_theta + r * 3 + c))), inv_sa),
+                                   __fmul_rn(sig, __ldg(z + r * 3 + c)));
   } else {
 #pragma unroll
-    for (int c = 0; c < 9; ++c) O_out[r * 9 + c] = Rt[c];
+    for (int c = 0; c < 3; ++c) x_out[r * 3 + c] = x_t[r * 3 + c];
   }
+  // orientations: O0 = O_t @ exp(v_theta)  (Denoiser tail, diffab_pytorch.py:594-596); O' = O0 @ exp(rotvec)
+  float Rt[9];
+#pragma unroll
+  for (int c = 0; c < 9; ++c) Rt[c] = O_t[r * 9 + c];
+  if (gen_str || O0_out) {
+    float Re[9], R0[9];
+    so3_exp(__ldg(v_theta + r * 3), __ldg(v_theta + r * 3 + 1), __ldg(v_theta + r * 3 + 2), Re);
+    mat3_mul(Rt, Re, R0);
+    if (O0_out) {
+#pragma unroll
+      for (int c = 0; c < 9; ++c) O0_out[r * 9 + c] = R0[c];
+    }
+    if (gen_str) {
+      if (noisy) {
+        float Rn[9];
+        so3_exp(rv[0], rv[1], rv[2], Rn);
+        mat3_mul(R0, Rn, Rt);
+      } else {
+#pragma unroll
+        for (int c = 0; c < 9; ++c) Rt[c] = R0[c];
+      }
+    }
+  }
+#pragma unroll
+  for (int c = 0; c < 9; ++c) O_out[r * 9 + c] = Rt[c];
 }
 
 }  // namespace dab

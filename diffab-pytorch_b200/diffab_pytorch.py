@@ -625,6 +625,21 @@ def _fwd_stages(dims, packed, x, e, bias, r, t, y, ws, stages, st):
                "dab_ipa_fwd_sm100_stages")
 
 
+def live_query_tiles(generation_mask, out=None):
+    """The 16-row query tiles (tile = row / 16 of the flattened B x L rows) that hold a generated residue, on the device and
+    without a host synchronisation: (int32 tile ids, the live ones first in ascending order; int32 (1,) their count).
+    Sampling computes the last IPA layer's attention core and the heads on these tiles only: the reverse update keeps
+    every other residue as it is.  ``out`` = a previous result, refilled in place (static buffers of a captured graph)."""
+    flags = generation_mask.reshape(-1, 16).ne(0).any(-1)
+    tiles = torch.argsort((~flags).to(torch.int32), stable=True).to(torch.int32)
+    count = flags.sum(dtype=torch.int32).view(1)
+    if out is None:
+        return tiles, count
+    out[0].copy_(tiles)
+    out[1].copy_(count)
+    return out
+
+
 def _pair_bias_planes(layers, e, out):
     """The pair-bias planes of ``layers`` into ``out`` (fp16 (n_layers, B, L, L, H), contiguous) from the bf16 pair
     tensor ``e``: one pass over it per six layers."""
@@ -1066,14 +1081,16 @@ class InvariantPointAttentionModule(nn.Module):
                 self.layers[0].fast_path_supported(L, True) and B * (L // FAST_L) >= 128)
 
     @torch.no_grad()
-    def _forward_fused_stack(self, res_emb, pair_emb, orientations, translations, pair_bias, front=None, heads=None):
+    def _forward_fused_stack(self, res_emb, pair_emb, orientations, translations, pair_bias, front=None, heads=None,
+                             live=None):
         """The layer stack launch by launch on ONE shared workspace: projections of layer 0, then per layer the attention
         core followed by ``dab_ipa_mid_sm100`` (its to_out + the next layer's projections in one kernel), to_out of the
         last layer.  2 n launches instead of 3 n; results bit-identical to ``forward_fast_io`` layer by layer.
         ``front`` = (sampling cache of the Denoiser, seq_idx_t) instead of ``res_emb``: the epsilon network's front MLP
         runs inside the first projection kernel (``dab_ipa_front_proj_sm100``).  ``heads`` = (packed head weights, beta per
         block): the last layer's to_out runs inside the heads kernel (``dab_out_heads_fwd_sm100``) and the call returns
-        (eps, rotvec, posterior) instead of the stack's output."""
+        (eps, rotvec, posterior) instead of the stack's output.  ``live`` (``live_query_tiles``): the last layer's attention
+        core and the heads compute only the rows of these tiles, the other rows of the result are undefined."""
         layers = self.layers
         n = len(layers)
         e = _lib.dev(pair_emb, torch.bfloat16, "e")
@@ -1104,7 +1121,12 @@ class InvariantPointAttentionModule(nn.Module):
                 ctypes.byref(dims), ptr(packed[0]), ptr(cache["c"]), ptr(cache["t1"]), ptr(_lib.dev(seq, torch.int64, "seq_idx")),
                 ptr(cache["w2_bf16"]), ptr(cache["b2"]), ptr(r), ptr(t), ptr(ws), ws.numel(), st), "dab_ipa_front_proj_sm100")
         for k in range(n):
-            stage(k, 2)
+            if k == n - 1 and live is not None:     # (earlier layers: every row feeds the next layer's keys and values)
+                _lib.check(lib.dab_ipa_core_sm100_live(ctypes.byref(dims), ptr(packed[k]), ptr(e), ptr(bias[k]), ptr(r), ptr(t),
+                                                       ptr(ws), ws.numel(), ptr(live[0]), ptr(live[1]), st),
+                           "dab_ipa_core_sm100_live")
+            else:
+                stage(k, 2)
             if k + 1 < n:
                 _lib.check(lib.dab_ipa_mid_sm100(ctypes.byref(dims), ptr(packed[k]), ptr(packed[k + 1]), ptr(r), ptr(t), ptr(ws),
                                                  ws.numel(), st), "dab_ipa_mid_sm100")
@@ -1125,7 +1147,8 @@ class InvariantPointAttentionModule(nn.Module):
         pk_last = packed[n - 1]
         _lib.check(lib.dab_out_heads_fwd_sm100(ptr(heads_packed), ws.data_ptr() + offs[4], pk_last.data_ptr() + poffs[1],
                                                pk_last.data_ptr() + poffs[3], ptr(beta_blk), nblk, FAST_L, ptr(eps), ptr(rot),
-                                               ptr(post), st), "dab_out_heads_fwd_sm100")
+                                               ptr(post), None if live is None else ptr(live[0]),
+                                               None if live is None else ptr(live[1]), st), "dab_out_heads_fwd_sm100")
         return eps, rot, post
 
     def precompute_pair_bias(self, pair_emb_bf16, out=None):
@@ -1248,12 +1271,13 @@ class Denoiser(nn.Module):
         }
 
     @torch.no_grad()
-    def heads_fast(self, seq_idx_t, translations_t, orientations_t, cache, pair_context_emb, beta, pair_bias=None):
-        """``heads`` with the per-run constants of ``sampling_cache``; returns (eps, rotvec, seq_posterior)."""
+    def heads_fast(self, seq_idx_t, translations_t, orientations_t, cache, pair_context_emb, beta, pair_bias=None,
+                   live=None):
+        """``heads`` with the per-run constants of ``sampling_cache``; returns (eps, rotvec, seq_posterior).
+        ``live`` (``live_query_tiles``, large batches only): the rows outside these tiles are left undefined."""
         B, L = seq_idx_t.shape
         D = cache["c"].shape[-1]
-        if (cache.get("w2_bf16") is not None and cache["c"].dtype == torch.float32 and cache["c"].is_contiguous() and
-                self.ipa.fused_stack_applicable(B, L, pair_context_emb, pair_bias)):
+        if self.fused_heads_applicable(cache, B, L, pair_context_emb, pair_bias):
             # large batches: the front MLP runs inside the first layer's projection kernel (same bits as the branch below)
             front = (cache, seq_idx_t.contiguous())
             if cache.get("heads_packed") is not None:
@@ -1261,8 +1285,9 @@ class Denoiser(nn.Module):
                 nb = L // FAST_L
                 beta_blk = beta.contiguous() if nb == 1 else beta.repeat_interleave(nb)
                 return self.ipa._forward_fused_stack(None, pair_context_emb, orientations_t, translations_t, pair_bias,
-                                                     front=front, heads=(cache["heads_packed"], beta_blk))
-            h = self.ipa._forward_fused_stack(None, pair_context_emb, orientations_t, translations_t, pair_bias, front=front)
+                                                     front=front, heads=(cache["heads_packed"], beta_blk), live=live)
+            h = self.ipa._forward_fused_stack(None, pair_context_emb, orientations_t, translations_t, pair_bias, front=front,
+                                              live=live)
             return self._heads_from(h, cache, pair_context_emb, beta)
         if cache.get("w2_bf16") is not None and pair_context_emb.dtype == torch.bfloat16 and (B * L) % 128 == 0:
             # bf16 out when the layer stack takes it (its first projection kernel rounds an fp32 input the same way)
@@ -1278,6 +1303,11 @@ class Denoiser(nn.Module):
             h = torch.addmm(cache["b2"], h.view(-1, D), cache["w2t"]).view(B, L, D)
         h = self.ipa(h, pair_context_emb, orientations_t, translations_t, pair_bias)
         return self._heads_from(h, cache, pair_context_emb, beta)
+
+    def fused_heads_applicable(self, cache, B, L, pair_context_emb, pair_bias):
+        """``heads_fast`` runs the fused stack (front MLP in the first projections) - the path that takes ``live``."""
+        return (cache.get("w2_bf16") is not None and cache["c"].dtype == torch.float32 and cache["c"].is_contiguous() and
+                self.ipa.fused_stack_applicable(B, L, pair_context_emb, pair_bias))
 
     def _heads_from(self, h, cache, pair_context_emb, beta):
         """The three heads on the stack's output (sampling)."""
@@ -1603,11 +1633,13 @@ class DiffAb(nn.Module):
 
     @torch.no_grad()
     def reverse_step(self, seq_idx_t, translations_t, orientations_t, res_context_emb, pair_context_emb,
-                     generation_mask, t, noise, inplace=False, pair_bias=None, glue_cache=None, beta=None, generate=3):
+                     generation_mask, t, noise, inplace=False, pair_bias=None, glue_cache=None, beta=None, generate=3,
+                     live=None):
         """One reverse-diffusion step: epsilon network + fused update kernel.  ``t`` is (B,) int64.
         ``glue_cache`` (``Denoiser.sampling_cache``) switches the dense glue to its regrouped form; ``beta`` = the
         schedule's beta at ``t`` when the caller has already gathered it.  ``generate`` (``diffusion.generate_bits``):
-        a modality that is not generated keeps its value."""
+        a modality that is not generated keeps its value.  ``live`` = ``live_query_tiles(generation_mask)`` (with
+        ``glue_cache``): the epsilon network's last layer and heads skip the tiles without a generated residue."""
         if beta is None:
             beta = self.dsched.tensors["beta"][t]
         rotvec = None
@@ -1621,7 +1653,7 @@ class DiffAb(nn.Module):
             with torch.cuda.stream(side):
                 self.so3_reverse.sample_isotropic_gaussian(t, L, noise=noise, out=rotvec)
             eps, v_eps, post = self.denoiser.heads_fast(seq_idx_t, translations_t, orientations_t, glue_cache,
-                                                        pair_context_emb, beta, pair_bias)
+                                                        pair_context_emb, beta, pair_bias, live=live)
             main.wait_stream(side)
         else:
             eps, v_eps, post = self.denoiser.heads(seq_idx_t, translations_t, orientations_t, res_context_emb,
@@ -1676,13 +1708,22 @@ class DiffAb(nn.Module):
             if pair_bias is not None and _valid_len is not None:
                 _mask_padded_keys(pair_bias, _valid_len)
             glue = self.denoiser.sampling_cache(res_context_emb) if pair_context_emb.dtype == torch.bfloat16 else None
+            live = self._live_tiles(generation_mask, pair_context_emb, pair_bias, glue)
             for step in range(t_start, t_stop - 1, -1):
                 t = torch.full((B,), step, device=dev, dtype=torch.int64)
                 noise = noises[step] if noises is not None else self.draw_step_noise(B, L, dev, generator=generator)
                 out = self.reverse_step(s, x, O, res_context_emb, pair_context_emb, generation_mask, t, noise,
-                                        inplace=True, pair_bias=pair_bias, glue_cache=glue, generate=generate)
+                                        inplace=True, pair_bias=pair_bias, glue_cache=glue, generate=generate, live=live)
                 s, x, O = out["seq_idx"], out["translations"], out["orientations"]
             return {"seq_idx": s, "translations": x, "orientations": O}
+
+    def _live_tiles(self, generation_mask, pair_ctx, pair_bias, glue, out=None):
+        """``live_query_tiles`` of the mask where the reverse step runs the fused stack (the only path that takes them),
+        else None."""
+        B, L = generation_mask.shape
+        if glue is None or not self.denoiser.fused_heads_applicable(glue, B, L, pair_ctx, pair_bias):
+            return None
+        return live_query_tiles(generation_mask, out=out)
 
     def _pair_bias_planes(self, pair_ctx):
         """Per-layer pair-bias planes of the tensor-core path (None on the fp32 path): the e . Wpb contraction
@@ -1718,7 +1759,7 @@ class DiffAb(nn.Module):
             cache = {"key": key, "s": torch.empty_like(s), "x": torch.empty_like(x), "O": torch.empty_like(O),
                      "t": torch.full((B,), t_start, device=dev, dtype=torch.int64),
                      "res": torch.empty_like(res_ctx), "pair": torch.empty_like(pair_ctx),
-                     "mask": torch.empty_like(generation_mask), "bias": None, "graph": None, "glue": None,
+                     "mask": torch.empty_like(generation_mask), "bias": None, "graph": None, "glue": None, "live": None,
                      "graph_block": None, "noise1": self.draw_step_noise(B, L, dev)}
         st = cache
         st["res"].copy_(res_ctx); st["pair"].copy_(pair_ctx); st["mask"].copy_(generation_mask)
@@ -1731,6 +1772,8 @@ class DiffAb(nn.Module):
             if valid_len is not None:          # padded batch of shorter patches: the padded keys are never attended to
                 st["bias_all"][:, :, :, valid_len:, :] = float("-inf")
             st["glue"] = self.denoiser.sampling_cache(st["res"], cache=st["glue"])
+            # the graphs are cached per shape, not per mask: the tile list is rebuilt into its static buffers on every call
+            st["live"] = self._live_tiles(st["mask"], st["pair"], st["bias"], st["glue"], out=st["live"])
         if fresh:
             st["s"].copy_(s); st["x"].copy_(x); st["O"].copy_(O)
             side = torch.cuda.Stream(device=dev)
@@ -1740,14 +1783,15 @@ class DiffAb(nn.Module):
                     self._fill_noise_(st["noise1"])
                     self.reverse_step(st["s"].clone(), st["x"].clone(), st["O"].clone(), st["res"], st["pair"],
                                       st["mask"], st["t"], st["noise1"], pair_bias=st["bias"], glue_cache=st["glue"],
-                                      generate=generate)
+                                      generate=generate, live=st["live"])
             torch.cuda.current_stream(dev).wait_stream(side)
             draw, graph = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
             with torch.cuda.graph(draw):
                 self._fill_noise_(st["noise1"])
             with torch.cuda.graph(graph, pool=draw.pool()):
                 self.reverse_step(st["s"], st["x"], st["O"], st["res"], st["pair"], st["mask"], st["t"], st["noise1"],
-                                  inplace=True, pair_bias=st["bias"], glue_cache=st["glue"], generate=generate)
+                                  inplace=True, pair_bias=st["bias"], glue_cache=st["glue"], generate=generate,
+                                  live=st["live"])
                 st["t"].sub_(1)
             st["graph"], st["draw"] = graph, draw
             self._graph_cache = st
@@ -1771,7 +1815,7 @@ class DiffAb(nn.Module):
                 for u in range(U):
                     self.reverse_step(st["s"], st["x"], st["O"], st["res"], st["pair"], st["mask"], t_blk[u],
                                       {k: v[u] for k, v in noiseU.items()}, inplace=True, pair_bias=st["bias"],
-                                      glue_cache=st["glue"], beta=beta_blk[u], generate=generate)
+                                      glue_cache=st["glue"], beta=beta_blk[u], generate=generate, live=st["live"])
                 st["t"].sub_(U)
             st["graph_block"] = (U, block, draw_block)
         st["s"].copy_(s); st["x"].copy_(x); st["O"].copy_(O)

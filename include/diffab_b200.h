@@ -192,6 +192,13 @@ int dab_ipa_pair_bias_multi(const DabIpaDims* d, const void* e_bf16, const float
 int dab_ipa_fwd_sm100_stages(const DabIpaDims* d, const void* packed, const float* x, const void* x_bf16, const void* e_bf16,
                              const void* bias_f16, const float* R, const float* t, float* y, void* y_bf16, void* workspace,
                              size_t workspace_bytes, int stages, void* stream);
+/* The attention core (stages(.., 2)) on a list of 16-row query tiles only: live_tiles = their ascending ids (global row / 16
+ * of the B*L rows), live_count[0] = their number, both in device memory and read by the kernel (no host synchronisation:
+ * the list may change between replays of a captured graph).  The concat features of the other rows keep what the
+ * workspace held.  Sampling runs the LAST layer of the stack this way on the tiles that hold generated residues. */
+int dab_ipa_core_sm100_live(const DabIpaDims* d, const void* packed, const void* e_bf16, const void* bias_f16, const float* R,
+                            const float* t, void* workspace, size_t workspace_bytes, const int* live_tiles,
+                            const int* live_count, void* stream);
 /* Between two layers of a stack (inference): the previous layer's to_out (`packed_prev`; input = the concat features its
  * attention core left in `workspace`) fused into this layer's projection kernel (`packed`): y is rounded to bf16 as
  * dab_ipa_fwd_sm100_stages would hand it over (y_bf16) but never exists in HBM.  Stack = stages(1) of layer 0, then per
@@ -255,9 +262,12 @@ int dab_heads_fwd_sm100(const void* packed, const float* x, const float* beta, i
 /* The same heads with the LAST IPA layer's to_out (diffab_pytorch.py:464: y = cat Wout^T + b) fused in front: cat_bf16
  * [n_patches*128, 1024] = the concat features the layer's attention core left in its workspace (dab_ipa_sm100_workspace_layout),
  * wout_bf16 [128][1024] and b_out [128] from the layer's packed weights (dab_ipa_packed_layout).  The stack's output never
- * exists in HBM; the same bits as dab_ipa_fwd_sm100_stages(.., 4) followed by dab_heads_fwd_sm100. */
+ * exists in HBM; the same bits as dab_ipa_fwd_sm100_stages(.., 4) followed by dab_heads_fwd_sm100.  tiles / n_tiles (device
+ * memory, both or neither): ascending ids of 16-row tiles (global row / 16) and their number - only the rows of those tiles
+ * are computed and written (sampling: the tiles that hold generated residues), with the same bits. */
 int dab_out_heads_fwd_sm100(const void* packed, const void* cat_bf16, const void* wout_bf16, const float* b_out, const float* beta,
-                            int n_patches, int L, float* eps, float* rotvec, float* post, void* stream);
+                            int n_patches, int L, float* eps, float* rotvec, float* post, const int* tiles, const int* n_tiles,
+                            void* stream);
 
 /* Front of the epsilon network during sampling (diffab_pytorch.py:572-574, to_res_emb on [res_ctx | emb(s_t)]):
  * x0[n_rows,128] = relu(c[row] + t1[seq[row]]) . w2^T + b2, where c = res_ctx . W1[:, :128]^T + b1 (per-run constant,

@@ -2,9 +2,12 @@
 """Where one graphed reverse step spends its time (GPU only): the step's sub-chains captured as separate CUDA graphs
 (ten repetitions each) and replayed - front MLP, the IPA stack, heads, IGSO(3) draw + update kernel - next to the whole
 step.  The difference between the whole and the sum of the parts is what the hand-offs between the parts cost.
+Then the whole step, the fused IPA stack and the last to_out + heads kernel with and without the live-tile list of the
+batch's generation mask (the last layer's core and the heads on the tiles of generated residues only), alternating.
 
     python tools/time_step_parts.py [B]
 """
+import ctypes
 import os
 import sys
 
@@ -16,7 +19,7 @@ import diffab_pytorch_b200  # noqa: E402,F401
 from diffab_pytorch_b200 import _lib, synth  # noqa: E402
 from diffab_pytorch_b200 import diffusion as _diffusion  # noqa: E402
 from diffab_pytorch_b200._lib import ptr  # noqa: E402
-from diffab_pytorch_b200.diffab_pytorch import DiffAb  # noqa: E402
+from diffab_pytorch_b200.diffab_pytorch import FAST_L, DiffAb, _ipa_structs, live_query_tiles  # noqa: E402
 
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 256
 REP = 10
@@ -103,3 +106,45 @@ with torch.no_grad():
     e = timed(eps_net, "epsilon network (front+stack+heads)")
     w = timed(whole, "whole reverse step")
     print(f"  sum of the four parts {sum(parts):.1f} us; epsilon network {e:.1f}; whole step {w:.1f}")
+
+    live = live_query_tiles(m)
+    n_live = int(live[1])
+    print(f"live tiles: {n_live} of {B * 128 // 16} (generation mask of the batch)")
+    ipa = den.ipa
+    front_arg = (glue, s)
+
+    def stack_fused(lv):
+        return lambda: ipa._forward_fused_stack(None, pair, O, x, bias, front=front_arg, live=lv)
+
+    # the last layer's to_out + heads alone, on the concat features the stack leaves in the shared workspace
+    lib = _lib.lib()
+    layers = ipa.layers
+    dims = _ipa_structs(layers[0], B, 128)
+    ws = layers[0]._workspace(max(lib.dab_ipa_sm100_workspace_bytes(ctypes.byref(dims)), 16), dev)
+    pk_last = layers[-1]._packed_weights(dims)
+    offs = (ctypes.c_size_t * 8)(); poffs = (ctypes.c_size_t * 7)()
+    _lib.check(lib.dab_ipa_sm100_workspace_layout(ctypes.byref(dims), offs), "layout")
+    _lib.check(lib.dab_ipa_packed_layout(ctypes.byref(dims), poffs), "packed layout")
+
+    def out_heads(lv):
+        return lambda: _lib.check(lib.dab_out_heads_fwd_sm100(
+            ptr(glue["heads_packed"]), ws.data_ptr() + offs[4], pk_last.data_ptr() + poffs[1], pk_last.data_ptr() + poffs[3],
+            ptr(beta), B, FAST_L, ptr(eps), ptr(rot), ptr(post), None if lv is None else ptr(lv[0]),
+            None if lv is None else ptr(lv[1]), _lib.stream_ptr()), "out_heads")
+
+    def whole_step(lv):
+        return lambda: model.reverse_step(s1, x1, O1, res, pair, m, t, noise, inplace=True, pair_bias=bias, glue_cache=glue,
+                                          beta=beta, live=lv)
+
+    rows = []
+    for name, mk in (("whole reverse step", whole_step), ("IPA stack (fused, 6 layers)", stack_fused),
+                     ("last to_out + heads", out_heads)):
+        a, b_ = [], []
+        for _ in range(3):   # alternating
+            a.append(timed(mk(None), f"{name}: all tiles"))
+            b_.append(timed(mk(live), f"{name}: live tiles"))
+        a.sort(); b_.sort()
+        rows.append((name, a[1], b_[1]))
+    print("medians of three alternating runs:")
+    for name, a, b_ in rows:
+        print(f"  {name:30s} all {a:8.1f} us  live {b_:8.1f} us  saved {a - b_:7.1f} us ({100 * (a - b_) / a:.1f} %)")
