@@ -67,6 +67,8 @@ EXPORTS = {
                               c_void_p, c_void_p]),
     "dab_reverse_step": (c_int, [POINTER(DabSchedule)] + [c_void_p] * 8 + [c_int, c_int] + [c_void_p] * 3 + [c_int] +
                          [c_void_p] * 5),
+    "dab_reverse_step_weighted": (c_int, [POINTER(DabSchedule)] + [c_void_p] * 8 + [c_int, c_int] + [c_void_p] * 4 +
+                                  [c_int] + [c_void_p] * 5),
     "dab_ipa_f32_workspace_bytes": (c_size_t, [POINTER(DabIpaDims), c_int]),
     "dab_ipa_fwd_f32": (c_int, [POINTER(DabIpaDims), POINTER(DabIpaWeights), c_void_p, c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_void_p, c_size_t, c_int, c_void_p]),

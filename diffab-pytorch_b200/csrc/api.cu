@@ -40,7 +40,7 @@ __global__ void __launch_bounds__(256) cast_bf16_kernel(const float4* __restrict
 
 extern "C" {
 
-int dab_version(void) { return 101; /* 0.1.1: `generate` bits of the diffusion and loss entry points */ }
+int dab_version(void) { return 102; /* 0.1.2: dab_reverse_step_weighted (per-residue amino-acid weights) */ }
 
 const char* dab_last_error(void) { return dab::g_error; }
 

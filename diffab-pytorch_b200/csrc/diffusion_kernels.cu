@@ -144,12 +144,12 @@ __global__ void __launch_bounds__(128) reverse_step_kernel(
     Sched sc, const int64_t* seq_t, const float* x_t, const float* O_t,  // may alias the outputs (in-place)
     const float* __restrict__ eps_theta, const float* __restrict__ v_theta, const float* __restrict__ seq_post,
     const uint8_t* __restrict__ mask, const int64_t* __restrict__ t, int B, int L,
-    const float* __restrict__ seq_exp, const float* __restrict__ z, const float* __restrict__ rotvec, int generate,
-    int64_t* seq_out, float* x_out, float* O_out, float* O0_out) {
+    const float* __restrict__ seq_exp, const float* __restrict__ z, const float* __restrict__ rotvec,
+    const float* __restrict__ seq_weight, int generate, int64_t* seq_out, float* x_out, float* O_out, float* O0_out) {
   int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= (int64_t)B * L) return;
   reverse_update_residue(sc, r, (int)t[r / L], seq_t, x_t, O_t, eps_theta, v_theta, seq_post, mask, seq_exp, z, rotvec + r * 3,
-                         generate, seq_out, x_out, O_out, O0_out);
+                         seq_weight, generate, seq_out, x_out, O_out, O0_out);
 }
 
 static int check_sched(const DabSchedule* s, Sched& out, const char* name) {
@@ -157,6 +157,28 @@ static int check_sched(const DabSchedule* s, Sched& out, const char* name) {
               DAB_EINVAL, "%s: incomplete schedule", name);
   out = Sched{s->T, s->alpha, s->alpha_bar, s->alpha_bar_sqrt, s->one_minus_alpha_bar_sqrt, s->beta};
   return DAB_OK;
+}
+
+// dab_reverse_step and dab_reverse_step_weighted (seq_weight may be NULL: the unweighted draw)
+static int reverse_step_launch(const char* name, const DabSchedule* sched, const int64_t* seq_t, const float* x_t,
+                               const float* O_t, const float* eps_theta, const float* v_theta, const float* seq_post,
+                               const uint8_t* mask, const int64_t* t, int B, int L, const float* seq_exp,
+                               const float* z, const float* rotvec, const float* seq_weight, int generate,
+                               int64_t* seq_out, float* x_out, float* O_out, float* O0_out, void* stream) {
+  Sched sc;
+  if (int rc = check_sched(sched, sc, name)) return rc;
+  if (int rc = check_generate(generate, name)) return rc;
+  DAB_REQUIRE(B >= 0 && L >= 0, DAB_EINVAL, "%s: negative size", name);
+  if ((int64_t)B * L == 0) return DAB_OK;
+  DAB_REQUIRE(seq_t && x_t && O_t && eps_theta && v_theta && seq_post && mask && t && seq_exp && z && rotvec &&
+                  seq_out && x_out && O_out,
+              DAB_EINVAL, "%s: null pointer", name);
+  int64_t n = (int64_t)B * L;
+  reverse_step_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
+      sc, seq_t, x_t, O_t, eps_theta, v_theta, seq_post, mask, t, B, L, seq_exp, z, rotvec, seq_weight, generate,
+      seq_out, x_out, O_out, O0_out);
+  count_launch();
+  return check_launch(name);
 }
 
 }  // namespace dab
@@ -201,20 +223,17 @@ int dab_reverse_step(const DabSchedule* sched, const int64_t* seq_t, const float
                      const float* eps_theta, const float* v_theta, const float* seq_post, const uint8_t* mask,
                      const int64_t* t, int B, int L, const float* seq_exp, const float* z, const float* rotvec,
                      int generate, int64_t* seq_out, float* x_out, float* O_out, float* O0_out, void* stream) {
-  Sched sc;
-  if (int rc = check_sched(sched, sc, "dab_reverse_step")) return rc;
-  if (int rc = check_generate(generate, "dab_reverse_step")) return rc;
-  DAB_REQUIRE(B >= 0 && L >= 0, DAB_EINVAL, "dab_reverse_step: negative size");
-  if ((int64_t)B * L == 0) return DAB_OK;
-  DAB_REQUIRE(seq_t && x_t && O_t && eps_theta && v_theta && seq_post && mask && t && seq_exp && z && rotvec &&
-                  seq_out && x_out && O_out,
-              DAB_EINVAL, "dab_reverse_step: null pointer");
-  int64_t n = (int64_t)B * L;
-  reverse_step_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
-      sc, seq_t, x_t, O_t, eps_theta, v_theta, seq_post, mask, t, B, L, seq_exp, z, rotvec, generate, seq_out, x_out,
-      O_out, O0_out);
-  count_launch();
-  return check_launch("dab_reverse_step");
+  return reverse_step_launch("dab_reverse_step", sched, seq_t, x_t, O_t, eps_theta, v_theta, seq_post, mask, t, B, L,
+                             seq_exp, z, rotvec, nullptr, generate, seq_out, x_out, O_out, O0_out, stream);
+}
+
+int dab_reverse_step_weighted(const DabSchedule* sched, const int64_t* seq_t, const float* x_t, const float* O_t,
+                              const float* eps_theta, const float* v_theta, const float* seq_post, const uint8_t* mask,
+                              const int64_t* t, int B, int L, const float* seq_exp, const float* z, const float* rotvec,
+                              const float* seq_weight, int generate, int64_t* seq_out, float* x_out, float* O_out,
+                              float* O0_out, void* stream) {
+  return reverse_step_launch("dab_reverse_step_weighted", sched, seq_t, x_t, O_t, eps_theta, v_theta, seq_post, mask, t,
+                             B, L, seq_exp, z, rotvec, seq_weight, generate, seq_out, x_out, O_out, O0_out, stream);
 }
 
 }  // extern "C"

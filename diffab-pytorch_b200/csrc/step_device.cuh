@@ -23,14 +23,46 @@ __device__ __forceinline__ int argmax_ratio(F prob, const float* __restrict__ q)
   return best;
 }
 
+// The draw of argmax_ratio under per-type weights w (DiffAb.sample's aa_bias, w = exp(b - max b)): only types with
+// w_k > 0 are eligible, key_k = fl(fl(p_k * w_k) / q_k), first eligible index wins ties.  If every eligible key is 0 (the
+// posterior mass on the allowed types underflowed) the draw is redone from the weights alone, key_k = w_k / q_k with
+// the same q, so a forbidden type is never drawn.  No eligible type: returns `fallback` (the residue keeps its type).
+__device__ __forceinline__ int64_t argmax_ratio_weighted(const float* __restrict__ p, const float* __restrict__ w,
+                                                         const float* __restrict__ q, int64_t fallback) {
+  int best = -1;
+  float best_key = -1.0f;
+#pragma unroll
+  for (int k = 0; k < DAB_VOCAB; ++k) {
+    float wk = __ldg(w + k);
+    if (wk > 0.f) {
+      float key = __fdiv_rn(__fmul_rn(__ldg(p + k), wk), q[k]);
+      if (key > best_key) { best_key = key; best = k; }
+    }
+  }
+  if (best < 0) return fallback;
+  if (best_key == 0.f) {
+    best_key = -1.0f;
+#pragma unroll
+    for (int k = 0; k < DAB_VOCAB; ++k) {
+      float wk = __ldg(w + k);
+      if (wk > 0.f) {
+        float key = __fdiv_rn(wk, q[k]);
+        if (key > best_key) { best_key = key; best = k; }
+      }
+    }
+  }
+  return best;
+}
+
 // Reverse step of residue r (patch b, timestep tt = t[b]); composition fixed by oracle/sampler.py (the reference has none).
 // `rv` = the residue's IGSO(3) rotation-vector draw (global or shared memory).  seq_t / x_t / O_t may alias the outputs.
-// `generate`: DAB_GEN_* bits.
+// `generate`: DAB_GEN_* bits.  `seq_weight` [B*L, 21] (may be NULL, uniform over the launch): the sequence is drawn by
+// argmax_ratio_weighted; its rows are read only where the sequence is generated, like seq_post.
 __device__ __forceinline__ void reverse_update_residue(
     const Sched& sc, int64_t r, int tt, const int64_t* seq_t, const float* x_t, const float* O_t,
     const float* __restrict__ eps_theta, const float* __restrict__ v_theta, const float* __restrict__ seq_post,
     const uint8_t* __restrict__ mask, const float* __restrict__ seq_exp, const float* __restrict__ z, const float* rv,
-    int generate, int64_t* seq_out, float* x_out, float* O_out, float* O0_out) {
+    const float* __restrict__ seq_weight, int generate, int64_t* seq_out, float* x_out, float* O_out, float* O0_out) {
   if (tt < 0 || tt > sc.T) asm volatile("trap;");   // out-of-range timestep: the reference raises IndexError
   bool gen = mask[r] != 0;
   // a modality the run does not generate keeps its old value (`generate` is uniform over the launch)
@@ -41,7 +73,10 @@ __device__ __forceinline__ void reverse_update_residue(
   int64_t s_old = seq_t[r];
   if (gen_seq) {
     const float* p = seq_post + r * DAB_VOCAB;
-    seq_out[r] = argmax_ratio([&](int k) { return __ldg(p + k); }, seq_exp + r * DAB_VOCAB);
+    if (seq_weight)
+      seq_out[r] = argmax_ratio_weighted(p, seq_weight + r * DAB_VOCAB, seq_exp + r * DAB_VOCAB, s_old);
+    else
+      seq_out[r] = argmax_ratio([&](int k) { return __ldg(p + k); }, seq_exp + r * DAB_VOCAB);
   } else {
     seq_out[r] = s_old;
   }

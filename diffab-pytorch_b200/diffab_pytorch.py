@@ -640,6 +640,32 @@ def live_query_tiles(generation_mask, out=None):
     return out
 
 
+def aa_bias_weights(aa_bias, generation_mask, generate_sequence=True):
+    """The per-type weights of the sequence draw, (B, L, 21) fp32 on ``generation_mask``'s device, from ``aa_bias`` (see
+    ``DiffAb.sample``): ``w = exp(b - max_k b)``, so ``w`` is in [0, 1], exactly 0 where ``b = -inf`` and all ones for a
+    bias that is constant over the types.  None stays None.  Raises ``ValueError`` on NaN or +inf, on a shape that does
+    not broadcast to (B, L, 21), on a generated residue with every type at -inf, and when the sequence is not generated
+    (``generate_sequence`` False: the bias would do nothing)."""
+    if aa_bias is None:
+        return None
+    if not generate_sequence:
+        raise ValueError("aa_bias: this design mode does not generate the sequence (generate_sequence is False)")
+    B, L = generation_mask.shape
+    b = torch.as_tensor(aa_bias, device=generation_mask.device)
+    b = b.to(torch.promote_types(b.dtype, torch.float32))
+    try:
+        b = b.expand(B, L, 21)
+    except RuntimeError:
+        raise ValueError(f"aa_bias: shape {tuple(b.shape)} does not broadcast to (B, L, 21) = {(B, L, 21)}") from None
+    if bool((torch.isnan(b) | (b == float("inf"))).any()):
+        raise ValueError("aa_bias: NaN or +inf (use -inf to forbid a type, finite values to bias it)")
+    if bool(((b == float("-inf")).all(-1) & generation_mask.bool()).any()):
+        raise ValueError("aa_bias: a generated residue has every residue type at -inf")
+    # a row at -inf throughout (a context residue) gets w = 0 instead of exp(-inf + inf) = NaN
+    mx = b.amax(-1, keepdim=True).clamp_min(torch.finfo(b.dtype).min)
+    return torch.exp(b - mx).to(torch.float32).contiguous()
+
+
 def _pair_bias_planes(layers, e, out):
     """The pair-bias planes of ``layers`` into ``out`` (fp16 (n_layers, B, L, L, H), contiguous) from the bf16 pair
     tensor ``e``: one pass over it per six layers."""
@@ -1629,17 +1655,27 @@ class DiffAb(nn.Module):
             "gauss": torch.randn(n_steps, B, L, device=device),
         }
 
+    @staticmethod
+    def draw_prior_sequence(B, L, device, generator=None, seq_weight=None):
+        """The t = T prior of the sequence, (B, L) int64: uniform over the 21 types, or with per-type weights
+        (``aa_bias_weights``) the categorical draw of w / sum(w) as ``argmax_k w_k / E_k``, E ~ Exp(1) of shape (B*L, 21)."""
+        if seq_weight is None:
+            return torch.randint(0, 21, (B, L), device=device, generator=generator)
+        E = torch.empty(B * L, 21, device=device).exponential_(generator=generator)
+        return (seq_weight.reshape(B * L, 21) / E).argmax(-1).view(B, L)
+
     graph_block_steps = 20   # reverse steps per replay of the multi-step graph (static noise: ~12 MB per step at B = 256)
 
     @torch.no_grad()
     def reverse_step(self, seq_idx_t, translations_t, orientations_t, res_context_emb, pair_context_emb,
                      generation_mask, t, noise, inplace=False, pair_bias=None, glue_cache=None, beta=None, generate=3,
-                     live=None):
+                     live=None, seq_weight=None):
         """One reverse-diffusion step: epsilon network + fused update kernel.  ``t`` is (B,) int64.
         ``glue_cache`` (``Denoiser.sampling_cache``) switches the dense glue to its regrouped form; ``beta`` = the
         schedule's beta at ``t`` when the caller has already gathered it.  ``generate`` (``diffusion.generate_bits``):
         a modality that is not generated keeps its value.  ``live`` = ``live_query_tiles(generation_mask)`` (with
-        ``glue_cache``): the epsilon network's last layer and heads skip the tiles without a generated residue."""
+        ``glue_cache``): the epsilon network's last layer and heads skip the tiles without a generated residue.
+        ``seq_weight`` = ``aa_bias_weights(...)`` or None: per-type weights of the sequence draw."""
         if beta is None:
             beta = self.dsched.tensors["beta"][t]
         rotvec = None
@@ -1660,16 +1696,17 @@ class DiffAb(nn.Module):
                                                    pair_context_emb, beta, pair_bias)
         return _diffusion.fused_reverse_step(self.dsched, self.so3_reverse, seq_idx_t, translations_t,
                                              orientations_t, eps, v_eps, post, generation_mask, t, noise,
-                                             inplace=inplace, rotvec=rotvec, generate=generate)
+                                             inplace=inplace, rotvec=rotvec, generate=generate, seq_weight=seq_weight)
 
     @torch.no_grad()
     def sample_from_context(self, seq_idx, translations, orientations, res_context_emb, pair_context_emb,
                             generation_mask, noises=None, generator=None, t_start=None, t_stop=1,
-                            use_cuda_graph=False, _valid_len=None):
+                            use_cuda_graph=False, _valid_len=None, seq_weight=None):
         """The reverse loop t_start..t_stop on resident tensors (this is what bench.py's ``value`` times).
         ``pair_context_emb`` may be fp32 (exact path) or bf16 (tensor-core path).  ``noises`` = {t: draws of step t}
         (``draw_step_noise``) injects every random draw (parity tests); it works with and without CUDA graphs.
-        Only the modalities of the design mode (``generate_sequence`` / ``generate_structure``) change."""
+        Only the modalities of the design mode (``generate_sequence`` / ``generate_structure``) change.  ``seq_weight``
+        (``aa_bias_weights``, already validated) weighs the sequence draw of every step."""
         generate = self._generate()
         T = self.T
         t_start = T if t_start is None else t_start
@@ -1694,7 +1731,8 @@ class DiffAb(nn.Module):
                 F.pad(seq_idx, (0, n)), F.pad(translations, (0, 0, 0, n)), torch.cat([orientations, eye], dim=1),
                 F.pad(res_context_emb, (0, 0, 0, n)), F.pad(pair_context_emb, (0, 0, 0, n, 0, n)),
                 F.pad(generation_mask, (0, n)), noises=pad_noise, generator=generator, t_start=t_start, t_stop=t_stop,
-                use_cuda_graph=use_cuda_graph, _valid_len=L0)
+                use_cuda_graph=use_cuda_graph, _valid_len=L0,
+                seq_weight=None if seq_weight is None else F.pad(seq_weight, (0, 0, 0, n), value=1.0))
             return {k: v[:, :L0].contiguous() for k, v in out.items()}
         s, x, O = seq_idx.clone(), translations.clone().contiguous(), orientations.clone().contiguous()
         B, L = s.shape
@@ -1703,7 +1741,7 @@ class DiffAb(nn.Module):
         with _tf32_matmuls(pair_context_emb.dtype == torch.bfloat16):
             if use_cuda_graph and generator is None:
                 return self._sample_graphed(s, x, O, res_context_emb, pair_context_emb, generation_mask, t_start,
-                                            t_stop, noises, _valid_len, generate)
+                                            t_stop, noises, _valid_len, generate, seq_weight)
             pair_bias = self._pair_bias_planes(pair_context_emb)
             if pair_bias is not None and _valid_len is not None:
                 _mask_padded_keys(pair_bias, _valid_len)
@@ -1713,7 +1751,8 @@ class DiffAb(nn.Module):
                 t = torch.full((B,), step, device=dev, dtype=torch.int64)
                 noise = noises[step] if noises is not None else self.draw_step_noise(B, L, dev, generator=generator)
                 out = self.reverse_step(s, x, O, res_context_emb, pair_context_emb, generation_mask, t, noise,
-                                        inplace=True, pair_bias=pair_bias, glue_cache=glue, generate=generate, live=live)
+                                        inplace=True, pair_bias=pair_bias, glue_cache=glue, generate=generate, live=live,
+                                        seq_weight=seq_weight)
                 s, x, O = out["seq_idx"], out["translations"], out["orientations"]
             return {"seq_idx": s, "translations": x, "orientations": O}
 
@@ -1739,20 +1778,22 @@ class DiffAb(nn.Module):
         bufs["hist_exp"].exponential_(); bufs["jitter"].uniform_(); bufs["gauss"].normal_()
 
     def _sample_graphed(self, s, x, O, res_ctx, pair_ctx, generation_mask, t_start, t_stop, noises=None, valid_len=None,
-                        generate=3):
+                        generate=3, seq_weight=None):
         """Reverse steps captured in CUDA graphs and replayed; the step index lives in a device tensor.
         The graphs work on static buffers (state, context, mask, pair-bias planes, noise) and are cached per shape and
         ``_lib.weight_key``, so repeated ``sample()`` calls only copy their context in (~1 GB device-to-device, well
         under a millisecond).  Two step graphs: one reverse step, and a block of ``graph_block_steps`` consecutive
         steps; each reads its random draws from static buffers that a small companion graph redraws before every
         replay - or that the caller's ``noises`` are copied into (injected draws, parity tests).  The ``generate`` bits of
-        the design mode are baked into the captured update kernels, so they are part of the cache key."""
+        the design mode are baked into the captured update kernels, so they are part of the cache key.  So is whether
+        ``seq_weight`` is given: the weights are copied into a static buffer on every call, like the mask, so new values
+        need no recapture; without them the graphs are those of the unweighted draw."""
         B, L = s.shape
         dev = s.device
         # the captured graphs bake in packed weights and per-run weight products: recapture when any parameter may have
         # changed (see _lib.weight_key for which updates are noticed on their own)
         key = (B, L, tuple(res_ctx.shape), tuple(pair_ctx.shape), pair_ctx.dtype, str(dev), generate,
-               _lib.weight_key(self.denoiser.parameters()))
+               seq_weight is not None, _lib.weight_key(self.denoiser.parameters()))
         cache = getattr(self, "_graph_cache", None)
         fresh = cache is None or cache["key"] != key
         if fresh:
@@ -1760,9 +1801,12 @@ class DiffAb(nn.Module):
                      "t": torch.full((B,), t_start, device=dev, dtype=torch.int64),
                      "res": torch.empty_like(res_ctx), "pair": torch.empty_like(pair_ctx),
                      "mask": torch.empty_like(generation_mask), "bias": None, "graph": None, "glue": None, "live": None,
-                     "graph_block": None, "noise1": self.draw_step_noise(B, L, dev)}
+                     "graph_block": None, "noise1": self.draw_step_noise(B, L, dev),
+                     "w": None if seq_weight is None else torch.empty_like(seq_weight)}
         st = cache
         st["res"].copy_(res_ctx); st["pair"].copy_(pair_ctx); st["mask"].copy_(generation_mask)
+        if seq_weight is not None:
+            st["w"].copy_(seq_weight)
         if pair_ctx.dtype == torch.bfloat16:   # per-layer pair-bias planes, written straight into the static buffers
             layers = self.denoiser.ipa.layers
             if st["bias"] is None:
@@ -1783,7 +1827,7 @@ class DiffAb(nn.Module):
                     self._fill_noise_(st["noise1"])
                     self.reverse_step(st["s"].clone(), st["x"].clone(), st["O"].clone(), st["res"], st["pair"],
                                       st["mask"], st["t"], st["noise1"], pair_bias=st["bias"], glue_cache=st["glue"],
-                                      generate=generate, live=st["live"])
+                                      generate=generate, live=st["live"], seq_weight=st["w"])
             torch.cuda.current_stream(dev).wait_stream(side)
             draw, graph = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
             with torch.cuda.graph(draw):
@@ -1791,7 +1835,7 @@ class DiffAb(nn.Module):
             with torch.cuda.graph(graph, pool=draw.pool()):
                 self.reverse_step(st["s"], st["x"], st["O"], st["res"], st["pair"], st["mask"], st["t"], st["noise1"],
                                   inplace=True, pair_bias=st["bias"], glue_cache=st["glue"], generate=generate,
-                                  live=st["live"])
+                                  live=st["live"], seq_weight=st["w"])
                 st["t"].sub_(1)
             st["graph"], st["draw"] = graph, draw
             self._graph_cache = st
@@ -1815,7 +1859,8 @@ class DiffAb(nn.Module):
                 for u in range(U):
                     self.reverse_step(st["s"], st["x"], st["O"], st["res"], st["pair"], st["mask"], t_blk[u],
                                       {k: v[u] for k, v in noiseU.items()}, inplace=True, pair_bias=st["bias"],
-                                      glue_cache=st["glue"], beta=beta_blk[u], generate=generate, live=st["live"])
+                                      glue_cache=st["glue"], beta=beta_blk[u], generate=generate, live=st["live"],
+                                      seq_weight=st["w"])
                 st["t"].sub_(U)
             st["graph_block"] = (U, block, draw_block)
         st["s"].copy_(s); st["x"].copy_(x); st["O"].copy_(O)
@@ -1858,7 +1903,7 @@ class DiffAb(nn.Module):
     def sample(self, seq_idx, xyz, orientations, backbone_dihedrals=None, distmat=None, pairwise_dihedrals=None,
                atom_mask=None, chain_idx=None, residue_idx=None, generation_mask=None, residue_mask=None,
                generator=None, precision="bf16", use_cuda_graph=True, context_chunk=32, t_start=None, t_stop=1,
-               init="prior"):
+               init="prior", aa_bias=None):
         """Reverse-diffusion sampling of the masked residues (the reference's stub, made real).
 
         Accepts host or device tensors (host tensors are copied to the model's device; pinned memory
@@ -1870,7 +1915,19 @@ class DiffAb(nn.Module):
         other one is context on every residue and comes back unchanged.  ``init="prior"`` starts the generated
         residues from the t = T prior; ``init="native"`` (optimisation of an existing antibody) starts from the given
         sequence and structure noised to step ``t_start`` (in [1, T], default T) by the forward process, then
-        denoises from there."""
+        denoises from there.
+
+        ``aa_bias`` constrains the designed sequence: a float log-space bias on the residue types, broadcastable to
+        (B, L, 21) - (21,), (L, 21) or (B, L, 21); column k is type k of ``seq_idx``, 20 = UNK.  ``-inf`` forbids a
+        type, 0 everywhere is no bias; on the generated residues it acts as a bias added to the sequence head's logits.
+        It is turned once into weights ``w = exp(b - max_k b)`` (``aa_bias_weights``), and every reverse step draws
+        ``argmax_k p_k w_k / E_k`` over the types with ``w_k > 0`` (E = the step's Exp(1) draw; when the posterior mass
+        on the allowed types underflows, ``argmax_k w_k / E_k``).  The t = T prior becomes ``argmax_k w_k / E_k`` with
+        E ~ Exp(1) of shape (B*L, 21) from ``generator``, in place of the uniform draw.  Every generated residue of the
+        returned ``seq_idx`` has ``w > 0``; context residues keep their type even where it is forbidden; translations
+        and orientations follow the same draws as without the bias.  Refused with ``ValueError``: NaN or +inf, a shape
+        that does not broadcast, a generated residue with every type at -inf, and a design mode that does not generate
+        the sequence."""
         generate = self._generate()
         gen_seq, gen_str = bool(generate & _diffusion.GEN_SEQUENCE), bool(generate & _diffusion.GEN_STRUCTURE)
         if init not in ("prior", "native"):
@@ -1887,6 +1944,7 @@ class DiffAb(nn.Module):
         if generation_mask is None:
             raise ValueError("sample() needs generation_mask: which residues to generate")
         generation_mask = mv(generation_mask).bool()
+        seq_weight = aa_bias_weights(aa_bias, generation_mask, gen_seq)
         residue_mask = torch.ones(B, L, dtype=torch.bool, device=dev) if residue_mask is None else mv(residue_mask).bool()
         atom_mask = torch.ones(B, L, A, dtype=torch.bool, device=dev) if atom_mask is None else mv(atom_mask)
         chain_idx = torch.ones(B, L, dtype=torch.long, device=dev) if chain_idx is None else mv(chain_idx)
@@ -1945,7 +2003,7 @@ class DiffAb(nn.Module):
             # t = T prior on generated residues: s ~ U{0..20}, x ~ N(0, I), O ~ uniform SO(3); drawn in every mode,
             # a modality that is not generated starts (and stays) at its native value
             from .synth import uniform_rotations
-            sT = torch.randint(0, 21, (B, L), device=dev, generator=generator)
+            sT = self.draw_prior_sequence(B, L, dev, generator=generator, seq_weight=seq_weight)
             xT = torch.randn(B, L, 3, device=dev, generator=generator)
             OT = uniform_rotations(B, L, generator=generator, device=dev)
             ms, mx = m & gen_seq, m & gen_str
@@ -1953,4 +2011,5 @@ class DiffAb(nn.Module):
             x = torch.where(mx[..., None], xT, x0)
             O = torch.where(mx[..., None, None], OT, orientations)
         return self.sample_from_context(s, x, O, res_ctx, pair_ctx, m, generator=generator, t_start=t_start,
-                                        t_stop=t_stop, use_cuda_graph=use_cuda_graph and generator is None)
+                                        t_stop=t_stop, use_cuda_graph=use_cuda_graph and generator is None,
+                                        seq_weight=seq_weight)

@@ -184,10 +184,12 @@ def fused_add_noise(dsched, so3_table, seq0, x0, O0, generation_mask, t, noise, 
 
 
 def fused_reverse_step(dsched, so3_rev, seq_t, x_t, O_t, eps_theta, v_theta, seq_post, generation_mask, t, noise,
-                       inplace=False, return_O0=False, rotvec=None, generate=3):
+                       inplace=False, return_O0=False, rotvec=None, generate=3, seq_weight=None):
     """Reverse step (oracle/sampler.py; not in the reference): IGSO(3) sampler + one fused kernel.  ``rotvec``: the step's
     IGSO(3) draw when the caller has already made it (it depends on t and the noise only, not on the network).
-    ``generate`` (``generate_bits``): a modality that is not generated keeps its old value."""
+    ``generate`` (``generate_bits``): a modality that is not generated keeps its old value.  ``seq_weight``: (B, L, 21)
+    fp32 per-type weights of the sequence draw in [0, 1], 0 = forbidden (``DiffAb.sample``'s ``aa_bias``; rule in
+    ``dab_reverse_step_weighted``), or None."""
     seq_t = _lib.dev(seq_t, torch.int64, "seq_idx_t")
     x_t = _lib.dev(x_t, torch.float32, "translations_t")
     O_t = _lib.dev(O_t, torch.float32, "orientations_t")
@@ -206,11 +208,16 @@ def fused_reverse_step(dsched, so3_rev, seq_t, x_t, O_t, eps_theta, v_theta, seq
     if rotvec is None:
         rotvec = so3_rev.sample_isotropic_gaussian(t, L, noise=noise)
     rotvec = _lib.dev(rotvec, torch.float32, "rotvec")
+    if seq_weight is not None:
+        seq_weight = _lib.dev(seq_weight, torch.float32, "seq_weight")
+        if seq_weight.shape != (B, L, V):
+            raise ValueError(f"seq_weight: expected shape {(B, L, V)}, got {tuple(seq_weight.shape)}")
     O0 = torch.empty_like(O_t) if return_O0 else None
-    _lib.check(_lib.lib().dab_reverse_step(dsched.ref(), ptr(seq_t), ptr(x_t), ptr(O_t), ptr(eps_theta), ptr(v_theta),
-                                           ptr(seq_post), ptr(m), ptr(t), B, L, ptr(seq_exp), ptr(z), ptr(rotvec),
-                                           generate, ptr(s_out), ptr(x_out), ptr(O_out), ptr(O0), _lib.stream_ptr()),
-               "dab_reverse_step")
+    _lib.check(_lib.lib().dab_reverse_step_weighted(dsched.ref(), ptr(seq_t), ptr(x_t), ptr(O_t), ptr(eps_theta),
+                                                    ptr(v_theta), ptr(seq_post), ptr(m), ptr(t), B, L, ptr(seq_exp),
+                                                    ptr(z), ptr(rotvec), ptr(seq_weight), generate, ptr(s_out),
+                                                    ptr(x_out), ptr(O_out), ptr(O0), _lib.stream_ptr()),
+               "dab_reverse_step_weighted")
     out = {"seq_idx": s_out, "translations": x_out, "orientations": O_out}
     if return_O0:
         out["orientations_t0"] = O0

@@ -65,10 +65,16 @@ def all_gather_samples(samples: Dict[str, torch.Tensor], n_total: int, group=Non
 
 
 def sample_sharded(model, batch: Dict[str, torch.Tensor], group=None, **sample_kwargs) -> Dict[str, torch.Tensor]:
-    """``DiffAb.sample`` on this rank's contiguous shard of `batch`, then an all-gather of the results."""
+    """``DiffAb.sample`` on this rank's contiguous shard of `batch`, then an all-gather of the results.  A per-patch
+    ``aa_bias`` of shape (B, L, 21) travels in ``batch["aa_bias"]`` and is sharded with it; one shared by every patch
+    ((21,) or (L, 21)) can go in ``sample_kwargs``, which are passed on unchanged."""
     rank, world = world_info(group)
     n = batch["seq_idx"].shape[0]
     local = shard_batch(batch, rank, world)
+    if "aa_bias" in local:
+        if "aa_bias" in sample_kwargs:
+            raise ValueError("sample_sharded: aa_bias given both in batch and as a keyword")
+        sample_kwargs = dict(sample_kwargs, aa_bias=local["aa_bias"])
     out = model.sample(local["seq_idx"], local["xyz"], local["orientations"], local.get("backbone_dihedrals"),
                        local.get("distmat"), local.get("pairwise_dihedrals"), local.get("atom_mask"),
                        local.get("chain_idx"), local.get("residue_idx"), local["generation_mask"],

@@ -38,7 +38,7 @@ extern "C" {
 
 #define DAB_VOCAB 21 /* diffusion.py:47 (hard-coded there) */
 
-/* `generate` bits of dab_forward_noise, dab_reverse_step and dab_losses_fwd/bwd: which modalities the masked
+/* `generate` bits of dab_forward_noise, dab_reverse_step(_weighted) and dab_losses_fwd/bwd: which modalities the masked
  * residues generate.  3 = co-design (the reference's training task), 1 = fixed-backbone sequence design,
  * 2 = structure prediction; any other value is refused with DAB_EINVAL. */
 #define DAB_GEN_SEQUENCE 1
@@ -115,6 +115,20 @@ int dab_reverse_step(const DabSchedule* sched, const int64_t* seq_t, const float
                      const uint8_t* mask, const int64_t* t, int B, int L, const float* seq_exp,
                      const float* z, const float* rotvec, int generate, int64_t* seq_out, float* x_out,
                      float* O_out, float* O0_out, void* stream);
+
+/* dab_reverse_step with per-residue amino-acid weights on the sequence draw (DiffAb.sample's aa_bias: the host turns
+ * a log-space bias b into w = exp(b - max_k b), so w is in [0, 1] and 0 forbids a type).  seq_weight[B*L,21] fp32,
+ * read only where the sequence is generated (mask set and DAB_GEN_SEQUENCE in `generate`), like seq_post.
+ * Only types with w_k > 0 are eligible; s' = the first eligible k with the largest fl(fl(p_k * w_k) / q_k), q = seq_exp.
+ * If every eligible key is 0 (the posterior mass on the allowed types underflowed), the draw is redone with
+ * key_k = w_k / q_k over the eligible types and the same q: a draw from the weights alone, never a forbidden type.
+ * A residue with no eligible type keeps its old type.  x', O' and O0 are those of dab_reverse_step, bit for bit.
+ * seq_weight == NULL is dab_reverse_step, bit for bit.  Argument checks as dab_reverse_step. */
+int dab_reverse_step_weighted(const DabSchedule* sched, const int64_t* seq_t, const float* x_t, const float* O_t,
+                              const float* eps_theta, const float* v_theta, const float* seq_post,
+                              const uint8_t* mask, const int64_t* t, int B, int L, const float* seq_exp,
+                              const float* z, const float* rotvec, const float* seq_weight, int generate,
+                              int64_t* seq_out, float* x_out, float* O_out, float* O0_out, void* stream);
 
 /* ------------------------------------------------------------------ invariant point attention */
 /* One InvariantPointAttentionLayer (diffab_pytorch.py:339-465, use_pair_bias=True).
